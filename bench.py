@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- encode+decode MPix/s of the jpezy hot path on N B200s (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c4] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c4] [--impl reference] [--dump-outputs DIR]
 
 A step = one pass of the hot path over one batch of synthetic input per GPU:
   c2 (default, BASELINE.json configs[1]): one 3840x2160 RGB image, encode then decode
@@ -11,6 +11,12 @@ A step = one pass of the hot path over one batch of synthetic input per GPU:
 through the host-buffer C-ABI calls (jpezyb200_encode / jpezyb200_decode) with pinned host buffers and the
 H2D/D2H copies inside the timed region.  L2: inputs/outputs rotate through a ring of distinct frames whose
 footprint exceeds the 126 MB L2 (see config.l2).
+
+--dump-outputs DIR writes what the last timed step returned to its caller (rank 0, by-image workloads) as float32 / float64
+.npy files, so that two builds can be compared output for output on identical seeded inputs:
+  segments.npy       the entropy-coded segments of the step's images, concatenated (a seeded sample when large)
+  segment_bytes.npy  the length of each image's segment
+  decoded.npy        the decoded planes, [3, batch, plane bytes] flattened (a seeded sample when large)
 """
 import argparse
 import json
@@ -22,6 +28,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 WORKLOADS = {
     "c2": dict(W=3840, H=2160, batch=1, gray=False, name="C2: single 3840x2160 RGB image, encode+decode round trip"),
@@ -522,6 +529,32 @@ def extra_configs(args, ctx, dist, rank, local_rank, world):
     return out
 
 
+# --dump-outputs stays under 64 MB: 12 Mi float32 decoded samples + 3 Mi float32 segment bytes + the segment lengths
+DUMP_DECODED_VALUES = 12 << 20
+DUMP_SEGMENT_VALUES = 3 << 20
+
+
+def dump_outputs(out_dir, scan, nbytes, planes):
+    """One ring slot's results, its work finished: scan [B, slot] uint8, nbytes [B] int64, planes [3, B, plane_len] uint8 on the
+    device -> out_dir/{segments,segment_bytes,decoded}.npy.  An array above its budget is replaced by the values at a seeded
+    sample of its positions (sorted; the same positions in every run with the same arguments)."""
+    import numpy as np
+    import torch
+
+    def sample(flat, budget, seed):
+        if flat.numel() > budget:
+            idx = np.unique(np.random.default_rng(seed).integers(0, flat.numel(), size=budget))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        return flat.cpu().numpy().astype(np.float32)
+
+    lengths = nbytes.cpu().numpy()
+    segments = torch.cat([scan[i, : int(n)] for i, n in enumerate(lengths)])
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "segments.npy"), sample(segments, DUMP_SEGMENT_VALUES, 1))
+    np.save(os.path.join(out_dir, "segment_bytes.npy"), lengths.astype(np.float64))
+    np.save(os.path.join(out_dir, "decoded.npy"), sample(planes.reshape(-1), DUMP_DECODED_VALUES, 2))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -542,7 +575,14 @@ def main():
     ap.add_argument("--e2e-lanes", type=int, default=2, help="host pipelines (encode thread + decode thread each) run side by side in the e2e measurement")
     ap.add_argument("--no-configs", action="store_true", help="skip the c3 / c5 / c4_shard measurements appended to the default line")
     ap.add_argument("--host-lengths", action="store_true", help="segment lengths through a host array between encoder and decoder (round-1 step)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the segments and decoded planes of the last timed step "
+                    "(rank 0) to DIR/*.npy; by-image workloads only")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    sharded = args.workload == "c5" or (args.workload == "c4" and int(os.environ.get("WORLD_SIZE", "1")) > 1 and args.shard)
+    if args.dump_outputs and (args.impl == "reference" or sharded):
+        ap.error("--dump-outputs covers the by-image workloads of --impl b200 (c1, c2, c3, c4 without --shard)")
     claim_stdout()
     wl = dict(WORKLOADS[args.workload])
     if args.batch:
@@ -553,7 +593,7 @@ def main():
         return run_reference(args, wl)
     if args.workload == "c5":
         return run_sharded(args, wl)
-    if args.workload == "c4" and int(os.environ.get("WORLD_SIZE", "1")) > 1 and args.shard:
+    if sharded:
         return run_sharded_gray(args, wl)
     args.steps = args.steps or 200
     args.warmup = args.warmup if args.warmup is not None else 10
@@ -707,6 +747,9 @@ def main():
     ms = timed_steps(n_fly)
     launches = sum(c.stat(capi.STAT_KERNEL_LAUNCHES) for c in fly_ctx) - l0
     psnr_after = check_round_trip((args.steps - 1) % ring)      # the last step's output, after the timed loop
+    if args.dump_outputs and rank == 0:
+        k_last = (args.steps - 1) % ring
+        dump_outputs(args.dump_outputs, d_scan[k_last], d_nbytes[k_last], d_out[k_last])
     value = world * B * npx * args.steps / (ms * 1e-3) / 1e6
     one_in_flight = None
     if n_fly > 1:      # the same K steps one after the other on one stream, for comparison
