@@ -61,11 +61,9 @@ enum {
     JPEZYB200_OPT_PAD_ONES = 1,   /* fill bits of the last scan byte: 1 (default, T.81 F.1.2.3) or 0.
                                      Replaces the padding decision inside srook::io::jpeg::bofstream
                                      (call site src/encoder/jpezy_writer.hpp:101-105). */
-    JPEZYB200_OPT_TRANSFORM = 2,  /* forward/inverse transform kernel variant: 0 = fast path with
+    JPEZYB200_OPT_TRANSFORM = 2,  /* forward/inverse transform kernels: 0 = fast path with
                                      guard band + exact recompute (default), 1 = FP64 separable
-                                     (validation build); A/B runs: 2 = one thread per block in the forward
-                                     kernel + first-generation inverse kernel, 3 = second-generation
-                                     (persistent, bulk-copy fed) forward kernel; same results        */
+                                     (validation build); same results.  Other values: EINVAL        */
     JPEZYB200_OPT_BATCH_GROUP_BYTES = 4, /* jpezyb200_encode_batch / decode_batch: host<->device bytes per pipeline stage
                                      (default 96 MiB; images per group = value / (3 * pixels), at least 1)      */
     JPEZYB200_OPT_SHARD_SCRATCH_BYTES = 5, /* jpezyb200_shard_encode_*: bytes of device scratch for this rank's un-stuffed bits;

@@ -16,7 +16,6 @@
 #include "dec_transform_g.cuh"
 #include "enc_entropy.cuh"
 #include "enc_transform.cuh"
-#include "enc_transform2.cuh"
 #include "enc_shard.cuh"
 #include "synth.cuh"
 
@@ -57,8 +56,6 @@ static void batch_pipe_destroy(jpezyb200_ctx* ctx);
 using namespace jz;
 
 extern "C" {
-
-static void host_pipe_destroy(jpezyb200_ctx* ctx);
 
 int jpezyb200_abi_version(void) { return JPEZYB200_ABI_VERSION; }
 
@@ -113,29 +110,24 @@ int jpezyb200_ctx_create(int device, jpezyb200_ctx** out)
         JZ_CUDA_TRY(ctx, cudaMemcpyToSymbol(cC, &h, sizeof h));
         JZ_CUDA_TRY(ctx, cudaMemcpyToSymbol(gCosRef, h.cos_ref, sizeof h.cos_ref));
         {
-            // constants of the FP32 AAN path: K folds the AAN scale factors, the /8 and 1/q; G is the guard band
-            // (1.25 x worst-case flowgraph error + the rounding of w itself) in w units; T the "quantises to 0" test
-            QuantConst qc{};
+            // constants of the FP32 AAN path per (class, column j): K folds the AAN scale factors, the /8 and 1/q; G is the guard
+            // band (1.25 x worst-case flowgraph error + the rounding of w itself) in w units; T the "quantises to 0" test
             double aan[8];
             aan[0] = 1.0;
             for (int k = 1; k < 8; ++k) aan[k] = std::cos(k * 3.14159265358979323846 / 16) * std::sqrt(2.0);
-            for (int c = 0; c < 2; ++c)
-                for (int i = 0; i < 8; ++i)
-                    for (int j = 0; j < 8; ++j) {
-                        const double q = c ? kQuantChroma[i * 8 + j] : kQuantLuma[i * 8 + j];
-                        const double K = 1.0 / (8.0 * aan[i] * aan[j] * q);
-                        const double Gd = (1.25 * kAanErrBound[i * 8 + j] + 5e-4) / q;
-                        qc.K[c][i * 8 + j] = float(K);
-                        qc.G[c][i * 8 + j] = float(Gd);
-                        qc.T[c][i * 8 + j] = float((1.0 - 2.0 * Gd) / K);
-                    }
-            JZ_CUDA_TRY(ctx, cudaMemcpyToSymbol(cQ, &qc, sizeof qc));
             QuantCol col[2][8];
             uint2 izzc[8];
             for (int j = 0; j < 8; ++j) {
                 uint8_t zb[8];
                 for (int i = 0; i < 8; ++i) {
-                    for (int c = 0; c < 2; ++c) col[c][j].K[i] = qc.K[c][i * 8 + j], col[c][j].T[i] = qc.T[c][i * 8 + j], col[c][j].G[i] = qc.G[c][i * 8 + j];
+                    for (int c = 0; c < 2; ++c) {
+                        const double q = c ? kQuantChroma[i * 8 + j] : kQuantLuma[i * 8 + j];
+                        const double K = 1.0 / (8.0 * aan[i] * aan[j] * q);
+                        const double Gd = (1.25 * kAanErrBound[i * 8 + j] + 5e-4) / q;
+                        col[c][j].K[i] = float(K);
+                        col[c][j].G[i] = float(Gd);
+                        col[c][j].T[i] = float((1.0 - 2.0 * Gd) / K);
+                    }
                     zb[i] = h.izz[i * 8 + j];
                 }
                 izzc[j].x = uint32_t(zb[0]) | (uint32_t(zb[1]) << 8) | (uint32_t(zb[2]) << 16) | (uint32_t(zb[3]) << 24);
@@ -143,25 +135,6 @@ int jpezyb200_ctx_create(int device, jpezyb200_ctx** out)
             }
             JZ_CUDA_TRY(ctx, cudaMemcpyToSymbol(gQcol, col, sizeof col));
             JZ_CUDA_TRY(ctx, cudaMemcpyToSymbol(gIzzCol, izzc, sizeof izzc));
-            // second-generation forward kernel (enc_transform2.cuh): (K, K) pairs per (class, column); the DC multiplier
-            // carries 1 - 2^-20 so that trunc(S * K) reproduces int(int(((S*c)*c)/4)/q) for every sum S; class 2 = zeros
-            Q2Tab q2;
-            std::memset(&q2, 0, sizeof q2);
-            for (int c = 0; c < 2; ++c) {
-                double gmax = 0.0;
-                for (int j = 0; j < 8; ++j)
-                    for (int i = 0; i < 8; ++i) {
-                        float K = qc.K[c][i * 8 + j];
-                        if ((i | j) == 0) K = float((1.0 - 1.0 / 1048576.0) / (8.0 * (c ? kQuantChroma[0] : kQuantLuma[0])));
-                        else gmax = std::max(gmax, double(qc.G[c][i * 8 + j]));
-                        q2.K[c][i >> 1][j][i & 1] = make_float2(K, K);
-                        q2.G[c][i][j] = qc.G[c][i * 8 + j];
-                    }
-                const float thr = float(1.0 - 2.0 * gmax);
-                std::memcpy(&q2.thr[c], &thr, 4);
-            }
-            for (int j = 0; j < 8; ++j) q2.izz[j] = izzc[j];
-            JZ_CUDA_TRY(ctx, cudaMemcpyToSymbol(gQ2, &q2, sizeof q2));
         }
         HuffEncLut lut[2];
         build_enc_lut(kDcLuma, kAcLuma, &lut[0]);
@@ -204,10 +177,10 @@ void jpezyb200_ctx_destroy(jpezyb200_ctx* ctx)
     for (void* tb : ctx->inv2_tab)
         if (tb) cudaFree(tb);
     jz::batch_pipe_destroy(ctx);
-    host_pipe_destroy(ctx);
     std::free(ctx->shard_state);
     if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
     if (ctx->h_sizes) cudaFreeHost(ctx->h_sizes);
+    if (ctx->h_words) cudaFreeHost(ctx->h_words);
     if (ctx->aux_stream) cudaStreamSynchronize(ctx->aux_stream), cudaStreamDestroy(ctx->aux_stream);
     if (ctx->aux_fork) cudaEventDestroy(ctx->aux_fork);
     if (ctx->aux_join) cudaEventDestroy(ctx->aux_join);
@@ -220,7 +193,10 @@ int jpezyb200_set_option(jpezyb200_ctx* ctx, int option, int64_t value)
     if (!ctx) return JPEZYB200_EINVAL;
     switch (option) {
     case JPEZYB200_OPT_PAD_ONES: ctx->pad_ones = value ? 1 : 0; return JPEZYB200_OK;
-    case JPEZYB200_OPT_TRANSFORM: ctx->transform_variant = int(value); return JPEZYB200_OK;
+    case JPEZYB200_OPT_TRANSFORM:
+        if (value != 0 && value != 1) return ctx->fail(JPEZYB200_EINVAL, "transform: 0 (production kernels) or 1 (FP64 validation kernels)");
+        ctx->fp64_transforms = value == 1;
+        return JPEZYB200_OK;
     case JPEZYB200_OPT_BATCH_GROUP_BYTES:
         if (value < 1) return ctx->fail(JPEZYB200_EINVAL, "group bytes must be positive");
         ctx->group_bytes = value;
@@ -261,55 +237,6 @@ int jpezyb200_get_stat(jpezyb200_ctx* ctx, int stat, uint64_t* value)
 // -------------------------------------------------------------------------------------------------
 // encoder
 // -------------------------------------------------------------------------------------------------
-// copy stream + events of the band-pipelined single-image host entry points (jpezyb200_encode / jpezyb200_decode)
-constexpr int kHostBands = 8;
-// bands of MCU rows whose copies overlap the transform kernels.  Measured on a 4K frame: 1 band 6.48 GPix/s, 2: 6.49, 3: 6.44,
-// 4: 6.34, 8: 6.23 -- the round trip is bound by the two 25 MB PCIe copies, the 77 us of transform time that could hide behind
-// them do not pay for the extra copy calls.  Default 1 (JPEZY_B200_HOST_BANDS overrides, for experiments).
-static size_t host_bands()
-{
-    static const size_t n = [] { const char* e = std::getenv("JPEZY_B200_HOST_BANDS"); const long v = e ? std::atol(e) : 1; return size_t(v < 1 ? 1 : (v > kHostBands ? kHostBands : v)); }();
-    return n;
-}
-struct HostPipe {
-    cudaStream_t copy = nullptr;
-    cudaEvent_t ev[kHostBands] = {};
-    uint64_t* h_sz = nullptr;      // pinned: sizes / status read back by the host
-};
-static void host_pipe_destroy(jpezyb200_ctx* ctx);
-static int host_pipe(jpezyb200_ctx* ctx, HostPipe** out)
-{
-    if (!ctx->host_pipe) {
-        // built completely before it is used: a half-made pipe (a failed stream / event / pinned allocation) is torn down again
-        HostPipe* hp = new (std::nothrow) HostPipe();
-        if (!hp) return JPEZYB200_ENOMEM;
-        ctx->host_pipe = hp;
-        const int rc = [&]() -> int {
-            JZ_CUDA_TRY(ctx, cudaStreamCreateWithFlags(&hp->copy, cudaStreamNonBlocking));
-            for (cudaEvent_t& e : hp->ev) JZ_CUDA_TRY(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            JZ_CUDA_TRY(ctx, cudaMallocHost(&hp->h_sz, 64));
-            return JPEZYB200_OK;
-        }();
-        if (rc != JPEZYB200_OK) {
-            host_pipe_destroy(ctx);
-            return rc;
-        }
-    }
-    *out = static_cast<HostPipe*>(ctx->host_pipe);
-    return JPEZYB200_OK;
-}
-static void host_pipe_destroy(jpezyb200_ctx* ctx)
-{
-    HostPipe* hp = static_cast<HostPipe*>(ctx->host_pipe);
-    if (!hp) return;
-    if (hp->copy) cudaStreamSynchronize(hp->copy), cudaStreamDestroy(hp->copy);
-    for (cudaEvent_t e : hp->ev)
-        if (e) cudaEventDestroy(e);
-    if (hp->h_sz) cudaFreeHost(hp->h_sz);
-    delete hp;
-    ctx->host_pipe = nullptr;
-}
-
 static int check_geometry(jpezyb200_ctx* ctx, uint32_t W, uint32_t H, uint32_t nimg)
 {
     if (!ctx) return JPEZYB200_EINVAL;
@@ -319,67 +246,18 @@ static int check_geometry(jpezyb200_ctx* ctx, uint32_t W, uint32_t H, uint32_t n
     return JPEZYB200_OK;
 }
 
-// the bulk copies of k_fwd_transform2 move whole 16-byte units: every pixel row and the coefficient buffer must start on one
-static bool fwd2_ok(const FwdParams& p)
-{
-    const uintptr_t a = reinterpret_cast<uintptr_t>(p.r) | reinterpret_cast<uintptr_t>(p.g) | reinterpret_cast<uintptr_t>(p.b) |
-                        reinterpret_cast<uintptr_t>(p.coefs);
-    return (p.W & 15u) == 0 && (a & 15u) == 0 && (p.plane_stride & 15u) == 0;
-}
-
-// picks the forward-transform kernel for the parameters (JPEZYB200_OPT_TRANSFORM, alignment) and launches it
+// picks the forward-transform kernel (JPEZYB200_OPT_TRANSFORM) and launches it
 static int launch_fwd_kernel(jpezyb200_ctx* ctx, const FwdParams& p, uint32_t nimg, cudaStream_t st)
 {
-    if (ctx->transform_variant == 1) {
+    if (ctx->fp64_transforms) {
         dim3 grid((p.HU + kMcuPerCta - 1) / kMcuPerCta, p.VU, nimg);
         k_fwd_transform_f64<<<grid, kFwdThreads, 0, st>>>(p);
-    } else if (ctx->transform_variant == 3 && fwd2_ok(p)) {
-        // second-generation kernel: persistent CTAs, rows fetched by bulk copies (needs 16-byte aligned rows and buffers).  Measured
-        // against the production kernel below in one run (DESIGN.md 7): equal on a single 4K frame (28.3 us), 10 % slower on batches
-        // (404 against 365 us for 64 HD frames), half as fast on S-noise -- so it stays an A/B variant (JPEZYB200_OPT_TRANSFORM = 3)
-        // JPEZY_B200_FWD_CFG (tuning runs): 83 = the compute warps store their own blocks (default), 82 = the DMA warp stores whole tiles,
-        // 84 = as 83 with four input stages
-        static const int cfg = [] { const char* e = std::getenv("JPEZY_B200_FWD_CFG"); return e ? std::atoi(e) : 83; }();
-        if (!ctx->fwd2_attr_set) {
-            JZ_CUDA_TRY(ctx, cudaFuncSetAttribute(k_fwd_transform2<8, 3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Fwd2<8, 3>::kSmem));
-            JZ_CUDA_TRY(ctx, cudaFuncSetAttribute(k_fwd_transform2<8, 3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, Fwd2<8, 3>::kSmem));
-            JZ_CUDA_TRY(ctx, cudaFuncSetAttribute(k_fwd_transform2<8, 4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Fwd2<8, 4>::kSmem));
-            JZ_CUDA_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->fwd2_occ[0], k_fwd_transform2<8, 3, true>, Fwd2<8, 3>::kThreads, Fwd2<8, 3>::kSmem));
-            JZ_CUDA_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->fwd2_occ[1], k_fwd_transform2<8, 3, false>, Fwd2<8, 3>::kThreads, Fwd2<8, 3>::kSmem));
-            JZ_CUDA_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->fwd2_occ[2], k_fwd_transform2<8, 4, true>, Fwd2<8, 4>::kThreads, Fwd2<8, 4>::kSmem));
-            JZ_CUDA_TRY(ctx, cudaDeviceGetAttribute(&ctx->num_sms, cudaDevAttrMultiProcessorCount, ctx->device));
-            ctx->fwd2_attr_set = true;
-        }
-        const int T = 8, v = cfg == 82 ? 1 : (cfg == 84 ? 2 : 0);
-        const uint32_t tpr = (p.HU + T - 1) / T;
-        const uint64_t ntiles64 = uint64_t(tpr) * p.VU * nimg;
-        if (ntiles64 > 0xffffffffull) return ctx->fail(JPEZYB200_EINVAL, "too many tiles");
-        const uint32_t ntiles = uint32_t(ntiles64);
-        static const int per_sm_cap = [] { const char* e = std::getenv("JPEZY_B200_FWD_CTAS"); return e ? std::atoi(e) : 0; }();
-        const int per_sm = per_sm_cap > 0 ? std::min(per_sm_cap, ctx->fwd2_occ[v]) : ctx->fwd2_occ[v];
-        const uint32_t grid = std::min<uint32_t>(ntiles, uint32_t(ctx->num_sms * std::max(1, per_sm)));
-        // how (image, MCU row, tile of the row) advance when the tile id grows by the grid size
-        TileStep ts{};
-        ts.tiles_per_row = tpr;
-        const uint32_t per_img = tpr * p.VU;
-        ts.dimg = grid / per_img;
-        ts.dmy = (grid % per_img) / tpr;
-        ts.dbx = (grid % per_img) % tpr;
-        static const uint32_t tsflags = [] { const char* e = std::getenv("JPEZY_B200_FWD_FLAGS"); return e ? uint32_t(std::atoi(e)) : 0u; }();
-        ts.flags = tsflags;
-        if (v == 0) (void)jz_launch(k_fwd_transform2<8, 3, true>, dim3(grid), dim3(Fwd2<8, 3>::kThreads), Fwd2<8, 3>::kSmem, st, p, ntiles, ts);
-        else if (v == 1) (void)jz_launch(k_fwd_transform2<8, 3, false>, dim3(grid), dim3(Fwd2<8, 3>::kThreads), Fwd2<8, 3>::kSmem, st, p, ntiles, ts);
-        else (void)jz_launch(k_fwd_transform2<8, 4, true>, dim3(grid), dim3(Fwd2<8, 4>::kThreads), Fwd2<8, 4>::kSmem, st, p, ntiles, ts);
     } else {
-        dim3 grid((p.HU + kTileMcu - 1) / kTileMcu, p.VU, nimg);
-        if (ctx->transform_variant == 2) (void)jz_launch(k_fwd_transform_t<false>, grid, dim3(256), 0, st, p);    // one thread per block (A/B runs)
-        else {
-            if (!ctx->fwd_attr_set) {   // static + dynamic shared memory exceed 48 KiB: opt in once per context
-                JZ_CUDA_TRY(ctx, cudaFuncSetAttribute(k_fwd_transform_t<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFwdTrSmem));
-                ctx->fwd_attr_set = true;
-            }
-            (void)jz_launch(k_fwd_transform_t<true>, grid, dim3(256), kFwdTrSmem, st, p);
+        if (!ctx->fwd_attr_set) {   // static + dynamic shared memory exceed 48 KiB: opt in once per context
+            JZ_CUDA_TRY(ctx, cudaFuncSetAttribute(k_fwd_transform, cudaFuncAttributeMaxDynamicSharedMemorySize, kFwdTrSmem));
+            ctx->fwd_attr_set = true;
         }
+        (void)jz_launch(k_fwd_transform, dim3((p.HU + kTileMcu - 1) / kTileMcu, p.VU, nimg), dim3(256), kFwdTrSmem, st, p);
     }
     ++ctx->launches;
     JZ_CUDA_TRY(ctx, cudaGetLastError());
@@ -402,7 +280,7 @@ static int launch_fwd(jpezyb200_ctx* ctx, const uint8_t* d_r, const uint8_t* d_g
     p.gray = gray;
     p.guard_counter = ctx->d_counters + 0;
     p.y_exact = ctx->d_y_exact;
-    if (with_meta && ctx->transform_variant != 1) {     // side information for launch_entropy (same context, same images)
+    if (with_meta && !ctx->fp64_transforms) {     // side information for launch_entropy (same context, same images)
         int rc;
         if ((rc = ctx->ensure(ctx->blk_meta, size_t(nimg) * (p.coef_stride >> 6) * 4))) return rc;
         p.bmeta = static_cast<uint32_t*>(ctx->blk_meta.p) + size_t(row0) * p.HU * 6;
@@ -421,7 +299,7 @@ static int launch_entropy(jpezyb200_ctx* ctx, const int16_t* d_coefs, uint32_t W
     EntParams p{};
     p.coefs = d_coefs;
     p.coef_stride = nmcu * 384;
-    p.bmeta = with_meta && ctx->transform_variant != 1 ? static_cast<const uint32_t*>(ctx->blk_meta.p) : nullptr;
+    p.bmeta = with_meta && !ctx->fp64_transforms ? static_cast<const uint32_t*>(ctx->blk_meta.p) : nullptr;
     p.nblk = uint32_t(nmcu * 6);
     p.ntile = (p.nblk + kEntThreads - 1) / kEntThreads;
     p.uslot = round_up(slot_bytes + 64, 16);
@@ -528,27 +406,16 @@ int jpezyb200_encode(jpezyb200_ctx* ctx, const uint8_t* r, const uint8_t* g, con
     uint8_t* d_in = static_cast<uint8_t*>(ctx->planes_in.p);
     uint64_t* d_sz = static_cast<uint64_t*>(ctx->sizes_io.p);
     int16_t* d_coefs = static_cast<int16_t*>(ctx->coefs.p);
+    if (!ctx->h_words) JZ_CUDA_TRY(ctx, cudaMallocHost(reinterpret_cast<void**>(&ctx->h_words), 8 * sizeof(uint64_t)));
     cudaStream_t st = ctx->stream;
-    // bands of MCU rows: the copy of band k+1 (copy stream) overlaps the transform of band k (compute stream)
-    HostPipe* hp;
-    if ((rc = host_pipe(ctx, &hp))) return rc;
-    const uint32_t nband = uint32_t(std::max<size_t>(1, std::min<size_t>(std::min<size_t>(host_bands(), VU), 3 * npx / (size_t(4) << 20))));
-    for (uint32_t k = 0; k < nband; ++k) {
-        const uint32_t row0 = uint32_t(uint64_t(VU) * k / nband), row1 = uint32_t(uint64_t(VU) * (k + 1) / nband);
-        const size_t y0 = std::min<size_t>(H, size_t(row0) * 16), y1 = std::min<size_t>(H, size_t(row1) * 16);
-        // (edge replication reads the last image row: the last band carries it)
-        const size_t off = y0 * W, len = (y1 - y0) * W;
-        if (len) {
-            JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + off, r + off, len, cudaMemcpyHostToDevice, hp->copy));
-            JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + npx + off, g + off, len, cudaMemcpyHostToDevice, hp->copy));
-            JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + 2 * npx + off, b + off, len, cudaMemcpyHostToDevice, hp->copy));
-        }
-        JZ_CUDA_TRY(ctx, cudaEventRecord(hp->ev[k], hp->copy));
-        JZ_CUDA_TRY(ctx, cudaStreamWaitEvent(st, hp->ev[k], 0));
-        if ((rc = launch_fwd(ctx, d_in, d_in + npx, d_in + 2 * npx, W, H, 1, gray, d_coefs, st, row0, row1 - row0, true))) return rc;
-    }
+    // (copies and transform on one stream: bands of MCU rows whose copies overlap the transform measured slower on a 4K frame,
+    // 6.23-6.49 GPix/s for 2-8 bands against 6.48 for one -- the round trip is bound by the PCIe copies)
+    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in, r, npx, cudaMemcpyHostToDevice, st));
+    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + npx, g, npx, cudaMemcpyHostToDevice, st));
+    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + 2 * npx, b, npx, cudaMemcpyHostToDevice, st));
+    if ((rc = launch_fwd(ctx, d_in, d_in + npx, d_in + 2 * npx, W, H, 1, gray, d_coefs, st, 0, 0, true))) return rc;
     if ((rc = launch_entropy(ctx, d_coefs, W, H, 1, static_cast<uint8_t*>(ctx->scan_io.p), scan_cap, d_sz, d_sz + 1, st, true))) return rc;
-    uint64_t* h_sz = hp->h_sz;
+    uint64_t* h_sz = ctx->h_words;
     JZ_CUDA_TRY(ctx, cudaMemcpyAsync(h_sz, d_sz, 2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
     JZ_CUDA_TRY(ctx, cudaStreamSynchronize(st));
     if (h_sz[0] == ~0ull || h_sz[0] > scan_cap) return ctx->fail(JPEZYB200_ECAPACITY, "entropy-coded segment does not fit in scan_cap");

@@ -18,7 +18,6 @@ namespace jz {
 // jz_launch() may be staged while its predecessor still runs.  The wait is a no-op for ordinary launches.
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 inline bool pdl_enabled()
 {
     static const bool on = [] { const char* e = std::getenv("JPEZY_B200_PDL"); return !e || e[0] != '0'; }();
@@ -98,14 +97,14 @@ struct jpezyb200_ctx {
     cudaEvent_t aux_fork = nullptr, aux_join = nullptr;
     std::string err;
     int pad_ones = 1;
-    int transform_variant = 0;
+    bool fp64_transforms = false;   // JPEZYB200_OPT_TRANSFORM = 1: the FP64 validation kernels
     int sync_guesses = 0;     // JPEZYB200_OPT_SYNC_GUESSES
     int sync_rounds = 3;      // launches behind launch 0 (which checks the CTA boundaries itself): two that repair, one that verifies
     int64_t shard_scratch = 0;                 // JPEZYB200_OPT_SHARD_SCRATCH_BYTES (0 = 3 bytes per pixel)
     int64_t group_bytes = int64_t(96) << 20;   // host<->device bytes per stage of the pipelined host batches
     uint64_t launches = 0;
-    bool inv_attr_set = false, fwd_attr_set = false, fwd2_attr_set = false, inv2_attr_set = false;
-    int fwd2_occ[3] = {1, 1, 1}, num_sms = 148;   // resident CTAs per SM of the persistent forward kernels, SMs of the device
+    bool inv_attr_set = false, fwd_attr_set = false, inv2_attr_set = false;
+    int num_sms = 148;                         // SMs of the device
     static constexpr int kInv2Slots = 4;       // tables of k_inv_transform2 per set of quantisation tables (capi_decode.inc)
     void* inv2_tab[kInv2Slots] = {};
     uint16_t inv2_key[kInv2Slots][3][64] = {};
@@ -131,9 +130,9 @@ struct jpezyb200_ctx {
     jz_devbuf dec_scanbytes, dec_chunk_cnt, dec_chunk_base, dec_ubytes, dec_state, dec_dirty, dec_subblk, dec_dc, dec_dcd, blk_meta, dec_status, dec_changed, dec_flags, dec_mcnt, dec_mbase, dec_seg;
     jz_devbuf shard_geom;      // ShardGeom + scratch of the MCU-row sharded encoder (enc_shard.cuh)
     void* batch_pipe = nullptr;    // streams, events and double buffers of the pipelined host batches (capi_batch.inc)
-    void* host_pipe = nullptr;     // copy stream and events of the band-pipelined single-image host entry points (capi.cu)
     void* shard_state = nullptr;   // host copy of the launch parameters between the phases (capi_shard.inc)
     uint64_t* h_sizes = nullptr;   // pinned, 8192 values (jpezyb200_read_sizes)
+    uint64_t* h_words = nullptr;   // pinned, 8 words: sizes / status read back by jpezyb200_encode / jpezyb200_decode
     void* h_pinned = nullptr;
     size_t h_pinned_cap = 0;
 

@@ -2,7 +2,7 @@
 //
 // Replaces inverse_quantization (src/decoder/jpezy_decoder.hpp:645-650), inverse_dct (:652-670), the pixel replication of
 // decode_mcu (:519-524) and make_rgb / to_r,g,b / revise_value (:531-578, :672-676), like k_inv_transform of dec_transform.cuh
-// (which stays as the A/B variant and for unaligned coefficient buffers).  ncu of round 1 showed that kernel bound by
+// (which stays for buffers that are not 16-byte aligned).  ncu of round 1 showed that kernel bound by
 // instruction issue and by its barriers (one thread per 8x8 block with 64 live samples, 96 registers, 25 % of the warp slots
 // filled, four CTA-wide barriers with different numbers of threads working).  Here:
 //
@@ -25,9 +25,70 @@
 // identical to the reference decoder's.  Algorithmic HBM traffic: 3 B/px read + 3 B/px written = 6 B/px.
 #pragma once
 #include "dec_transform.cuh"
-#include "enc_transform2.cuh"
 
 namespace jz {
+
+// ---- async proxy: the bulk copy of a tile's coefficients and its barrier ----
+__device__ __forceinline__ uint32_t smem_u32(const void* p) { return uint32_t(__cvta_generic_to_shared(p)); }
+__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory"); }
+__device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
+__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes)
+{
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+}
+// global -> shared, `bytes` a multiple of 16, both addresses 16-byte aligned; completes `bytes` on the barrier
+__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar)
+{
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
+}
+// wait with a watchdog: a protocol error must trap, not hang the device
+// (try_wait with a suspend-time hint: the warp sleeps in hardware until the phase completes instead of polling)
+__device__ __forceinline__ void mbar_wait_wd(uint32_t bar, uint32_t parity)
+{
+    uint32_t ok, spins = 0;
+    do {
+        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(ok) : "r"(bar), "r"(parity), "r"(1000000u) : "memory");
+        if (!ok && ++spins > (1u << 16)) __trap();
+    } while (!ok);
+}
+
+// ---- packed FP32 pairs (FADD2 / FMUL2 / FFMA2 of sm_100): the two blocks of a pair go through a flowgraph at once; every
+// lane of a pair is an ordinary IEEE add / mul / fma, so the results equal the scalar flowgraph's bit for bit ----
+typedef unsigned long long f32x2;
+__device__ __forceinline__ f32x2 pk2(float lo, float hi)
+{
+    f32x2 r;
+    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
+    return r;
+}
+__device__ __forceinline__ f32x2 add2(f32x2 a, f32x2 b)
+{
+    f32x2 r;
+    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
+    return r;
+}
+__device__ __forceinline__ f32x2 sub2(f32x2 a, f32x2 b)
+{
+    f32x2 r;
+    asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
+    return r;
+}
+__device__ __forceinline__ f32x2 mul2(f32x2 a, f32x2 b)
+{
+    f32x2 r;
+    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
+    return r;
+}
+__device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c)
+{
+    f32x2 r;
+    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
+    return r;
+}
+__device__ __forceinline__ float lo2(f32x2 v) { return __uint_as_float(uint32_t(v)); }
+__device__ __forceinline__ float hi2(f32x2 v) { return __uint_as_float(uint32_t(v >> 32)); }
+
+constexpr float kMagic15 = 12582912.0f;    // 1.5 * 2^23: float(kMagic15 + n) has the integer n in its low mantissa bits (|n| < 2^22)
 
 // per frame descriptor (quantisation tables), laid out for the column lanes; built by k_build_inv2_tab when the tables change
 struct Inv2Tab {
@@ -173,22 +234,9 @@ __device__ __noinline__ uint32_t colour_exact4r(int y0, int y1, int y2, int y3, 
     return colour_exact4(y, sx_lo(cc0), sx_hi(cc0), sx_lo(cc1), sx_hi(cc1), which);
 }
 
-// the colour offsets of one chroma pair (phase 1c of k_inv_transform): fr | fg << 16 and fb | suspect << 16
-__device__ __forceinline__ uint2 chroma_offsets(int cb, int cr)
-{
-    const float a = float(cb - 128), b = float(cr - 128);
-    const int fr = __float2int_rd(b * 1.4020f);
-    const int fb = __float2int_rd(a * 1.7718f);
-    const float tg = fmaf(b, -0.7139f, a * -0.3441f);
-    const int fg = __float2int_rd(tg);
-    const float kf = (tg + kMagic15) - kMagic15;
-    const bool near_int = fabsf(tg - kf) < 7.5e-5f && ((cb ^ 128) | (cr ^ 128)) != 0;
-    const bool wild = (uint32_t(cb + 128) | uint32_t(cr + 128)) > 512u;
-    return make_uint2(__byte_perm(uint32_t(fr), uint32_t(fg), 0x5410), (uint32_t(fb) & 0xffffu) | ((near_int || wild) ? 0x10000u : 0u));
-}
-
-// the same from the packed samples cb | cr << 16, without conversion instructions: floor(x) is the low mantissa bits of
-// x + 1.5 * 2^23 rounded down (|x| < 2^22), two of the three offsets share packed instructions
+// the colour offsets of one chroma pair (as phase 1c of k_inv_transform computes them) from the packed samples cb | cr << 16: fr | fg << 16 and
+// fb | suspect << 16.  No conversion instructions: floor(x) is the low mantissa bits of x + 1.5 * 2^23 rounded down (|x| < 2^22),
+// two of the three offsets share packed instructions
 __device__ __forceinline__ uint2 chroma_offsets_w(uint32_t ccw)
 {
     const f32x2 ab = add2(pk2(float(sx_lo(ccw)), float(sx_hi(ccw))), pk2(-128.0f, -128.0f));       // (cb - 128, cr - 128)

@@ -193,7 +193,7 @@ __global__ void __launch_bounds__(kFwdThreads) k_fwd_transform_f64(const FwdPara
 }
 
 // =====================================================================================================
-// Production kernel: integer colour conversion + FP32 AAN DCT, one thread per 8x8 block.
+// Production kernel: integer colour conversion + FP32 AAN DCT, eight lanes per 8x8 block.
 //
 //  * tile = 16 rows x 512 pixels (32 MCUs, 192 blocks) per CTA of 256 threads
 //  * phase 1 (256 threads): lane = MCU, warp = row pair; 16-byte loads per plane and row; the weighted
@@ -201,9 +201,9 @@ __global__ void __launch_bounds__(kFwdThreads) k_fwd_transform_f64(const FwdPara
 //    quotient is the reference's truncated value unless the weighted sum is an exact multiple of the
 //    denominator, where the reference's FP64 rounding decides (ref_Y/ref_Cb/ref_Cr).  Results are stored
 //    as value+128 bytes in row-major shared tiles (conflict-free 16-byte stores).
-//  * phase 2 (192 threads): warps 0..3 = luma blocks (top/bottom block rows alternate per warp so that the
-//    8-byte row loads of a half-warp are contiguous), warp 4 = Cb, warp 5 = Cr.  AAN flowgraph (5 mul + 29
-//    add per 1-D transform) fully in registers; the AAN scale factors and 1/q are folded into one multiplier.
+//  * phase 2 (256 threads): four blocks per warp and pass (4 luma passes, 2 chroma passes); lane j transforms
+//    row j, the 8x8 transpose goes through a per-warp scratch, lane j transforms column j.  AAN flowgraph (5 mul
+//    + 29 add per 1-D transform) in registers; the AAN scale factors and 1/q are folded into one multiplier.
 //    w = y*K; coefficients with |w| < 1 - guard quantise to 0 without further work (whole-warp test per
 //    natural row); otherwise trunc(w) and the guard test |w - k| < G, k != 0.  G covers the worst-case FP32
 //    error of the flowgraph (tools/aan_error_bound.py); flagged coefficients are recomputed in FP64 (tier 2)
@@ -215,20 +215,14 @@ constexpr int kTileBlk = kTileMcu * 6;
 constexpr int kYStride = 528;      // bytes per row of the luma tile (512 + 16: keeps 16-byte alignment)
 constexpr int kCStride = 272;      // bytes per row of a chroma tile (256 + 16)
 constexpr int kOutStride = 144;    // bytes per block in the staging buffer (128 + 16)
-constexpr int kFwdTrSmem = 8 * 4 * 72 * 4;   // dynamic shared memory of k_fwd_transform_t<true>: the transpose scratch
+constexpr int kFwdTrSmem = 8 * 4 * 72 * 4;   // dynamic shared memory of k_fwd_transform: the transpose scratch
 
-struct QuantConst {
-    float K[2][64];   // 1 / (8 * aan_i * aan_j * q_ij)
-    float T[2][64];   // |y| below this => |w| < 1 - 2G  => quantises to 0, cannot be flagged
-    float G[2][64];   // guard band in w units
-};
-static __constant__ QuantConst cQ;
-// the same constants per (class, column j), for the eight-lanes-per-block DCT whose lanes hold one column each (a
-// constant-bank load with a lane-dependent index would serialise): K and G of coefficients (i, j), i = 0..7
+// quantisation constants per (class, column j), for the DCT lanes that hold one column each (a constant-bank load with a
+// lane-dependent index would serialise), coefficients (i, j), i = 0..7:
 struct QuantCol {
-    float K[8];
-    float T[8];
-    float G[8];
+    float K[8];   // 1 / (8 * aan_i * aan_j * q_ij)
+    float T[8];   // |y| below this => |w| < 1 - 2G  => quantises to 0, cannot be flagged
+    float G[8];   // guard band in w units
 };
 static __device__ QuantCol gQcol[2][8];
 static __device__ uint2 gIzzCol[8];     // zig-zag positions of coefficients (0..7, j), one byte each
@@ -331,7 +325,7 @@ __device__ __forceinline__ void c2(uint32_t rw, uint32_t gw, uint32_t bw, uint32
     cr2 = q[2] | (q[3] << 8);
 }
 
-// AAN forward 1-D DCT on 8 registers (outputs scaled by 8*aan_k per dimension pair, see QuantConst::K)
+// AAN forward 1-D DCT on 8 registers (outputs scaled by 8*aan_k per dimension pair, see QuantCol::K)
 __device__ __forceinline__ void aan_fdct8(float& d0, float& d1, float& d2, float& d3, float& d4, float& d5, float& d6, float& d7)
 {
     const float t0 = d0 + d7, t7 = d0 - d7, t1 = d1 + d6, t6 = d1 - d6;
@@ -352,65 +346,6 @@ __device__ __forceinline__ void aan_fdct8(float& d0, float& d1, float& d2, float
     d3 = z13 - z2;
     d1 = z11 + z4;
     d7 = z11 - z4;
-}
-
-// ---- packed FP32 pairs (FADD2 / FMUL2 / FFMA2 of sm_100): two rows of a block go through the row pass at once; every
-// lane of a pair is an ordinary IEEE add / mul / fma, so the results equal the scalar flowgraph's bit for bit ----
-typedef unsigned long long f32x2;
-__device__ __forceinline__ f32x2 pk2(float lo, float hi)
-{
-    f32x2 r;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-    return r;
-}
-__device__ __forceinline__ void unpk2(f32x2 v, float& lo, float& hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v)); }
-__device__ __forceinline__ f32x2 add2(f32x2 a, f32x2 b)
-{
-    f32x2 r;
-    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
-__device__ __forceinline__ f32x2 sub2(f32x2 a, f32x2 b)
-{
-    f32x2 r;
-    asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
-__device__ __forceinline__ f32x2 mul2(f32x2 a, f32x2 b)
-{
-    f32x2 r;
-    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
-__device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c)
-{
-    f32x2 r;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
-    return r;
-}
-// aan_fdct8 on two independent 8-vectors at once (same operation order)
-__device__ __forceinline__ void aan_fdct8_x2(f32x2& d0, f32x2& d1, f32x2& d2, f32x2& d3, f32x2& d4, f32x2& d5, f32x2& d6, f32x2& d7)
-{
-    const f32x2 c707 = pk2(0.707106781186547524f, 0.707106781186547524f), c382 = pk2(0.382683432365089772f, 0.382683432365089772f);
-    const f32x2 c541 = pk2(0.541196100146196985f, 0.541196100146196985f), c1306 = pk2(1.306562964876376528f, 1.306562964876376528f);
-    const f32x2 t0 = add2(d0, d7), t7 = sub2(d0, d7), t1 = add2(d1, d6), t6 = sub2(d1, d6);
-    const f32x2 t2 = add2(d2, d5), t5 = sub2(d2, d5), t3 = add2(d3, d4), t4 = sub2(d3, d4);
-    const f32x2 t10 = add2(t0, t3), t13 = sub2(t0, t3), t11 = add2(t1, t2), t12 = sub2(t1, t2);
-    d0 = add2(t10, t11);
-    d4 = sub2(t10, t11);
-    const f32x2 z1 = mul2(add2(t12, t13), c707);
-    d2 = add2(t13, z1);
-    d6 = sub2(t13, z1);
-    const f32x2 u10 = add2(t4, t5), u11 = add2(t5, t6), u12 = add2(t6, t7);
-    const f32x2 z5 = mul2(sub2(u10, u12), c382);
-    const f32x2 z2 = fma2(u10, c541, z5);
-    const f32x2 z4 = fma2(u12, c1306, z5);
-    const f32x2 z3 = mul2(u11, c707);
-    const f32x2 z11 = add2(t7, z3), z13 = sub2(t7, z3);
-    d5 = add2(z13, z2);
-    d3 = sub2(z13, z2);
-    d1 = add2(z11, z4);
-    d7 = sub2(z11, z4);
 }
 
 // Fix-up queue: coefficients whose FP32 value is inside the guard band are not decided in the hot loop;
@@ -456,49 +391,6 @@ __device__ __noinline__ int requant_exact(const uint8_t* __restrict__ tile, int 
     return requant_finish(acc, tile, stride, i, j, q, counter);
 }
 
-// quantisation of the 64 AAN outputs of one block; CLS selects the (compile-time) constant set
-template <int CLS>
-__device__ __forceinline__ void quant_block(float (&d)[64], const uint32_t blk, uint32_t* s_nfix, uint16_t* s_fix, uint4* __restrict__ out16)
-{
-    int qv[64];
-    // DC: the reference's sum is an exact integer (cos row 0 is 1.0), so its value is ((S*c)*c)/4 exactly as evaluated
-    {
-        const double v = __dmul_rn(__dmul_rn(__dmul_rn(double(d[0]), cC.inv_sqrt2_ref), cC.inv_sqrt2_ref), 0.25);
-        qv[0] = __double2int_rz(v) / int(CLS ? 17 : 16);
-    }
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        bool large = false;
-#pragma unroll
-        for (int j = (i == 0 ? 1 : 0); j < 8; ++j) large |= fabsf(d[i * 8 + j]) >= cQ.T[CLS][i * 8 + j];
-        if (!__any_sync(0xffffffffu, large)) {
-#pragma unroll
-            for (int j = (i == 0 ? 1 : 0); j < 8; ++j) qv[i * 8 + j] = 0;
-            continue;
-        }
-#pragma unroll
-        for (int j = (i == 0 ? 1 : 0); j < 8; ++j) {
-            const float w = d[i * 8 + j] * cQ.K[CLS][i * 8 + j];
-            qv[i * 8 + j] = __float2int_rz(w);
-            // distance of |w| to the nearest integer >= 1
-            const float a = fabsf(w) - 0.5f;
-            const float kf = (a + 12582912.0f) - 12582912.0f;      // rint(|w| - 0.5)
-            const float delta = a - kf;                             // frac(|w|) - 0.5 in [-0.5, 0.5]
-            if (fabsf(delta) > 0.5f - cQ.G[CLS][i * 8 + j] && fabsf(w) > 0.5f) push_fix(s_nfix, s_fix, (blk << 6) | uint32_t(i * 8 + j));
-        }
-    }
-    // zig-zag, two coefficients per 32-bit word, 16-byte stores into the padded staging buffer
-#pragma unroll
-    for (int c = 0; c < 8; ++c) {
-        uint4 v;
-        v.x = __byte_perm(uint32_t(qv[zz_at(c * 8 + 0)]), uint32_t(qv[zz_at(c * 8 + 1)]), 0x5410);
-        v.y = __byte_perm(uint32_t(qv[zz_at(c * 8 + 2)]), uint32_t(qv[zz_at(c * 8 + 3)]), 0x5410);
-        v.z = __byte_perm(uint32_t(qv[zz_at(c * 8 + 4)]), uint32_t(qv[zz_at(c * 8 + 5)]), 0x5410);
-        v.w = __byte_perm(uint32_t(qv[zz_at(c * 8 + 6)]), uint32_t(qv[zz_at(c * 8 + 7)]), 0x5410);
-        out16[c] = v;
-    }
-}
-
 // location of block `blk` (= mcu*6 + k) of the tile in the shared sample tiles
 __device__ __forceinline__ const uint8_t* block_samples(const uint8_t* s_y, const uint8_t* s_cb, const uint8_t* s_cr, uint32_t blk, int& stride)
 {
@@ -511,14 +403,13 @@ __device__ __forceinline__ const uint8_t* block_samples(const uint8_t* s_y, cons
     return (k == 4u ? s_cb : s_cr) + mcu * 8;
 }
 
-// V8 = true: phase 2 with eight lanes per block (one row, then one column each; the 8x8 transpose goes through a
-// per-warp scratch in shared memory).  A thread then carries 8 samples instead of 64: half the registers, twice the
-// resident warps -- the kernel is latency bound (ncu: issue slots 42 % busy at 16 warps per SM), not throughput bound.
-template <bool V8>
-__global__ void __launch_bounds__(256, V8 ? 4 : 2) k_fwd_transform_t(const FwdParams p)
+// Phase 2 works with eight lanes per block (one row, then one column each; the 8x8 transpose goes through a per-warp
+// scratch in shared memory).  A thread then carries 8 samples instead of the 64 of one thread per block: half the
+// registers, twice the resident warps -- the kernel is latency bound (ncu: issue slots 42 % busy at 16 warps per SM).
+__global__ void __launch_bounds__(256, 4) k_fwd_transform(const FwdParams p)
 {
     pdl_wait();
-    extern __shared__ __align__(16) float s_tr[];                 // V8: [warp][block of the pass][8 rows x 8 + 8 pad] (kFwdTrSmem)
+    extern __shared__ __align__(16) float s_tr[];                 // [warp][block of the pass][8 rows x 8 + 8 pad] (kFwdTrSmem)
     __shared__ __align__(16) uint8_t s_y[16 * kYStride];
     __shared__ __align__(16) uint8_t s_cb[8 * kCStride];
     __shared__ __align__(16) uint8_t s_cr[8 * kCStride];
@@ -593,132 +484,80 @@ __global__ void __launch_bounds__(256, V8 ? 4 : 2) k_fwd_transform_t(const FwdPa
     }
     __syncthreads();
 
-    if constexpr (V8) {
-        // ---- phase 2: DCT + quantisation, eight lanes per block, four blocks per warp and pass ----
-        // passes 0..3: the 128 luma blocks (luma block lb = pass * 32 + warp * 4 + g: MCU lb >> 2, block lb & 3);
-        // passes 4..5: the 32 Cb and the 32 Cr blocks
-        const int g = lane >> 3, j = lane & 7;
-        float* scr = &s_tr[(warp * 4 + g) * 72];
-        const uint2 izz = gIzzCol[j];
+    // ---- phase 2: DCT + quantisation, eight lanes per block, four blocks per warp and pass ----
+    // passes 0..3: the 128 luma blocks (luma block lb = pass * 32 + warp * 4 + g: MCU lb >> 2, block lb & 3);
+    // passes 4..5: the 32 Cb and the 32 Cr blocks
+    const int g = lane >> 3, j = lane & 7;
+    float* scr = &s_tr[(warp * 4 + g) * 72];
+    const uint2 izz = gIzzCol[j];
 #pragma unroll
-        for (int cls = 0; cls < 2; ++cls) {
-            float K[8], T[8];
-            {
-                const float4* q4 = reinterpret_cast<const float4*>(&gQcol[cls][j]);
-                const float4 k0 = q4[0], k1 = q4[1], t0 = q4[2], t1 = q4[3];
-                K[0] = k0.x, K[1] = k0.y, K[2] = k0.z, K[3] = k0.w, K[4] = k1.x, K[5] = k1.y, K[6] = k1.z, K[7] = k1.w;
-                T[0] = t0.x, T[1] = t0.y, T[2] = t0.z, T[3] = t0.w, T[4] = t1.x, T[5] = t1.y, T[6] = t1.z, T[7] = t1.w;
-                if (j == 0) T[0] = 3.0e38f;        // the DC coefficient takes its own path
-            }
+    for (int cls = 0; cls < 2; ++cls) {
+        float K[8], T[8];
+        {
+            const float4* q4 = reinterpret_cast<const float4*>(&gQcol[cls][j]);
+            const float4 k0 = q4[0], k1 = q4[1], t0 = q4[2], t1 = q4[3];
+            K[0] = k0.x, K[1] = k0.y, K[2] = k0.z, K[3] = k0.w, K[4] = k1.x, K[5] = k1.y, K[6] = k1.z, K[7] = k1.w;
+            T[0] = t0.x, T[1] = t0.y, T[2] = t0.z, T[3] = t0.w, T[4] = t1.x, T[5] = t1.y, T[6] = t1.z, T[7] = t1.w;
+            if (j == 0) T[0] = 3.0e38f;        // the DC coefficient takes its own path
+        }
 #pragma unroll 1
-            for (int pass = 0; pass < (cls ? 2 : 4); ++pass) {
-                const uint32_t n = uint32_t(pass) * 32u + uint32_t(warp) * 4u + uint32_t(g);
-                uint32_t blk;
-                const uint8_t* row;
-                if (cls == 0) {
-                    const uint32_t mcu = n >> 2, k = n & 3u;
-                    blk = mcu * 6u + k;
-                    row = &s_y[((k >> 1) * 8 + j) * kYStride + mcu * 16 + (k & 1u) * 8];
-                } else {
-                    const uint32_t mcu = n & 31u, comp = n >> 5;
-                    blk = mcu * 6u + 4u + comp;
-                    row = (comp ? s_cr : s_cb) + j * kCStride + mcu * 8;
-                }
-                float d[8];
-                {
-                    const uint2 w = *reinterpret_cast<const uint2*>(row);
-                    d[0] = float(w.x & 255u), d[1] = float((w.x >> 8) & 255u), d[2] = float((w.x >> 16) & 255u), d[3] = float(w.x >> 24);
-                    d[4] = float(w.y & 255u), d[5] = float((w.y >> 8) & 255u), d[6] = float((w.y >> 16) & 255u), d[7] = float(w.y >> 24);
-                }
-                aan_fdct8(d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7]);      // row j of the block
-                *reinterpret_cast<float4*>(&scr[j * 8]) = make_float4(d[0], d[1], d[2], d[3]);
-                *reinterpret_cast<float4*>(&scr[j * 8 + 4]) = make_float4(d[4], d[5], d[6], d[7]);
-                __syncwarp();
-#pragma unroll
-                for (int i = 0; i < 8; ++i) d[i] = scr[i * 8 + j];
-                __syncwarp();
-                aan_fdct8(d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7]);      // column j: d[i] = coefficient (i, j)
-                int16_t* out = reinterpret_cast<int16_t*>(&s_out[blk * kOutStride]);
-                // rows of coefficients in which some lane of the warp may quantise to a non-zero value (|y| >= T <=> |w| >= 1 - 2G)
-                uint32_t lm = 0;
-#pragma unroll
-                for (int i = 0; i < 8; ++i) lm |= (fabsf(d[i]) >= T[i] ? 1u : 0u) << i;
-                const uint32_t wm = __reduce_or_sync(0xffffffffu, lm);
-                int qv[8];
-#pragma unroll
-                for (int i = 0; i < 8; ++i) {
-                    qv[i] = 0;
-                    if (wm & (1u << i)) {
-                        const float w = d[i] * K[i];
-                        qv[i] = __float2int_rz(w);
-                        // distance of |w| to the nearest integer >= 1
-                        const float a = fabsf(w) - 0.5f;
-                        const float kf = (a + 12582912.0f) - 12582912.0f;      // rint(|w| - 0.5)
-                        const float delta = a - kf;                             // frac(|w|) - 0.5 in [-0.5, 0.5]
-                        if (fabsf(delta) > 0.5f - gQcol[cls][j].G[i] && fabsf(w) > 0.5f && (i | j) != 0)
-                            push_fix(&s_nfix, s_fix, (blk << 6) | uint32_t(i * 8 + j));
-                    }
-                }
-                if (j == 0) {
-                    // DC: the reference's sum is an exact integer (cos row 0 is 1.0), so its value is ((S*c)*c)/4 exactly as
-                    // evaluated; level shift: the samples are stored as value + 128 (64 * 128, exact)
-                    const double v = __dmul_rn(__dmul_rn(__dmul_rn(double(d[0] - 8192.0f), cC.inv_sqrt2_ref), cC.inv_sqrt2_ref), 0.25);
-                    qv[0] = cls ? __double2int_rz(v) / 17 : __double2int_rz(v) / 16;
-                }
-#pragma unroll
-                for (int i = 0; i < 8; ++i) out[__byte_perm(i < 4 ? izz.x : izz.y, 0, 0x4440 + (i & 3))] = int16_t(qv[i]);
+        for (int pass = 0; pass < (cls ? 2 : 4); ++pass) {
+            const uint32_t n = uint32_t(pass) * 32u + uint32_t(warp) * 4u + uint32_t(g);
+            uint32_t blk;
+            const uint8_t* row;
+            if (cls == 0) {
+                const uint32_t mcu = n >> 2, k = n & 3u;
+                blk = mcu * 6u + k;
+                row = &s_y[((k >> 1) * 8 + j) * kYStride + mcu * 16 + (k & 1u) * 8];
+            } else {
+                const uint32_t mcu = n & 31u, comp = n >> 5;
+                blk = mcu * 6u + 4u + comp;
+                row = (comp ? s_cr : s_cb) + j * kCStride + mcu * 8;
             }
+            float d[8];
+            {
+                const uint2 w = *reinterpret_cast<const uint2*>(row);
+                d[0] = float(w.x & 255u), d[1] = float((w.x >> 8) & 255u), d[2] = float((w.x >> 16) & 255u), d[3] = float(w.x >> 24);
+                d[4] = float(w.y & 255u), d[5] = float((w.y >> 8) & 255u), d[6] = float((w.y >> 16) & 255u), d[7] = float(w.y >> 24);
+            }
+            aan_fdct8(d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7]);      // row j of the block
+            *reinterpret_cast<float4*>(&scr[j * 8]) = make_float4(d[0], d[1], d[2], d[3]);
+            *reinterpret_cast<float4*>(&scr[j * 8 + 4]) = make_float4(d[4], d[5], d[6], d[7]);
+            __syncwarp();
+#pragma unroll
+            for (int i = 0; i < 8; ++i) d[i] = scr[i * 8 + j];
+            __syncwarp();
+            aan_fdct8(d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7]);      // column j: d[i] = coefficient (i, j)
+            int16_t* out = reinterpret_cast<int16_t*>(&s_out[blk * kOutStride]);
+            // rows of coefficients in which some lane of the warp may quantise to a non-zero value (|y| >= T <=> |w| >= 1 - 2G)
+            uint32_t lm = 0;
+#pragma unroll
+            for (int i = 0; i < 8; ++i) lm |= (fabsf(d[i]) >= T[i] ? 1u : 0u) << i;
+            const uint32_t wm = __reduce_or_sync(0xffffffffu, lm);
+            int qv[8];
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+                qv[i] = 0;
+                if (wm & (1u << i)) {
+                    const float w = d[i] * K[i];
+                    qv[i] = __float2int_rz(w);
+                    // distance of |w| to the nearest integer >= 1
+                    const float a = fabsf(w) - 0.5f;
+                    const float kf = (a + 12582912.0f) - 12582912.0f;      // rint(|w| - 0.5)
+                    const float delta = a - kf;                             // frac(|w|) - 0.5 in [-0.5, 0.5]
+                    if (fabsf(delta) > 0.5f - gQcol[cls][j].G[i] && fabsf(w) > 0.5f && (i | j) != 0)
+                        push_fix(&s_nfix, s_fix, (blk << 6) | uint32_t(i * 8 + j));
+                }
+            }
+            if (j == 0) {
+                // DC: the reference's sum is an exact integer (cos row 0 is 1.0), so its value is ((S*c)*c)/4 exactly as
+                // evaluated; level shift: the samples are stored as value + 128 (64 * 128, exact)
+                const double v = __dmul_rn(__dmul_rn(__dmul_rn(double(d[0] - 8192.0f), cC.inv_sqrt2_ref), cC.inv_sqrt2_ref), 0.25);
+                qv[0] = cls ? __double2int_rz(v) / 17 : __double2int_rz(v) / 16;
+            }
+#pragma unroll
+            for (int i = 0; i < 8; ++i) out[__byte_perm(i < 4 ? izz.x : izz.y, 0, 0x4440 + (i & 3))] = int16_t(qv[i]);
         }
-    } else
-    // ---- phase 2: DCT + quantisation, one thread per block (warps 0..3 luma, 4 Cb, 5 Cr) ----
-    if (warp < 6) {
-        // luma: warp 0 = top blocks of MCUs 0..15, warp 1 = bottom blocks of MCUs 0..15, warps 2/3 = MCUs 16..31,
-        // so that the 8-byte row loads of a half-warp are contiguous in the row-major tile
-        uint32_t blk;
-        const uint8_t* tile;
-        int stride;
-        if (warp < 4) {
-            const uint32_t mcu = (warp >> 1) * 16 + (lane >> 1), k = (warp & 1) * 2 + (lane & 1);
-            blk = mcu * 6 + k;
-            tile = &s_y[(warp & 1) * 8 * kYStride + mcu * 16 + (lane & 1) * 8];
-            stride = kYStride;
-        } else {
-            blk = lane * 6 + warp;
-            tile = (warp == 4 ? s_cb : s_cr) + lane * 8;
-            stride = kCStride;
-        }
-        float d[64];
-#pragma unroll
-        for (int y = 0; y < 8; ++y) {
-            const uint2 w = *reinterpret_cast<const uint2*>(tile + y * stride);
-            d[y * 8 + 0] = float(w.x & 255u), d[y * 8 + 1] = float((w.x >> 8) & 255u);
-            d[y * 8 + 2] = float((w.x >> 16) & 255u), d[y * 8 + 3] = float(w.x >> 24);
-            d[y * 8 + 4] = float(w.y & 255u), d[y * 8 + 5] = float((w.y >> 8) & 255u);
-            d[y * 8 + 6] = float((w.y >> 16) & 255u), d[y * 8 + 7] = float(w.y >> 24);
-        }
-        // row pass: rows 2k and 2k+1 as packed pairs; column pass: columns 2k and 2k+1 as packed pairs
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            f32x2 q[8];
-#pragma unroll
-            for (int x = 0; x < 8; ++x) q[x] = pk2(d[(2 * k) * 8 + x], d[(2 * k + 1) * 8 + x]);
-            aan_fdct8_x2(q[0], q[1], q[2], q[3], q[4], q[5], q[6], q[7]);
-#pragma unroll
-            for (int x = 0; x < 8; ++x) unpk2(q[x], d[(2 * k) * 8 + x], d[(2 * k + 1) * 8 + x]);
-        }
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            f32x2 q[8];
-#pragma unroll
-            for (int y = 0; y < 8; ++y) q[y] = pk2(d[y * 8 + 2 * k], d[y * 8 + 2 * k + 1]);
-            aan_fdct8_x2(q[0], q[1], q[2], q[3], q[4], q[5], q[6], q[7]);
-#pragma unroll
-            for (int y = 0; y < 8; ++y) unpk2(q[y], d[y * 8 + 2 * k], d[y * 8 + 2 * k + 1]);
-        }
-        d[0] -= 8192.0f;   // level shift: the samples are stored as value + 128 (64 * 128, exact)
-        uint4* out16 = reinterpret_cast<uint4*>(&s_out[blk * kOutStride]);
-        if (warp < 4) quant_block<0>(d, blk, &s_nfix, s_fix, out16);
-        else quant_block<1>(d, blk, &s_nfix, s_fix, out16);
     }
     __syncthreads();
 

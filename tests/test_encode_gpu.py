@@ -50,17 +50,13 @@ def test_coefficients_bit_exact(ctx, oracle, W, H, family, gray):
 @pytest.mark.parametrize("W,H", [(64, 48), (208, 128), (512, 512), (1920, 16), (4080, 48), (1024, 272)])
 @pytest.mark.parametrize("family", [0, 1, 2])
 @pytest.mark.parametrize("gray", [False, True])
-def test_second_generation_forward_kernel_bit_exact(ctx, oracle, W, H, family, gray):
-    """JPEZYB200_OPT_TRANSFORM = 3: the persistent, bulk-copy fed forward kernel (enc_transform2.cuh; rows must be 16-byte aligned).
-    An A/B variant since it lost to the production kernel on batches (DESIGN.md 7) -- and held to the same bar."""
+def test_forward_kernel_16_byte_row_loads_bit_exact(ctx, oracle, W, H, family, gray):
+    """widths that are multiples of 16 take the 16-byte row loads of the production forward kernel: coefficients and scan
+    bit-exact on whole and partial 32-MCU tiles and on frames of one MCU row (1920x16)."""
     r, g, b = planes(family, W, H)
     want = oracle.coefs(r, g, b, W, H, gray=gray)
-    ctx.set_option(capi.OPT_TRANSFORM, 3)
-    try:
-        got = gpu_coefs(ctx, r, g, b, W, H, gray=gray)[0]
-        scan, _ = ctx.encode(r, g, b, W, H, gray=gray)
-    finally:
-        ctx.set_option(capi.OPT_TRANSFORM, 0)
+    got = gpu_coefs(ctx, r, g, b, W, H, gray=gray)[0]
+    scan, _ = ctx.encode(r, g, b, W, H, gray=gray)
     assert (want == got).all(), "%d coefficients differ" % int((want != got).sum())
     assert scan == oracle.encode(r, g, b, W, H, gray=gray, scan_only=True)
 
@@ -174,6 +170,15 @@ def test_pad_policy(ctx, oracle, pad_ones):
     finally:
         ctx.set_option(capi.OPT_PAD_ONES, 1)
     assert got[0] == oracle.scan_from_coefs(coefs, pad_ones=bool(pad_ones))
+
+
+@pytest.mark.parametrize("value", [2, 3, -1])
+def test_transform_option_takes_only_production_or_validation(ctx, value):
+    with pytest.raises(capi.JpezyError) as e:
+        ctx.set_option(capi.OPT_TRANSFORM, value)
+    assert e.value.code == capi.EINVAL
+    for ok in (1, 0):
+        ctx.set_option(capi.OPT_TRANSFORM, ok)
 
 
 @pytest.mark.parametrize("W,H,family,gray", [(200, 120, 0, False), (512, 512, 0, False), (512, 512, 1, False), (96, 80, 2, True),

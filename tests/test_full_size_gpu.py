@@ -42,20 +42,6 @@ def test_full_size_byte_and_sample_parity(ctx, oracle, name, W, H, gray, family)
 
 
 @pytest.mark.parametrize("family", [0, 1])
-def test_full_size_second_generation_forward_kernel(ctx, oracle, family):
-    # the A/B forward kernel (JPEZYB200_OPT_TRANSFORM = 3) on a whole 4K frame: same file, S-photo and S-noise
-    W, H = 3840, 2160
-    d = synth_dev(ctx, W, H, family=family)
-    r, g, b = (d[c].cpu().numpy() for c in range(3))
-    ctx.set_option(capi.OPT_TRANSFORM, 3)
-    try:
-        scan, nbits = ctx.encode(r, g, b, W, H)
-    finally:
-        ctx.set_option(capi.OPT_TRANSFORM, 0)
-    assert hashlib.sha256(scan).hexdigest() == hashlib.sha256(oracle.encode(r, g, b, W, H, scan_only=True)).hexdigest()
-
-
-@pytest.mark.parametrize("family", [0, 1])
 def test_full_size_one_chain_per_guess(ctx, oracle, family):
     # the latency form of the first synchronisation launch (JPEZYB200_OPT_SYNC_GUESSES = 1) on a whole 4K frame
     W, H = 3840, 2160

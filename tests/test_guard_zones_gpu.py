@@ -13,16 +13,18 @@ GUARD = 4096
 
 
 class Guarded:
-    """n bytes of `dtype` elements with GUARD poisoned bytes on either side (the payload stays 256-byte aligned)"""
-    def __init__(self, nelem, dtype, fill=0):
+    """n bytes of `dtype` elements with GUARD poisoned bytes on either side (the payload starts `offset` bytes past a 256-byte
+    boundary)"""
+    def __init__(self, nelem, dtype, fill=0, offset=0):
         self.esz = torch.empty(0, dtype=dtype).element_size()
         self.n = nelem * self.esz
-        self.raw = torch.full((GUARD + self.n + GUARD,), 0xA5, dtype=torch.uint8, device="cuda")
-        self.view = self.raw[GUARD: GUARD + self.n].view(dtype)
+        self.lo = GUARD + offset
+        self.raw = torch.full((self.lo + self.n + GUARD,), 0xA5, dtype=torch.uint8, device="cuda")
+        self.view = self.raw[self.lo: self.lo + self.n].view(dtype)
         self.view.fill_(fill)
 
     def intact(self):
-        return bool((self.raw[:GUARD] == 0xA5).all().item()) and bool((self.raw[GUARD + self.n:] == 0xA5).all().item())
+        return bool((self.raw[:self.lo] == 0xA5).all().item()) and bool((self.raw[self.lo + self.n:] == 0xA5).all().item())
 
 
 @pytest.mark.parametrize("W,H,family,gray,nimg", [(208, 128, 0, False, 1), (1920, 1080, 0, False, 2), (200, 120, 1, False, 3),
@@ -72,6 +74,32 @@ def test_device_entry_points_stay_inside_their_buffers(ctx, W, H, family, gray, 
     for name, gbuf in [("planes_in", planes_in[0]), ("planes_in", planes_in[1]), ("planes_in", planes_in[2]), ("coefs", coefs), ("coefs2", coefs2),
                        ("scan", scan), ("nbytes", nbytes), ("nbits", nbits), ("status", status), ("out", out[0]), ("out", out[1]), ("out", out[2])]:
         assert gbuf.intact(), "guard zone around %s was written" % name
+
+
+def test_unaligned_planes_take_the_first_generation_inverse_kernel(ctx):
+    """4:2:0 output planes that start 1 byte past a 256-byte boundary (coefficients aligned) go to k_inv_transform, the 4:2:0
+    kernel that needs no 16-byte aligned buffers: the planes equal those of the aligned call and the guard zones stay intact.
+    (W is not a multiple of 16: that kernel stores whole 16-byte rows of an MCU when it is.)"""
+    W, H, nimg = 200, 120, 2
+    frame = J.default_frame(W, H)
+    pl = capi.plane_bytes(frame)
+    nm = capi.num_mcus(W, H)
+    sp = torch.cuda.current_stream().cuda_stream
+    planes_in = [Guarded(nimg * W * H, torch.uint8) for _ in range(3)]
+    coefs = Guarded(nimg * nm * 384, torch.int16)
+    ctx.synth_dev(planes_in[0].view, planes_in[1].view, planes_in[2].view, W, H, nimg=nimg, first_frame=7, family=1, stream=sp)
+    ctx.transform_fwd_dev(planes_in[0].view, planes_in[1].view, planes_in[2].view, W, H, nimg, False, coefs.view, stream=sp)
+    outs = []
+    for offset in (0, 1):
+        out = [Guarded(nimg * pl, torch.uint8, fill=0x44, offset=offset) for _ in range(3)]
+        ctx.transform_inv_dev(coefs.view, frame, nimg, False, out[0].view, out[1].view, out[2].view, pl, stream=sp)
+        torch.cuda.synchronize()
+        for o in out:
+            assert o.intact(), "guard zone around an output plane was written (offset %d)" % offset
+        outs.append([o.view.clone() for o in out])
+    assert coefs.intact()
+    for a, b in zip(*outs):
+        assert torch.equal(a, b), "%d samples differ between the unaligned and the aligned planes" % int((a != b).sum())
 
 
 LAYOUTS = {"444": ((1, 1, 1), (1, 1, 1)), "422": ((2, 1, 1), (1, 1, 1)), "440": ((1, 1, 1), (2, 1, 1)), "gray1": ((1,), (1,))}

@@ -9,8 +9,7 @@ import jpezy_b200 as J
 from jpezy_b200 import shard
 
 ctx = J.Context(0)
-# (sizes with 16-byte aligned rows take the second-generation transform kernels -- TMA bulk copies, mbarriers, warp-specialised
-# pipeline --, the others the first-generation ones; S-noise fills the guard-band queues)
+# (the inverse transform takes the second-generation kernel -- TMA bulk copy, mbarrier --; S-noise fills the guard-band queues)
 for fam, W, H, gray in ((0, 208, 128, False), (1, 64, 48, False), (2, 17, 33, True), (1, 640, 360, False), (0, 1, 1, False),
                         (0, 1920, 1080, False), (1, 320, 200, True)):
     r, g, b = J.synth.image(fam, W, H)

@@ -21,7 +21,7 @@ def main():
     ap.add_argument("--family", type=int, default=0)
     ap.add_argument("--gray", action="store_true")
     ap.add_argument("--iters", type=int, default=50)
-    ap.add_argument("--variant", type=int, default=0, help="JPEZYB200_OPT_TRANSFORM")
+    ap.add_argument("--variant", type=int, default=0, choices=[0, 1], help="JPEZYB200_OPT_TRANSFORM: 0 production, 1 FP64 validation kernels")
     ap.add_argument("--guesses", type=int, default=0, help="JPEZYB200_OPT_SYNC_GUESSES")
     ap.add_argument("--lib", default="", help="A/B runs: another build of libjpezy_b200.so to load instead of the in-tree one")
     a = ap.parse_args()
@@ -84,7 +84,7 @@ def main():
     except Exception:
         pass
     print(json.dumps({"stage": a.stage, "W": W, "H": H, "batch": B, "family": a.family, "gray": gray, "variant": a.variant, "lib": os.path.basename(a.lib),
-                      "tile": os.environ.get("JPEZY_B200_FWD_TILE", ""), "us_per_launch": round(us, 2), "GBs": round(gbs, 1),
+                      "us_per_launch": round(us, 2), "GBs": round(gbs, 1),
                       "frac_of_measured_peak": round(gbs / peak, 4), "guard_fwd": ctx.stat(capi.STAT_GUARD_FWD),
                       "sync_iters": [ctx.stat(capi.STAT_SYNC_ITERS0), ctx.stat(capi.STAT_SYNC_ITERS1)], "sync_rounds": ctx.stat(capi.STAT_SYNC_ROUNDS)}))
 
