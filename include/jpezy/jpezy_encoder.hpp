@@ -15,6 +15,10 @@
 
 namespace jpezy {
 
+// encode<MODE>(file, optimize_huffman): Huffman tables fitted to the image instead of the Annex K tables
+struct optimize_huffman_t {};
+inline constexpr optimize_huffman_t optimize_huffman{};
+
 template <class T>
 struct encoder {
     static_assert(sizeof(T) == 1, "8-bit samples");
@@ -51,6 +55,43 @@ struct encoder {
             }
             s.resize(head + nbytes);
         }
+        {
+            raii_messenger mes("Write EOI ...");
+            jpeg.write_eoi();
+        }
+        jpeg.output_file();
+        return jpeg.wrote_size();
+    }
+
+    // The same file with optimised Huffman tables (jpezyb200_encode_optimized): the tables exist only after the encode, so the
+    // segment is encoded first, then the header with the tables' DHT segments, the segment and EOI are written.
+    template <class MODE_TAG = COLOR_MODE>
+    std::size_t encode(const char* output_file, optimize_huffman_t)
+    {
+        const std::size_t W = pr.get<property::At::HSize>(), H = pr.get<property::At::VSize>();
+        std::size_t size = W * H * 3;
+        if (size < 10240) size = 10240;
+        jpezy_writer jpeg(size, pr, output_file);
+        if (!jpeg) throw std::runtime_error(__func__);
+        std::vector<byte> scan(size);
+        std::size_t nbytes = 0;
+        jpezyb200_huff ht[2][2];
+        {
+            raii_messenger mes("Encoding ...");
+            if (r.size() < W * H || g.size() < W * H || b.size() < W * H) throw std::runtime_error("encode: planes smaller than width*height");
+            const int rc = jpezyb200_encode_optimized(b200::runtime::ctx(), reinterpret_cast<const std::uint8_t*>(r.data()),
+                                                      reinterpret_cast<const std::uint8_t*>(g.data()), reinterpret_cast<const std::uint8_t*>(b.data()),
+                                                      static_cast<std::uint32_t>(W), static_cast<std::uint32_t>(H),
+                                                      std::is_same_v<MODE_TAG, GRAY_MODE> ? 1 : 0, scan.data(), scan.size(), &nbytes, nullptr, ht);
+            if (rc != JPEZYB200_OK) throw b200::runtime::error("encode", rc);
+        }
+        {
+            raii_messenger mes("Write JPEG Header ...");
+            jpeg.write_header(ht);
+        }
+        jpezy_writer::stream_type& s = jpeg.get_stream();
+        if (s.size() + nbytes + 2 > jpeg.capacity()) throw std::runtime_error("jpezy_writer: buffer overflow");
+        s.insert(s.end(), scan.begin(), scan.begin() + std::ptrdiff_t(nbytes));
         {
             raii_messenger mes("Write EOI ...");
             jpeg.write_eoi();

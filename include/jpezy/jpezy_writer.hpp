@@ -6,10 +6,12 @@
 #define JPEZY_B200_JPEZY_WRITER_HPP
 
 #include <cstdio>
+#include <initializer_list>
 #include <stdexcept>
 #include <string>
 #include <vector>
 
+#include "../jpezy_b200.h"
 #include "jpezy.hpp"
 
 namespace jpezy {
@@ -76,33 +78,22 @@ struct jpezy_writer {
     }
 
     // src/encoder/jpezy_writer.hpp:20-94, byte for byte (644 bytes for the 16-character comments jpezy uses)
-    void write_header()
+    void write_header() { write_header_with({&tables::YDcDht, &tables::CDcDht, &tables::YAcDht, &tables::CAcDht}); }
+
+    // the same header with the four DHT segments carrying the tables of an optimised encode ([0=DC,1=AC][0=luma,1=chroma],
+    // jpezyb200_encode_optimized) instead of the Annex K tables: same segments in the same order, lengths from the tables
+    void write_header(const jpezyb200_huff (&ht)[2][2])
     {
-        if (!fp) throw std::runtime_error(__func__);
-        marker(MARKER::SOI);
-        marker(MARKER::APP0), word(16), bytes("JFIF", 5), word(0x0102), put(static_cast<int>(pr.get<property::At::Units>()));
-        word(pr.get<property::At::HDensity>()), word(pr.get<property::At::VDensity>());
-        put(pr.get<property::At::HThumbnail>()), put(pr.get<property::At::VThumbnail>());
-        if (const std::string& c = pr.get<property::At::Comment>(); !c.empty()) {
-            marker(MARKER::COM), word(static_cast<unsigned>(c.size() + 3)), bytes(c.c_str(), c.size() + 1);
+        tables::dht_spec d[4];
+        const unsigned char tc_th[4] = {0x00, 0x01, 0x10, 0x11};
+        for (int k = 0; k < 4; ++k) {
+            const jpezyb200_huff& h = ht[tc_th[k] >> 4][tc_th[k] & 1];
+            d[k].tc_th = tc_th[k];
+            d[k].nvals = 0;
+            for (int i = 0; i < 16; ++i) d[k].bits[i] = h.bits[i], d[k].nvals += h.bits[i];
+            d[k].vals = h.vals;
         }
-        marker(MARKER::DQT), word(67), put(0);
-        for (int i = 0; i < 64; ++i) put(tables::YQuantumTb[tables::ZZ[i]]);
-        marker(MARKER::DQT), word(67), put(1);
-        for (int i = 0; i < 64; ++i) put(tables::CQuantumTb[tables::ZZ[i]]);
-        for (const tables::dht_spec* d : {&tables::YDcDht, &tables::CDcDht, &tables::YAcDht, &tables::CAcDht}) {
-            marker(MARKER::DHT), word(2 + 1 + 16 + d->nvals), put(d->tc_th);
-            for (unsigned char b : d->bits) put(b);
-            for (int i = 0; i < d->nvals; ++i) put(d->vals[i]);
-        }
-        const int dim = pr.get<property::At::Dimension>();
-        marker(MARKER::SOF0), word(3 * dim + 8), put(pr.get<property::At::SamplePrecision>());
-        word(static_cast<unsigned>(pr.get<property::At::VSize>())), word(static_cast<unsigned>(pr.get<property::At::HSize>())), put(dim);
-        put(0), put(0x22), put(0);
-        for (int i = 1; i < 3; ++i) put(i), put(0x11), put(1);
-        marker(MARKER::SOS), word(2 * dim + 6), put(dim);
-        for (int i = 0; i < dim; ++i) put(i), put(i == 0 ? 0 : 0x11);
-        put(0), put(63), put(0);
+        write_header_with({&d[0], &d[1], &d[2], &d[3]});
     }
 
     stream_type& get_stream() noexcept { return buf; }
@@ -122,6 +113,35 @@ struct jpezy_writer {
     explicit operator bool() const noexcept { return fp != nullptr; }
 
 private:
+    void write_header_with(std::initializer_list<const tables::dht_spec*> dhts)
+    {
+        if (!fp) throw std::runtime_error(__func__);
+        marker(MARKER::SOI);
+        marker(MARKER::APP0), word(16), bytes("JFIF", 5), word(0x0102), put(static_cast<int>(pr.get<property::At::Units>()));
+        word(pr.get<property::At::HDensity>()), word(pr.get<property::At::VDensity>());
+        put(pr.get<property::At::HThumbnail>()), put(pr.get<property::At::VThumbnail>());
+        if (const std::string& c = pr.get<property::At::Comment>(); !c.empty()) {
+            marker(MARKER::COM), word(static_cast<unsigned>(c.size() + 3)), bytes(c.c_str(), c.size() + 1);
+        }
+        marker(MARKER::DQT), word(67), put(0);
+        for (int i = 0; i < 64; ++i) put(tables::YQuantumTb[tables::ZZ[i]]);
+        marker(MARKER::DQT), word(67), put(1);
+        for (int i = 0; i < 64; ++i) put(tables::CQuantumTb[tables::ZZ[i]]);
+        for (const tables::dht_spec* d : dhts) {
+            marker(MARKER::DHT), word(2 + 1 + 16 + d->nvals), put(d->tc_th);
+            for (unsigned char b : d->bits) put(b);
+            for (int i = 0; i < d->nvals; ++i) put(d->vals[i]);
+        }
+        const int dim = pr.get<property::At::Dimension>();
+        marker(MARKER::SOF0), word(3 * dim + 8), put(pr.get<property::At::SamplePrecision>());
+        word(static_cast<unsigned>(pr.get<property::At::VSize>())), word(static_cast<unsigned>(pr.get<property::At::HSize>())), put(dim);
+        put(0), put(0x22), put(0);
+        for (int i = 1; i < 3; ++i) put(i), put(0x11), put(1);
+        marker(MARKER::SOS), word(2 * dim + 6), put(dim);
+        for (int i = 0; i < dim; ++i) put(i), put(i == 0 ? 0 : 0x11);
+        put(0), put(63), put(0);
+    }
+
     void put(int v)
     {
         if (buf.size() >= cap) throw std::runtime_error("jpezy_writer: buffer overflow");

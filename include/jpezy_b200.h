@@ -131,6 +131,35 @@ JPEZYB200_API int jpezyb200_read_sizes(jpezyb200_ctx* ctx, const uint64_t* d_val
 JPEZYB200_API int jpezyb200_encode_batch(jpezyb200_ctx* ctx, const uint8_t* r, const uint8_t* g, const uint8_t* b, uint32_t W, uint32_t H,
                            uint32_t nimg, int gray, uint8_t* scan_out, size_t slot_bytes, uint64_t* scan_bytes);
 
+/* One Huffman table as a DHT segment carries it: written by the optimised encoders below, read by the decoders. */
+typedef struct jpezyb200_huff {
+    uint8_t present;
+    uint8_t bits[16];   /* number of codes of length 1..16 (DHT, src/decoder/jpezy_decoder.hpp:208-211) */
+    uint8_t vals[256];  /* symbol values in code order (:240)                                         */
+} jpezyb200_huff;
+
+/* Optimised Huffman tables (the counterpart of libjpeg's -optimize; the reference has none).  The same encodes as
+ * jpezyb200_encode, jpezyb200_encode_batch_dev and jpezyb200_entropy_encode_dev, but every image is coded with Huffman
+ * tables fitted to its own symbol counts (T.81 section K.2, code lengths limited to 16, no all-1-bits code word) instead
+ * of the Annex K tables K.3-K.6: the same coefficients and decoded pixels in a smaller segment.  The counts and the
+ * tables are computed on the device; nothing waits for the host in between.
+ *
+ * ht / d_ht: [class 0=DC,1=AC][0=luma (Y), 1=chroma (Cb and Cr)] records with present = 1.  They take the place of the
+ * DHT contents that the host writer emits from the Annex K tables (write_header, src/encoder/jpezy_writer.hpp:20-94,
+ * src/encoder/huffman_table.hpp): copy them into the file's four DHT segments to write it, and into
+ * jpezyb200_frame.ht[c][i] (jpezyb200_default_frame's td = {0,1,1}) to decode it.  d_ht is a device array of
+ * [nimg][2][2] records.  jpezyb200_encode_optimized reads the sizes and the tables back in one copy; it synchronises
+ * as often as jpezyb200_encode.  The MCU-row sharded encoders and jpezyb200_encode_batch have no optimised form. */
+JPEZYB200_API int jpezyb200_encode_optimized(jpezyb200_ctx* ctx, const uint8_t* r, const uint8_t* g, const uint8_t* b, uint32_t W,
+                               uint32_t H, int gray, uint8_t* scan_out, size_t scan_cap, size_t* scan_bytes, uint64_t* scan_bits,
+                               jpezyb200_huff ht[2][2]);
+JPEZYB200_API int jpezyb200_encode_batch_optimized_dev(jpezyb200_ctx* ctx, const uint8_t* d_r, const uint8_t* d_g, const uint8_t* d_b,
+                               uint32_t W, uint32_t H, uint32_t nimg, int gray, uint8_t* d_scan, size_t slot_bytes,
+                               uint64_t* d_scan_bytes, uint64_t* d_scan_bits, jpezyb200_huff* d_ht, void* stream);
+JPEZYB200_API int jpezyb200_entropy_encode_optimized_dev(jpezyb200_ctx* ctx, const int16_t* d_coefs, uint32_t W, uint32_t H,
+                               uint32_t nimg, int gray, uint8_t* d_scan, size_t slot_bytes, uint64_t* d_scan_bytes,
+                               uint64_t* d_scan_bits, jpezyb200_huff* d_ht, void* stream);
+
 /* Stage E1+E2 only: planar RGB -> quantised coefficients, int16, zig-zag order
  * (src/jpezy.hpp:36-45), block order Y0 Y1 Y2 Y3 Cb Cr per MCU, MCUs row-major
  * (src/encoder/jpezy_encoder.hpp:227-242).  d_coefs holds nimg * num_mcus * 6 * 64 int16. */
@@ -151,12 +180,6 @@ JPEZYB200_API int jpezyb200_entropy_encode_dev(jpezyb200_ctx* ctx, const int16_t
  * (srook::io::jpeg::bifstream, call sites :589,612,634).  Marker parsing (:171-502) stays on the
  * host and hands its result over in jpezyb200_frame.
  * ---------------------------------------------------------------------------------------------- */
-typedef struct jpezyb200_huff {
-    uint8_t present;
-    uint8_t bits[16];   /* number of codes of length 1..16 (DHT, src/decoder/jpezy_decoder.hpp:208-211) */
-    uint8_t vals[256];  /* symbol values in code order (:240)                                         */
-} jpezyb200_huff;
-
 typedef struct jpezyb200_frame {
     uint32_t width, height;        /* SOF0 (src/decoder/jpezy_decoder.hpp:286-289)                    */
     uint8_t sample_precision;      /* 8                                                               */

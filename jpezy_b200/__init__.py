@@ -8,9 +8,9 @@ PyTorch only supplies device memory, streams and torch.distributed.
 There is no CPU path: importing works anywhere (so the build can be checked on a CPU box), but
 creating a Context without the library or without a CUDA device raises.
 """
-from .capi import (Context, Frame, JpezyError, abi_version, build_library, default_frame, library_path, load_library,  # noqa: F401
-                   plane_bytes)
+from .capi import (Context, Frame, HuffTables, JpezyError, abi_version, build_library, default_frame, huff_tables,  # noqa: F401
+                   library_path, load_library, optimized_frame, plane_bytes)
 from . import synth  # noqa: F401
 
-__all__ = ["Context", "Frame", "JpezyError", "abi_version", "build_library", "default_frame", "library_path",
-           "load_library", "plane_bytes", "synth"]
+__all__ = ["Context", "Frame", "HuffTables", "JpezyError", "abi_version", "build_library", "default_frame", "huff_tables",
+           "library_path", "load_library", "optimized_frame", "plane_bytes", "synth"]

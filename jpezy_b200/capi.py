@@ -19,7 +19,8 @@ EXPORTS = [
     "jpezyb200_shard_encode_c", "jpezyb200_shard_encode_d", "jpezyb200_ipc_alloc", "jpezyb200_ipc_open", "jpezyb200_ipc_close",
     "jpezyb200_ipc_free", "jpezyb200_shard_decode_dev", "jpezyb200_encode_batch", "jpezyb200_decode_batch", "jpezyb200_read_sizes",
     "jpezyb200_group_create", "jpezyb200_group_destroy", "jpezyb200_group_size", "jpezyb200_group_last_error", "jpezyb200_group_ctx",
-    "jpezyb200_group_partition", "jpezyb200_group_encode",
+    "jpezyb200_group_partition", "jpezyb200_group_encode", "jpezyb200_encode_optimized", "jpezyb200_encode_batch_optimized_dev",
+    "jpezyb200_entropy_encode_optimized_dev",
 ]
 
 
@@ -31,6 +32,10 @@ class JpezyError(RuntimeError):
 
 class Huff(C.Structure):
     _fields_ = [("present", C.c_uint8), ("bits", C.c_uint8 * 16), ("vals", C.c_uint8 * 256)]
+
+
+HuffTables = (Huff * 2) * 2   # [class 0=DC,1=AC][0=luma, 1=chroma], as the optimised encoders write them
+HUFF_TABLES_BYTES = C.sizeof(HuffTables)
 
 
 class Frame(C.Structure):
@@ -75,6 +80,10 @@ def load_library():
     L.jpezyb200_get_stat.argtypes = [vp, C.c_int, C.POINTER(C.c_uint64)]
     L.jpezyb200_encode.argtypes = [vp, u8p, u8p, u8p, u32, u32, C.c_int, u8p, sz, C.POINTER(sz), C.POINTER(C.c_uint64)]
     L.jpezyb200_encode_batch_dev.argtypes = [vp, u8p, u8p, u8p, u32, u32, u32, C.c_int, u8p, sz, u64p, u64p, vp]
+    L.jpezyb200_encode_optimized.argtypes = [vp, u8p, u8p, u8p, u32, u32, C.c_int, u8p, sz, C.POINTER(sz), C.POINTER(C.c_uint64),
+                                             C.POINTER(HuffTables)]
+    L.jpezyb200_encode_batch_optimized_dev.argtypes = [vp, u8p, u8p, u8p, u32, u32, u32, C.c_int, u8p, sz, u64p, u64p, vp, vp]
+    L.jpezyb200_entropy_encode_optimized_dev.argtypes = [vp, i16p, u32, u32, u32, C.c_int, u8p, sz, u64p, u64p, vp, vp]
     L.jpezyb200_transform_fwd_dev.argtypes = [vp, u8p, u8p, u8p, u32, u32, u32, C.c_int, i16p, vp]
     L.jpezyb200_read_sizes.argtypes = [vp, u64p, u32, u64p, vp]
     L.jpezyb200_entropy_encode_dev.argtypes = [vp, i16p, u32, u32, u32, C.c_int, u8p, sz, u64p, u64p, vp]
@@ -112,6 +121,26 @@ def default_frame(W, H):
     rc = load_library().jpezyb200_default_frame(W, H, C.byref(f))
     if rc:
         raise JpezyError(rc, "default_frame")
+    return f
+
+
+def huff_tables(data):
+    """HuffTables from the HUFF_TABLES_BYTES bytes of one image's records (e.g. a slice of d_ht copied to the host)"""
+    if isinstance(data, HuffTables):
+        return data
+    if hasattr(data, "cpu"):
+        data = data.cpu().numpy()
+    return HuffTables.from_buffer_copy(bytes(memoryview(data).cast("B")))
+
+
+def optimized_frame(W, H, ht):
+    """default_frame(W, H) with the Huffman tables an optimised encode returned (HuffTables or its bytes): the frame
+    descriptor that decodes that image"""
+    f = default_frame(W, H)
+    ht = huff_tables(ht)
+    for c in range(2):
+        for i in range(2):
+            f.ht[c][i] = ht[c][i]
     return f
 
 
@@ -182,6 +211,17 @@ class Context:
                                             C.byref(nb)))
         return out[: n.value].tobytes(), nb.value
 
+    def encode_optimized(self, r, g, b, W, H, gray=False, scan_cap=None):
+        """encode with Huffman tables fitted to the image -> (segment, bit count, HuffTables)"""
+        import numpy as np
+        r, g, b = (np.ascontiguousarray(x, dtype=np.uint8).reshape(-1) for x in (r, g, b))
+        cap = int(scan_cap if scan_cap is not None else max(W * H * 3, 10240))
+        out = np.empty(cap, dtype=np.uint8)
+        n, nb, ht = C.c_size_t(0), C.c_uint64(0), HuffTables()
+        self._chk(self.lib.jpezyb200_encode_optimized(self.h, _dp(r), _dp(g), _dp(b), W, H, int(gray), _dp(out), cap, C.byref(n),
+                                                      C.byref(nb), C.byref(ht)))
+        return out[: n.value].tobytes(), nb.value, ht
+
     def decode(self, scan, frame, gray=False):
         import numpy as np
         a = np.frombuffer(scan, dtype=np.uint8)
@@ -195,6 +235,12 @@ class Context:
         self._chk(self.lib.jpezyb200_encode_batch_dev(self.h, _dp(d_r), _dp(d_g), _dp(d_b), W, H, nimg, int(gray), _dp(d_scan),
                                                       slot_bytes, _dp(d_bytes), _dp(d_bits), stream))
 
+    def encode_batch_optimized_dev(self, d_r, d_g, d_b, W, H, nimg, gray, d_scan, slot_bytes, d_ht, d_bytes=None, d_bits=None,
+                                   stream=None):
+        """d_ht: device buffer of nimg * HUFF_TABLES_BYTES bytes, the tables of image i at i * HUFF_TABLES_BYTES"""
+        self._chk(self.lib.jpezyb200_encode_batch_optimized_dev(self.h, _dp(d_r), _dp(d_g), _dp(d_b), W, H, nimg, int(gray),
+                                                                _dp(d_scan), slot_bytes, _dp(d_bytes), _dp(d_bits), _dp(d_ht), stream))
+
     def read_sizes(self, d_values, n, h_out, stream=None):
         """n uint64 values of a device array into the numpy uint64 array h_out; returns when `stream` has reached this point"""
         self._chk(self.lib.jpezyb200_read_sizes(self.h, _dp(d_values), n, _dp(h_out), stream))
@@ -206,6 +252,11 @@ class Context:
     def entropy_encode_dev(self, d_coefs, W, H, nimg, gray, d_scan, slot_bytes, d_bytes=None, d_bits=None, stream=None):
         self._chk(self.lib.jpezyb200_entropy_encode_dev(self.h, _dp(d_coefs), W, H, nimg, int(gray), _dp(d_scan), slot_bytes,
                                                         _dp(d_bytes), _dp(d_bits), stream))
+
+    def entropy_encode_optimized_dev(self, d_coefs, W, H, nimg, gray, d_scan, slot_bytes, d_ht, d_bytes=None, d_bits=None,
+                                     stream=None):
+        self._chk(self.lib.jpezyb200_entropy_encode_optimized_dev(self.h, _dp(d_coefs), W, H, nimg, int(gray), _dp(d_scan), slot_bytes,
+                                                                  _dp(d_bytes), _dp(d_bits), _dp(d_ht), stream))
 
     def decode_batch_dev(self, d_scan, slot_bytes, h_scan_bytes, nimg, frame, gray, d_r, d_g, d_b, plane_len, d_status=None,
                          stream=None):

@@ -15,6 +15,7 @@
 #include "dec_transform2.cuh"
 #include "dec_transform_g.cuh"
 #include "enc_entropy.cuh"
+#include "enc_huffopt.cuh"
 #include "enc_transform.cuh"
 #include "enc_shard.cuh"
 #include "synth.cuh"
@@ -165,7 +166,7 @@ void jpezyb200_ctx_destroy(jpezyb200_ctx* ctx)
     jz_devbuf* bufs[] = {&ctx->coefs, &ctx->blk_off, &ctx->tile_sum, &ctx->tile_base, &ctx->img_bits, &ctx->ustream,
                          &ctx->ff_sum, &ctx->ff_base, &ctx->planes_in, &ctx->planes_out, &ctx->scan_io, &ctx->sizes_io,
                          &ctx->dec_scanbytes, &ctx->dec_chunk_cnt, &ctx->dec_chunk_base, &ctx->dec_ubytes, &ctx->dec_state,
-                         &ctx->dec_dirty, &ctx->dec_subblk, &ctx->dec_dc, &ctx->dec_dcd, &ctx->blk_meta, &ctx->dec_status, &ctx->dec_changed, &ctx->dec_flags, &ctx->inv_samples, &ctx->shard_geom, &ctx->dec_mcnt, &ctx->dec_mbase, &ctx->dec_seg};
+                         &ctx->dec_dirty, &ctx->dec_subblk, &ctx->dec_dc, &ctx->dec_dcd, &ctx->blk_meta, &ctx->dec_status, &ctx->dec_changed, &ctx->dec_flags, &ctx->inv_samples, &ctx->shard_geom, &ctx->dec_mcnt, &ctx->dec_mbase, &ctx->dec_seg, &ctx->sym_hist, &ctx->huff_lut};
     for (jz_devbuf* b : bufs)
         if (b->p) cudaFree(b->p);
     if (ctx->d_enc_lut) cudaFree(ctx->d_enc_lut);
@@ -181,6 +182,7 @@ void jpezyb200_ctx_destroy(jpezyb200_ctx* ctx)
     if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
     if (ctx->h_sizes) cudaFreeHost(ctx->h_sizes);
     if (ctx->h_words) cudaFreeHost(ctx->h_words);
+    if (ctx->h_huff) cudaFreeHost(ctx->h_huff);
     if (ctx->aux_stream) cudaStreamSynchronize(ctx->aux_stream), cudaStreamDestroy(ctx->aux_stream);
     if (ctx->aux_fork) cudaEventDestroy(ctx->aux_fork);
     if (ctx->aux_join) cudaEventDestroy(ctx->aux_join);
@@ -290,8 +292,10 @@ static int launch_fwd(jpezyb200_ctx* ctx, const uint8_t* d_r, const uint8_t* d_g
 
 static size_t round_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// d_ht != nullptr: code every image with its own optimised tables (enc_huffopt.cuh) and write them to d_ht[nimg][2][2]
 static int launch_entropy(jpezyb200_ctx* ctx, const int16_t* d_coefs, uint32_t W, uint32_t H, uint32_t nimg, uint8_t* d_scan,
-                          size_t slot_bytes, uint64_t* d_scan_bytes, uint64_t* d_scan_bits, cudaStream_t st, bool with_meta = false)
+                          size_t slot_bytes, uint64_t* d_scan_bytes, uint64_t* d_scan_bits, cudaStream_t st, bool with_meta = false,
+                          jpezyb200_huff* d_ht = nullptr)
 {
     const uint32_t HU = mcu_units(W), VU = mcu_units(H);
     const size_t nmcu = size_t(HU) * VU;
@@ -327,6 +331,20 @@ static int launch_entropy(jpezyb200_ctx* ctx, const int16_t* d_coefs, uint32_t W
     p.ff_sum = static_cast<uint32_t*>(ctx->ff_sum.p);
     p.ff_base = static_cast<uint64_t*>(ctx->ff_base.p);
 
+    if (d_ht) {
+        const size_t hist_bytes = size_t(nimg) * 2 * kHistBins * sizeof(unsigned long long);
+        const bool fresh = hist_bytes > ctx->sym_hist.cap;
+        if ((rc = ctx->ensure(ctx->sym_hist, hist_bytes))) return rc;
+        if (fresh) JZ_CUDA_TRY(ctx, cudaMemsetAsync(ctx->sym_hist.p, 0, ctx->sym_hist.cap, st));   // k_huff_build keeps it zeroed
+        if ((rc = ctx->ensure(ctx->huff_lut, size_t(nimg) * 2 * sizeof(HuffEncLut)))) return rc;
+        unsigned long long* counts = static_cast<unsigned long long*>(ctx->sym_hist.p);
+        HuffEncLut* lut = static_cast<HuffEncLut*>(ctx->huff_lut.p);
+        (void)jz_launch(k_sym_hist, dim3(p.ntile, nimg), dim3(kEntThreads), 0, st, p, counts);
+        (void)jz_launch(k_huff_build, dim3(nimg), dim3(128), 0, st, counts, lut, d_ht);
+        ctx->launches += 2;
+        p.lut = lut;
+        p.lut_stride = 2;
+    }
     (void)jz_launch(k_block_bits, dim3(p.ntile, nimg), dim3(kEntThreads), 0, st, p);
     (void)jz_launch(k_scan_tiles, dim3(nimg), dim3(1024), 0, st, p);
     // grid-stride helpers: enough CTAs to fill the machine, split evenly over the images
@@ -421,6 +439,73 @@ int jpezyb200_encode(jpezyb200_ctx* ctx, const uint8_t* r, const uint8_t* g, con
     if (h_sz[0] == ~0ull || h_sz[0] > scan_cap) return ctx->fail(JPEZYB200_ECAPACITY, "entropy-coded segment does not fit in scan_cap");
     JZ_CUDA_TRY(ctx, cudaMemcpyAsync(scan_out, ctx->scan_io.p, h_sz[0], cudaMemcpyDeviceToHost, st));
     JZ_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    *scan_bytes = size_t(h_sz[0]);
+    if (scan_bits) *scan_bits = h_sz[1];
+    return JPEZYB200_OK;
+}
+
+int jpezyb200_entropy_encode_optimized_dev(jpezyb200_ctx* ctx, const int16_t* d_coefs, uint32_t W, uint32_t H, uint32_t nimg, int gray,
+                                           uint8_t* d_scan, size_t slot_bytes, uint64_t* d_scan_bytes, uint64_t* d_scan_bits,
+                                           jpezyb200_huff* d_ht, void* stream)
+{
+    (void)gray;
+    int rc = check_geometry(ctx, W, H, nimg);
+    if (rc) return rc;
+    if (!d_coefs || !d_scan || !d_ht || slot_bytes == 0) return ctx->fail(JPEZYB200_EINVAL, "null pointer / empty slot");
+    JZ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return launch_entropy(ctx, d_coefs, W, H, nimg, d_scan, slot_bytes, d_scan_bytes, d_scan_bits, pick_stream(ctx, stream), false, d_ht);
+}
+
+int jpezyb200_encode_batch_optimized_dev(jpezyb200_ctx* ctx, const uint8_t* d_r, const uint8_t* d_g, const uint8_t* d_b, uint32_t W,
+                                         uint32_t H, uint32_t nimg, int gray, uint8_t* d_scan, size_t slot_bytes, uint64_t* d_scan_bytes,
+                                         uint64_t* d_scan_bits, jpezyb200_huff* d_ht, void* stream)
+{
+    int rc = check_geometry(ctx, W, H, nimg);
+    if (rc) return rc;
+    if (!d_r || !d_g || !d_b || !d_scan || !d_ht || slot_bytes == 0) return ctx->fail(JPEZYB200_EINVAL, "null pointer / empty slot");
+    JZ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const size_t ncoef = size_t(mcu_units(W)) * mcu_units(H) * 384 * nimg;
+    if ((rc = ctx->ensure(ctx->coefs, ncoef * sizeof(int16_t)))) return rc;
+    cudaStream_t st = pick_stream(ctx, stream);
+    if ((rc = launch_fwd(ctx, d_r, d_g, d_b, W, H, nimg, gray, static_cast<int16_t*>(ctx->coefs.p), st, 0, 0, true))) return rc;
+    return launch_entropy(ctx, static_cast<int16_t*>(ctx->coefs.p), W, H, nimg, d_scan, slot_bytes, d_scan_bytes, d_scan_bits, st, true,
+                          d_ht);
+}
+
+int jpezyb200_encode_optimized(jpezyb200_ctx* ctx, const uint8_t* r, const uint8_t* g, const uint8_t* b, uint32_t W, uint32_t H, int gray,
+                               uint8_t* scan_out, size_t scan_cap, size_t* scan_bytes, uint64_t* scan_bits, jpezyb200_huff ht[2][2])
+{
+    int rc = check_geometry(ctx, W, H, 1);
+    if (rc) return rc;
+    if (!r || !g || !b || !scan_out || !scan_bytes || !ht || scan_cap == 0) return ctx->fail(JPEZYB200_EINVAL, "null pointer / empty buffer");
+    JZ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    // sizes (2 words) and the four table records side by side: one device-to-host copy before the segment's
+    constexpr size_t kHuffReadback = 16 + 4 * sizeof(jpezyb200_huff);
+    const size_t npx = size_t(W) * H;
+    const uint32_t HU = mcu_units(W), VU = mcu_units(H);
+    if ((rc = ctx->ensure(ctx->planes_in, 3 * npx))) return rc;
+    if ((rc = ctx->ensure(ctx->scan_io, scan_cap))) return rc;
+    if ((rc = ctx->ensure(ctx->sizes_io, kHuffReadback))) return rc;
+    if ((rc = ctx->ensure(ctx->coefs, size_t(HU) * VU * 384 * sizeof(int16_t)))) return rc;
+    uint8_t* d_in = static_cast<uint8_t*>(ctx->planes_in.p);
+    uint64_t* d_sz = static_cast<uint64_t*>(ctx->sizes_io.p);
+    jpezyb200_huff* d_ht = reinterpret_cast<jpezyb200_huff*>(d_sz + 2);
+    int16_t* d_coefs = static_cast<int16_t*>(ctx->coefs.p);
+    if (!ctx->h_huff) JZ_CUDA_TRY(ctx, cudaMallocHost(&ctx->h_huff, kHuffReadback));
+    cudaStream_t st = ctx->stream;
+    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in, r, npx, cudaMemcpyHostToDevice, st));
+    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + npx, g, npx, cudaMemcpyHostToDevice, st));
+    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + 2 * npx, b, npx, cudaMemcpyHostToDevice, st));
+    if ((rc = launch_fwd(ctx, d_in, d_in + npx, d_in + 2 * npx, W, H, 1, gray, d_coefs, st, 0, 0, true))) return rc;
+    if ((rc = launch_entropy(ctx, d_coefs, W, H, 1, static_cast<uint8_t*>(ctx->scan_io.p), scan_cap, d_sz, d_sz + 1, st, true, d_ht))) return rc;
+    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_huff, d_sz, kHuffReadback, cudaMemcpyDeviceToHost, st));
+    JZ_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    uint64_t h_sz[2];
+    std::memcpy(h_sz, ctx->h_huff, sizeof h_sz);
+    if (h_sz[0] == ~0ull || h_sz[0] > scan_cap) return ctx->fail(JPEZYB200_ECAPACITY, "entropy-coded segment does not fit in scan_cap");
+    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(scan_out, ctx->scan_io.p, h_sz[0], cudaMemcpyDeviceToHost, st));
+    JZ_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    std::memcpy(&ht[0][0], static_cast<const uint8_t*>(ctx->h_huff) + 16, 4 * sizeof(jpezyb200_huff));
     *scan_bytes = size_t(h_sz[0]);
     if (scan_bits) *scan_bits = h_sz[1];
     return JPEZYB200_OK;

@@ -128,11 +128,13 @@ struct jpezyb200_ctx {
     // scratch
     jz_devbuf coefs, blk_off, tile_sum, tile_base, img_bits, ustream, ff_sum, ff_base, planes_in, planes_out, scan_io, sizes_io;
     jz_devbuf dec_scanbytes, dec_chunk_cnt, dec_chunk_base, dec_ubytes, dec_state, dec_dirty, dec_subblk, dec_dc, dec_dcd, blk_meta, dec_status, dec_changed, dec_flags, dec_mcnt, dec_mbase, dec_seg;
+    jz_devbuf sym_hist, huff_lut;  // optimised Huffman tables (enc_huffopt.cuh): symbol counts (zeroed when allocated), [nimg][2] LUTs
     jz_devbuf shard_geom;      // ShardGeom + scratch of the MCU-row sharded encoder (enc_shard.cuh)
     void* batch_pipe = nullptr;    // streams, events and double buffers of the pipelined host batches (capi_batch.inc)
     void* shard_state = nullptr;   // host copy of the launch parameters between the phases (capi_shard.inc)
     uint64_t* h_sizes = nullptr;   // pinned, 8192 values (jpezyb200_read_sizes)
     uint64_t* h_words = nullptr;   // pinned, 8 words: sizes / status read back by jpezyb200_encode / jpezyb200_decode
+    void* h_huff = nullptr;        // pinned, kHuffReadback bytes: sizes + the four tables read back by jpezyb200_encode_optimized
     void* h_pinned = nullptr;
     size_t h_pinned_cap = 0;
 

@@ -34,7 +34,7 @@ struct EntParams {
     uint64_t* img_bytes;     // [nimg]         stuffed byte count
     uint8_t* ustream;        // [nimg][uslot]  un-stuffed stream
     size_t uslot;            // bytes per image in ustream (multiple of 16)
-    const HuffEncLut* lut;   // [2]
+    const HuffEncLut* lut;   // [2], or [nimg][2] with lut_stride = 2
     const int32_t* dc_init;  // [nimg][3] predictors of the first blocks (nullptr = 0), shards
     int pad_ones;
     // stuffing
@@ -45,6 +45,7 @@ struct EntParams {
     size_t slot;
     uint64_t* out_bytes;     // [nimg] or nullptr
     uint64_t* out_bits;      // [nimg] or nullptr
+    uint32_t lut_stride;     // HuffEncLut per image: 0 = every image reads lut[0..1], 2 = per-image tables (enc_huffopt.cuh)
 };
 
 // index of the previous block of the same component in scan order, or -1
@@ -180,7 +181,7 @@ __global__ void __launch_bounds__(kEntThreads) k_block_bits(const EntParams p)
     __shared__ uint32_t s_ac[2][256];
     __shared__ uint32_t s_dc[2][16];
     __shared__ uint32_t s_warp[kEntThreads / 32];
-    load_lut(p.lut, s_ac, s_dc);
+    load_lut(p.lut + blockIdx.y * p.lut_stride, s_ac, s_dc);
     __syncthreads();
     const size_t img = blockIdx.y;
     const uint32_t b = blockIdx.x * kEntThreads + threadIdx.x;
@@ -258,7 +259,7 @@ __global__ void __launch_bounds__(kEntThreads) k_scatter(const EntParams p)
     pdl_wait();
     __shared__ uint32_t s_ac[2][256];
     __shared__ uint32_t s_dc[2][16];
-    load_lut(p.lut, s_ac, s_dc);
+    load_lut(p.lut + blockIdx.y * p.lut_stride, s_ac, s_dc);
     __syncthreads();
     const size_t img = blockIdx.y;
     const uint32_t b = blockIdx.x * kEntThreads + threadIdx.x;
