@@ -19,6 +19,7 @@
 #include "enc_transform.cuh"
 #include "enc_shard.cuh"
 #include "synth.cuh"
+#include "context.h"
 
 namespace jz {
 
@@ -50,7 +51,6 @@ static void build_enc_lut(const HuffSpec& dc, const HuffSpec& ac, HuffEncLut* ou
 }
 
 static cudaStream_t pick_stream(jpezyb200_ctx* ctx, void* s) { return s ? static_cast<cudaStream_t>(s) : ctx->stream; }
-static void batch_pipe_destroy(jpezyb200_ctx* ctx);
 
 }  // namespace jz
 
@@ -97,6 +97,11 @@ int jpezyb200_ctx_create(int device, jpezyb200_ctx** out)
     if (const char* e = std::getenv("JPEZY_B200_DEC_HYP")) ctx->sync_guesses = std::max(0, std::min(2, std::atoi(e)));      // (JPEZYB200_OPT_SYNC_GUESSES of every new context)      // (debugging: JPEZYB200_OPT_SYNC_ROUNDS of every new context)
     int rc = [&]() -> int {
         JZ_CUDA_TRY(ctx, cudaSetDevice(device));
+        // static + dynamic shared memory of these kernels exceed 48 KiB: opt in once per context
+        JZ_CUDA_TRY(ctx, cudaFuncSetAttribute(k_fwd_transform, cudaFuncAttributeMaxDynamicSharedMemorySize, kFwdTrSmem));
+        JZ_CUDA_TRY(ctx, cudaFuncSetAttribute(k_inv_transform, cudaFuncAttributeMaxDynamicSharedMemorySize, kInvSmem));
+        JZ_CUDA_TRY(ctx, cudaFuncSetAttribute(k_inv_transform2<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, Inv2<8>::kSmem));
+        JZ_CUDA_TRY(ctx, cudaFuncSetAttribute(k_idct_blocks, cudaFuncAttributeMaxDynamicSharedMemorySize, InvG::kSmem));
         JZ_CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
         DevConst h{};
         for (int i = 0; i < 64; ++i) {
@@ -162,32 +167,9 @@ void jpezyb200_ctx_destroy(jpezyb200_ctx* ctx)
 {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
-    if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-    jz_devbuf* bufs[] = {&ctx->coefs, &ctx->blk_off, &ctx->tile_sum, &ctx->tile_base, &ctx->img_bits, &ctx->ustream,
-                         &ctx->ff_sum, &ctx->ff_base, &ctx->planes_in, &ctx->planes_out, &ctx->scan_io, &ctx->sizes_io,
-                         &ctx->dec_scanbytes, &ctx->dec_chunk_cnt, &ctx->dec_chunk_base, &ctx->dec_ubytes, &ctx->dec_state,
-                         &ctx->dec_dirty, &ctx->dec_subblk, &ctx->dec_dc, &ctx->dec_dcd, &ctx->blk_meta, &ctx->dec_status, &ctx->dec_changed, &ctx->dec_flags, &ctx->inv_samples, &ctx->shard_geom, &ctx->dec_mcnt, &ctx->dec_mbase, &ctx->dec_seg, &ctx->sym_hist, &ctx->huff_lut};
-    for (jz_devbuf* b : bufs)
-        if (b->p) cudaFree(b->p);
-    if (ctx->d_enc_lut) cudaFree(ctx->d_enc_lut);
-    if (ctx->d_dec_lut) cudaFree(ctx->d_dec_lut);
-    if (ctx->d_counters) cudaFree(ctx->d_counters);
-    if (ctx->d_y_exact) cudaFree(ctx->d_y_exact);
-    for (void* tb : ctx->invg_tab)
-        if (tb) cudaFree(tb);
-    for (void* tb : ctx->inv2_tab)
-        if (tb) cudaFree(tb);
-    jz::batch_pipe_destroy(ctx);
-    std::free(ctx->shard_state);
-    if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
-    if (ctx->h_sizes) cudaFreeHost(ctx->h_sizes);
-    if (ctx->h_words) cudaFreeHost(ctx->h_words);
-    if (ctx->h_huff) cudaFreeHost(ctx->h_huff);
-    if (ctx->aux_stream) cudaStreamSynchronize(ctx->aux_stream), cudaStreamDestroy(ctx->aux_stream);
-    if (ctx->aux_fork) cudaEventDestroy(ctx->aux_fork);
-    if (ctx->aux_join) cudaEventDestroy(ctx->aux_join);
-    if (ctx->stream) cudaStreamDestroy(ctx->stream);
-    delete ctx;
+    for (cudaStream_t st : {ctx->stream, ctx->aux_stream, ctx->pipe.h2d, ctx->pipe.d2h})
+        if (st) cudaStreamSynchronize(st);
+    delete ctx;     // (the context's members release what they own)
 }
 
 int jpezyb200_set_option(jpezyb200_ctx* ctx, int option, int64_t value)
@@ -255,10 +237,6 @@ static int launch_fwd_kernel(jpezyb200_ctx* ctx, const FwdParams& p, uint32_t ni
         dim3 grid((p.HU + kMcuPerCta - 1) / kMcuPerCta, p.VU, nimg);
         k_fwd_transform_f64<<<grid, kFwdThreads, 0, st>>>(p);
     } else {
-        if (!ctx->fwd_attr_set) {   // static + dynamic shared memory exceed 48 KiB: opt in once per context
-            JZ_CUDA_TRY(ctx, cudaFuncSetAttribute(k_fwd_transform, cudaFuncAttributeMaxDynamicSharedMemorySize, kFwdTrSmem));
-            ctx->fwd_attr_set = true;
-        }
         (void)jz_launch(k_fwd_transform, dim3((p.HU + kTileMcu - 1) / kTileMcu, p.VU, nimg), dim3(256), kFwdTrSmem, st, p);
     }
     ++ctx->launches;
@@ -266,31 +244,52 @@ static int launch_fwd_kernel(jpezyb200_ctx* ctx, const FwdParams& p, uint32_t ni
     return JPEZYB200_OK;
 }
 
-// rows: MCU rows [row0, row0 + nrows) only (nrows == 0: all); the planes always hold the whole image
 static int launch_fwd(jpezyb200_ctx* ctx, const uint8_t* d_r, const uint8_t* d_g, const uint8_t* d_b, uint32_t W, uint32_t H,
-                      uint32_t nimg, int gray, int16_t* d_coefs, cudaStream_t st, uint32_t row0 = 0, uint32_t nrows = 0,
-                      bool with_meta = false)
+                      uint32_t nimg, int gray, int16_t* d_coefs, cudaStream_t st, bool with_meta = false)
 {
     FwdParams p{};
     p.r = d_r, p.g = d_g, p.b = d_b;
     p.plane_stride = size_t(W) * H;
     p.W = W, p.H = H;
-    p.HU = mcu_units(W), p.VU = nrows ? nrows : mcu_units(H);
-    p.coefs = d_coefs + size_t(row0) * p.HU * 384;
-    p.coef_stride = size_t(p.HU) * mcu_units(H) * 384;
-    p.row0 = row0, p.y_origin = 0;
+    p.HU = mcu_units(W), p.VU = mcu_units(H);
+    p.coefs = d_coefs;
+    p.coef_stride = size_t(p.HU) * p.VU * 384;
+    p.row0 = 0, p.y_origin = 0;
     p.gray = gray;
     p.guard_counter = ctx->d_counters + 0;
     p.y_exact = ctx->d_y_exact;
     if (with_meta && !ctx->fp64_transforms) {     // side information for launch_entropy (same context, same images)
         int rc;
         if ((rc = ctx->ensure(ctx->blk_meta, size_t(nimg) * (p.coef_stride >> 6) * 4))) return rc;
-        p.bmeta = static_cast<uint32_t*>(ctx->blk_meta.p) + size_t(row0) * p.HU * 6;
+        p.bmeta = static_cast<uint32_t*>(ctx->blk_meta.p);
     }
     return launch_fwd_kernel(ctx, p, nimg, st);
 }
 
 static size_t round_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// the entropy coder's scratch for nimg images of p.nblk blocks, p.ntile tiles, p.uslot un-stuffed bytes and p.nchunk
+// stuffing chunks each; sets p's pointers to it
+static int ensure_entropy_scratch(jpezyb200_ctx* ctx, EntParams& p, uint32_t nimg)
+{
+    int rc;
+    if ((rc = ctx->ensure(ctx->blk_off, size_t(nimg) * p.nblk * 4))) return rc;
+    if ((rc = ctx->ensure(ctx->tile_sum, size_t(nimg) * p.ntile * 4))) return rc;
+    if ((rc = ctx->ensure(ctx->tile_base, size_t(nimg) * p.ntile * 8))) return rc;
+    if ((rc = ctx->ensure(ctx->img_bits, size_t(nimg) * 16))) return rc;
+    if ((rc = ctx->ensure(ctx->ustream, size_t(nimg) * p.uslot))) return rc;
+    if ((rc = ctx->ensure(ctx->ff_sum, size_t(nimg) * p.nchunk * 4))) return rc;
+    if ((rc = ctx->ensure(ctx->ff_base, size_t(nimg) * p.nchunk * 8))) return rc;
+    p.blk_off = static_cast<uint32_t*>(ctx->blk_off.p);
+    p.tile_sum = static_cast<uint32_t*>(ctx->tile_sum.p);
+    p.tile_base = static_cast<uint64_t*>(ctx->tile_base.p);
+    p.img_bits = static_cast<uint64_t*>(ctx->img_bits.p);
+    p.img_bytes = p.img_bits + nimg;
+    p.ustream = static_cast<uint8_t*>(ctx->ustream.p);
+    p.ff_sum = static_cast<uint32_t*>(ctx->ff_sum.p);
+    p.ff_base = static_cast<uint64_t*>(ctx->ff_base.p);
+    return JPEZYB200_OK;
+}
 
 // d_ht != nullptr: code every image with its own optimised tables (enc_huffopt.cuh) and write them to d_ht[nimg][2][2]
 static int launch_entropy(jpezyb200_ctx* ctx, const int16_t* d_coefs, uint32_t W, uint32_t H, uint32_t nimg, uint8_t* d_scan,
@@ -315,22 +314,7 @@ static int launch_entropy(jpezyb200_ctx* ctx, const int16_t* d_coefs, uint32_t W
     p.dc_init = nullptr;
     p.pad_ones = ctx->pad_ones;
     int rc;
-    if ((rc = ctx->ensure(ctx->blk_off, size_t(nimg) * p.nblk * 4))) return rc;
-    if ((rc = ctx->ensure(ctx->tile_sum, size_t(nimg) * p.ntile * 4))) return rc;
-    if ((rc = ctx->ensure(ctx->tile_base, size_t(nimg) * p.ntile * 8))) return rc;
-    if ((rc = ctx->ensure(ctx->img_bits, size_t(nimg) * 16))) return rc;
-    if ((rc = ctx->ensure(ctx->ustream, size_t(nimg) * p.uslot))) return rc;
-    if ((rc = ctx->ensure(ctx->ff_sum, size_t(nimg) * p.nchunk * 4))) return rc;
-    if ((rc = ctx->ensure(ctx->ff_base, size_t(nimg) * p.nchunk * 8))) return rc;
-    p.blk_off = static_cast<uint32_t*>(ctx->blk_off.p);
-    p.tile_sum = static_cast<uint32_t*>(ctx->tile_sum.p);
-    p.tile_base = static_cast<uint64_t*>(ctx->tile_base.p);
-    p.img_bits = static_cast<uint64_t*>(ctx->img_bits.p);
-    p.img_bytes = p.img_bits + nimg;
-    p.ustream = static_cast<uint8_t*>(ctx->ustream.p);
-    p.ff_sum = static_cast<uint32_t*>(ctx->ff_sum.p);
-    p.ff_base = static_cast<uint64_t*>(ctx->ff_base.p);
-
+    if ((rc = ensure_entropy_scratch(ctx, p, nimg))) return rc;
     if (d_ht) {
         const size_t hist_bytes = size_t(nimg) * 2 * kHistBins * sizeof(unsigned long long);
         const bool fresh = hist_bytes > ctx->sym_hist.cap;
@@ -359,16 +343,65 @@ static int launch_entropy(jpezyb200_ctx* ctx, const int16_t* d_coefs, uint32_t W
     return JPEZYB200_OK;
 }
 
+// the fused encode of nimg device images (d_ht: as launch_entropy)
+static int encode_dev(jpezyb200_ctx* ctx, const uint8_t* d_r, const uint8_t* d_g, const uint8_t* d_b, uint32_t W, uint32_t H, uint32_t nimg,
+                      int gray, uint8_t* d_scan, size_t slot_bytes, uint64_t* d_scan_bytes, uint64_t* d_scan_bits, cudaStream_t st,
+                      jpezyb200_huff* d_ht)
+{
+    int rc;
+    if ((rc = ctx->ensure(ctx->coefs, size_t(mcu_units(W)) * mcu_units(H) * 384 * nimg * sizeof(int16_t)))) return rc;
+    int16_t* d_coefs = static_cast<int16_t*>(ctx->coefs.p);
+    if ((rc = launch_fwd(ctx, d_r, d_g, d_b, W, H, nimg, gray, d_coefs, st, true))) return rc;
+    return launch_entropy(ctx, d_coefs, W, H, nimg, d_scan, slot_bytes, d_scan_bytes, d_scan_bits, st, true, d_ht);
+}
+
+// the encode of one host image on the context's stream; ht != nullptr: with optimised tables, read back into ht
+static int encode_host(jpezyb200_ctx* ctx, const uint8_t* r, const uint8_t* g, const uint8_t* b, uint32_t W, uint32_t H, int gray,
+                       uint8_t* scan_out, size_t scan_cap, size_t* scan_bytes, uint64_t* scan_bits, jpezyb200_huff (*ht)[2])
+{
+    // the sizes (2 words) and the four table records side by side: one device-to-host copy before the segment's
+    const size_t readback = 16 + (ht ? 4 * sizeof(jpezyb200_huff) : 0);
+    const size_t npx = size_t(W) * H;
+    int rc;
+    if ((rc = ctx->ensure(ctx->planes_in, 3 * npx))) return rc;
+    if ((rc = ctx->ensure(ctx->scan_io, scan_cap))) return rc;
+    if ((rc = ctx->ensure(ctx->sizes_io, readback))) return rc;
+    uint64_t* h;
+    if ((rc = ctx->readback(&h))) return rc;
+    uint8_t* d_in = static_cast<uint8_t*>(ctx->planes_in.p);
+    uint64_t* d_sz = static_cast<uint64_t*>(ctx->sizes_io.p);
+    cudaStream_t st = ctx->stream;
+    // (copies and transform on one stream: bands of MCU rows whose copies overlap the transform measured slower on a 4K frame,
+    // 6.23-6.49 GPix/s for 2-8 bands against 6.48 for one -- the round trip is bound by the PCIe copies)
+    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in, r, npx, cudaMemcpyHostToDevice, st));
+    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + npx, g, npx, cudaMemcpyHostToDevice, st));
+    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + 2 * npx, b, npx, cudaMemcpyHostToDevice, st));
+    if ((rc = encode_dev(ctx, d_in, d_in + npx, d_in + 2 * npx, W, H, 1, gray, static_cast<uint8_t*>(ctx->scan_io.p), scan_cap, d_sz, d_sz + 1,
+                         st, ht ? reinterpret_cast<jpezyb200_huff*>(d_sz + 2) : nullptr)))
+        return rc;
+    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(h, d_sz, readback, cudaMemcpyDeviceToHost, st));
+    JZ_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    if (h[0] == ~0ull || h[0] > scan_cap) return ctx->fail(JPEZYB200_ECAPACITY, "entropy-coded segment does not fit in scan_cap");
+    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(scan_out, ctx->scan_io.p, h[0], cudaMemcpyDeviceToHost, st));
+    JZ_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    if (ht) std::memcpy(&ht[0][0], h + 2, 4 * sizeof(jpezyb200_huff));
+    *scan_bytes = size_t(h[0]);
+    if (scan_bits) *scan_bits = h[1];
+    return JPEZYB200_OK;
+}
+
 int jpezyb200_read_sizes(jpezyb200_ctx* ctx, const uint64_t* d_values, uint32_t n, uint64_t* h_out, void* stream)
 {
     if (!ctx) return JPEZYB200_EINVAL;
-    if (!d_values || !h_out || n == 0 || n > 8192u) return ctx->fail(JPEZYB200_EINVAL, "null pointer / bad count");
+    if (!d_values || !h_out || n == 0 || n > jpezyb200_ctx::kReadbackWords) return ctx->fail(JPEZYB200_EINVAL, "null pointer / bad count");
     JZ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    if (!ctx->h_sizes) JZ_CUDA_TRY(ctx, cudaMallocHost(reinterpret_cast<void**>(&ctx->h_sizes), 8192 * sizeof(uint64_t)));
+    uint64_t* h;
+    int rc = ctx->readback(&h);
+    if (rc) return rc;
     cudaStream_t st = pick_stream(ctx, stream);
-    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_sizes, d_values, size_t(n) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(h, d_values, size_t(n) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
     JZ_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    std::memcpy(h_out, ctx->h_sizes, size_t(n) * sizeof(uint64_t));
+    std::memcpy(h_out, h, size_t(n) * sizeof(uint64_t));
     return JPEZYB200_OK;
 }
 
@@ -393,57 +426,6 @@ int jpezyb200_entropy_encode_dev(jpezyb200_ctx* ctx, const int16_t* d_coefs, uin
     return launch_entropy(ctx, d_coefs, W, H, nimg, d_scan, slot_bytes, d_scan_bytes, d_scan_bits, pick_stream(ctx, stream));
 }
 
-int jpezyb200_encode_batch_dev(jpezyb200_ctx* ctx, const uint8_t* d_r, const uint8_t* d_g, const uint8_t* d_b, uint32_t W,
-                               uint32_t H, uint32_t nimg, int gray, uint8_t* d_scan, size_t slot_bytes, uint64_t* d_scan_bytes,
-                               uint64_t* d_scan_bits, void* stream)
-{
-    int rc = check_geometry(ctx, W, H, nimg);
-    if (rc) return rc;
-    if (!d_r || !d_g || !d_b || !d_scan || slot_bytes == 0) return ctx->fail(JPEZYB200_EINVAL, "null pointer / empty slot");
-    JZ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t ncoef = size_t(mcu_units(W)) * mcu_units(H) * 384 * nimg;
-    if ((rc = ctx->ensure(ctx->coefs, ncoef * sizeof(int16_t)))) return rc;
-    cudaStream_t st = pick_stream(ctx, stream);
-    if ((rc = launch_fwd(ctx, d_r, d_g, d_b, W, H, nimg, gray, static_cast<int16_t*>(ctx->coefs.p), st, 0, 0, true))) return rc;
-    return launch_entropy(ctx, static_cast<int16_t*>(ctx->coefs.p), W, H, nimg, d_scan, slot_bytes, d_scan_bytes, d_scan_bits, st, true);
-}
-
-int jpezyb200_encode(jpezyb200_ctx* ctx, const uint8_t* r, const uint8_t* g, const uint8_t* b, uint32_t W, uint32_t H, int gray,
-                     uint8_t* scan_out, size_t scan_cap, size_t* scan_bytes, uint64_t* scan_bits)
-{
-    int rc = check_geometry(ctx, W, H, 1);
-    if (rc) return rc;
-    if (!r || !g || !b || !scan_out || !scan_bytes || scan_cap == 0) return ctx->fail(JPEZYB200_EINVAL, "null pointer / empty buffer");
-    JZ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t npx = size_t(W) * H;
-    const uint32_t HU = mcu_units(W), VU = mcu_units(H);
-    if ((rc = ctx->ensure(ctx->planes_in, 3 * npx))) return rc;
-    if ((rc = ctx->ensure(ctx->scan_io, scan_cap))) return rc;
-    if ((rc = ctx->ensure(ctx->sizes_io, 64))) return rc;
-    if ((rc = ctx->ensure(ctx->coefs, size_t(HU) * VU * 384 * sizeof(int16_t)))) return rc;
-    uint8_t* d_in = static_cast<uint8_t*>(ctx->planes_in.p);
-    uint64_t* d_sz = static_cast<uint64_t*>(ctx->sizes_io.p);
-    int16_t* d_coefs = static_cast<int16_t*>(ctx->coefs.p);
-    if (!ctx->h_words) JZ_CUDA_TRY(ctx, cudaMallocHost(reinterpret_cast<void**>(&ctx->h_words), 8 * sizeof(uint64_t)));
-    cudaStream_t st = ctx->stream;
-    // (copies and transform on one stream: bands of MCU rows whose copies overlap the transform measured slower on a 4K frame,
-    // 6.23-6.49 GPix/s for 2-8 bands against 6.48 for one -- the round trip is bound by the PCIe copies)
-    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in, r, npx, cudaMemcpyHostToDevice, st));
-    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + npx, g, npx, cudaMemcpyHostToDevice, st));
-    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + 2 * npx, b, npx, cudaMemcpyHostToDevice, st));
-    if ((rc = launch_fwd(ctx, d_in, d_in + npx, d_in + 2 * npx, W, H, 1, gray, d_coefs, st, 0, 0, true))) return rc;
-    if ((rc = launch_entropy(ctx, d_coefs, W, H, 1, static_cast<uint8_t*>(ctx->scan_io.p), scan_cap, d_sz, d_sz + 1, st, true))) return rc;
-    uint64_t* h_sz = ctx->h_words;
-    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(h_sz, d_sz, 2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    JZ_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    if (h_sz[0] == ~0ull || h_sz[0] > scan_cap) return ctx->fail(JPEZYB200_ECAPACITY, "entropy-coded segment does not fit in scan_cap");
-    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(scan_out, ctx->scan_io.p, h_sz[0], cudaMemcpyDeviceToHost, st));
-    JZ_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    *scan_bytes = size_t(h_sz[0]);
-    if (scan_bits) *scan_bits = h_sz[1];
-    return JPEZYB200_OK;
-}
-
 int jpezyb200_entropy_encode_optimized_dev(jpezyb200_ctx* ctx, const int16_t* d_coefs, uint32_t W, uint32_t H, uint32_t nimg, int gray,
                                            uint8_t* d_scan, size_t slot_bytes, uint64_t* d_scan_bytes, uint64_t* d_scan_bits,
                                            jpezyb200_huff* d_ht, void* stream)
@@ -456,6 +438,17 @@ int jpezyb200_entropy_encode_optimized_dev(jpezyb200_ctx* ctx, const int16_t* d_
     return launch_entropy(ctx, d_coefs, W, H, nimg, d_scan, slot_bytes, d_scan_bytes, d_scan_bits, pick_stream(ctx, stream), false, d_ht);
 }
 
+int jpezyb200_encode_batch_dev(jpezyb200_ctx* ctx, const uint8_t* d_r, const uint8_t* d_g, const uint8_t* d_b, uint32_t W,
+                               uint32_t H, uint32_t nimg, int gray, uint8_t* d_scan, size_t slot_bytes, uint64_t* d_scan_bytes,
+                               uint64_t* d_scan_bits, void* stream)
+{
+    int rc = check_geometry(ctx, W, H, nimg);
+    if (rc) return rc;
+    if (!d_r || !d_g || !d_b || !d_scan || slot_bytes == 0) return ctx->fail(JPEZYB200_EINVAL, "null pointer / empty slot");
+    JZ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return encode_dev(ctx, d_r, d_g, d_b, W, H, nimg, gray, d_scan, slot_bytes, d_scan_bytes, d_scan_bits, pick_stream(ctx, stream), nullptr);
+}
+
 int jpezyb200_encode_batch_optimized_dev(jpezyb200_ctx* ctx, const uint8_t* d_r, const uint8_t* d_g, const uint8_t* d_b, uint32_t W,
                                          uint32_t H, uint32_t nimg, int gray, uint8_t* d_scan, size_t slot_bytes, uint64_t* d_scan_bytes,
                                          uint64_t* d_scan_bits, jpezyb200_huff* d_ht, void* stream)
@@ -464,12 +457,17 @@ int jpezyb200_encode_batch_optimized_dev(jpezyb200_ctx* ctx, const uint8_t* d_r,
     if (rc) return rc;
     if (!d_r || !d_g || !d_b || !d_scan || !d_ht || slot_bytes == 0) return ctx->fail(JPEZYB200_EINVAL, "null pointer / empty slot");
     JZ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t ncoef = size_t(mcu_units(W)) * mcu_units(H) * 384 * nimg;
-    if ((rc = ctx->ensure(ctx->coefs, ncoef * sizeof(int16_t)))) return rc;
-    cudaStream_t st = pick_stream(ctx, stream);
-    if ((rc = launch_fwd(ctx, d_r, d_g, d_b, W, H, nimg, gray, static_cast<int16_t*>(ctx->coefs.p), st, 0, 0, true))) return rc;
-    return launch_entropy(ctx, static_cast<int16_t*>(ctx->coefs.p), W, H, nimg, d_scan, slot_bytes, d_scan_bytes, d_scan_bits, st, true,
-                          d_ht);
+    return encode_dev(ctx, d_r, d_g, d_b, W, H, nimg, gray, d_scan, slot_bytes, d_scan_bytes, d_scan_bits, pick_stream(ctx, stream), d_ht);
+}
+
+int jpezyb200_encode(jpezyb200_ctx* ctx, const uint8_t* r, const uint8_t* g, const uint8_t* b, uint32_t W, uint32_t H, int gray,
+                     uint8_t* scan_out, size_t scan_cap, size_t* scan_bytes, uint64_t* scan_bits)
+{
+    int rc = check_geometry(ctx, W, H, 1);
+    if (rc) return rc;
+    if (!r || !g || !b || !scan_out || !scan_bytes || scan_cap == 0) return ctx->fail(JPEZYB200_EINVAL, "null pointer / empty buffer");
+    JZ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return encode_host(ctx, r, g, b, W, H, gray, scan_out, scan_cap, scan_bytes, scan_bits, nullptr);
 }
 
 int jpezyb200_encode_optimized(jpezyb200_ctx* ctx, const uint8_t* r, const uint8_t* g, const uint8_t* b, uint32_t W, uint32_t H, int gray,
@@ -479,36 +477,7 @@ int jpezyb200_encode_optimized(jpezyb200_ctx* ctx, const uint8_t* r, const uint8
     if (rc) return rc;
     if (!r || !g || !b || !scan_out || !scan_bytes || !ht || scan_cap == 0) return ctx->fail(JPEZYB200_EINVAL, "null pointer / empty buffer");
     JZ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    // sizes (2 words) and the four table records side by side: one device-to-host copy before the segment's
-    constexpr size_t kHuffReadback = 16 + 4 * sizeof(jpezyb200_huff);
-    const size_t npx = size_t(W) * H;
-    const uint32_t HU = mcu_units(W), VU = mcu_units(H);
-    if ((rc = ctx->ensure(ctx->planes_in, 3 * npx))) return rc;
-    if ((rc = ctx->ensure(ctx->scan_io, scan_cap))) return rc;
-    if ((rc = ctx->ensure(ctx->sizes_io, kHuffReadback))) return rc;
-    if ((rc = ctx->ensure(ctx->coefs, size_t(HU) * VU * 384 * sizeof(int16_t)))) return rc;
-    uint8_t* d_in = static_cast<uint8_t*>(ctx->planes_in.p);
-    uint64_t* d_sz = static_cast<uint64_t*>(ctx->sizes_io.p);
-    jpezyb200_huff* d_ht = reinterpret_cast<jpezyb200_huff*>(d_sz + 2);
-    int16_t* d_coefs = static_cast<int16_t*>(ctx->coefs.p);
-    if (!ctx->h_huff) JZ_CUDA_TRY(ctx, cudaMallocHost(&ctx->h_huff, kHuffReadback));
-    cudaStream_t st = ctx->stream;
-    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in, r, npx, cudaMemcpyHostToDevice, st));
-    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + npx, g, npx, cudaMemcpyHostToDevice, st));
-    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + 2 * npx, b, npx, cudaMemcpyHostToDevice, st));
-    if ((rc = launch_fwd(ctx, d_in, d_in + npx, d_in + 2 * npx, W, H, 1, gray, d_coefs, st, 0, 0, true))) return rc;
-    if ((rc = launch_entropy(ctx, d_coefs, W, H, 1, static_cast<uint8_t*>(ctx->scan_io.p), scan_cap, d_sz, d_sz + 1, st, true, d_ht))) return rc;
-    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_huff, d_sz, kHuffReadback, cudaMemcpyDeviceToHost, st));
-    JZ_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    uint64_t h_sz[2];
-    std::memcpy(h_sz, ctx->h_huff, sizeof h_sz);
-    if (h_sz[0] == ~0ull || h_sz[0] > scan_cap) return ctx->fail(JPEZYB200_ECAPACITY, "entropy-coded segment does not fit in scan_cap");
-    JZ_CUDA_TRY(ctx, cudaMemcpyAsync(scan_out, ctx->scan_io.p, h_sz[0], cudaMemcpyDeviceToHost, st));
-    JZ_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    std::memcpy(&ht[0][0], static_cast<const uint8_t*>(ctx->h_huff) + 16, 4 * sizeof(jpezyb200_huff));
-    *scan_bytes = size_t(h_sz[0]);
-    if (scan_bits) *scan_bits = h_sz[1];
-    return JPEZYB200_OK;
+    return encode_host(ctx, r, g, b, W, H, gray, scan_out, scan_cap, scan_bytes, scan_bits, ht);
 }
 
 // -------------------------------------------------------------------------------------------------
