@@ -1,6 +1,8 @@
 // include/jpezy/encode_io.hpp -- drop-in for jpezy::encode_io, to_jpeg, gray_scale (src/encoder/encode_io.hpp:33-209):
 //   jpezy::encode_io pnm("in.ppm");  ofs << (pnm | jpezy::to_jpeg("out.jpg"));  ofs << (pnm | to_jpeg(f) | jpezy::gray_scale);
-//   ofs << (pnm | jpezy::to_jpeg(f, jpezy::optimize_huffman)) writes the file with Huffman tables fitted to the image.
+//   ofs << (pnm | jpezy::to_jpeg(f, jpezy::optimize_huffman)) writes the file with Huffman tables fitted to the image,
+//   jpezy::to_jpeg(f, jpezy::restart_interval{n}) (or to_jpeg(f, optimize_huffman, restart_interval{n})) one with restart
+//   markers every n MCUs.
 // The P3 grammar is the reference's, quirks included (SURVEY.md appendix A.1): lines containing '#' are dropped wherever
 // they appear, the size line must split into exactly two tokens, maxval is parsed and ignored, a final line without a
 // newline is dropped, an interior empty token makes std::stoi throw std::invalid_argument.  One pass over the file
@@ -29,8 +31,12 @@ struct to_jpeg {
     explicit constexpr to_jpeg(const char* file_) : file(file_) {}
     // to_jpeg(f, optimize_huffman): the file carries Huffman tables fitted to the image instead of the Annex K tables
     constexpr to_jpeg(const char* file_, optimize_huffman_t) : file(file_), optimize(true) {}
+    // restart markers every rst.mcus MCUs (0 = none), with or without optimised tables
+    constexpr to_jpeg(const char* file_, restart_interval rst_) : file(file_), rst(rst_) {}
+    constexpr to_jpeg(const char* file_, optimize_huffman_t, restart_interval rst_) : file(file_), optimize(true), rst(rst_) {}
     const char* file;
     bool optimize = false;
+    restart_interval rst{};
 };
 struct gray_scale_t {};
 inline constexpr gray_scale_t gray_scale{};
@@ -205,7 +211,8 @@ private:
                                            .extension_code = property::ExtensionCodes::undefined, .decodable = property::Yet});
         auto [r, g, b] = pnm.second.split_rgb();
         encoder enc(pr, r, g, b);
-        const std::size_t size = pnm.first.optimize ? enc.encode<COLOR_MODE>(pnm.first.file, optimize_huffman) : enc.encode<COLOR_MODE>(pnm.first.file);
+        const std::size_t size = pnm.first.optimize ? enc.encode<COLOR_MODE>(pnm.first.file, optimize_huffman, pnm.first.rst)
+                                                    : enc.encode<COLOR_MODE>(pnm.first.file, pnm.first.rst);
         std::cout << "Output size: " << size << " byte" << std::endl;
         return ofs;
     }
@@ -218,8 +225,8 @@ private:
                           property::Units::dots_inch, 96, 96, 0, 0, property::ExtensionCodes::undefined};
         auto [r, g, b] = pnm.second.second.split_rgb();
         encoder enc(pr, r, g, b);
-        const std::size_t size = pnm.second.first.optimize ? enc.encode<GRAY_MODE>(pnm.second.first.file, optimize_huffman)
-                                                            : enc.encode<GRAY_MODE>(pnm.second.first.file);
+        const std::size_t size = pnm.second.first.optimize ? enc.encode<GRAY_MODE>(pnm.second.first.file, optimize_huffman, pnm.second.first.rst)
+                                                            : enc.encode<GRAY_MODE>(pnm.second.first.file, pnm.second.first.rst);
         std::cout << "Output size: " << size << " srook::byte" << std::endl;   // sic (:193)
         return ofs;
     }

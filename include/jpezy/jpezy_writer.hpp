@@ -77,12 +77,17 @@ struct jpezy_writer {
         if (fp) std::fclose(fp);
     }
 
-    // src/encoder/jpezy_writer.hpp:20-94, byte for byte (644 bytes for the 16-character comments jpezy uses)
-    void write_header() { write_header_with({&tables::YDcDht, &tables::CDcDht, &tables::YAcDht, &tables::CAcDht}); }
+    // src/encoder/jpezy_writer.hpp:20-94, byte for byte (644 bytes for the 16-character comments jpezy uses).  A non-zero
+    // restart_interval (MCUs, JPEZYB200_OPT_RESTART_INTERVAL of the encode) adds a DRI segment in front of SOS, where libjpeg
+    // writes it.
+    void write_header(unsigned restart_interval = 0)
+    {
+        write_header_with({&tables::YDcDht, &tables::CDcDht, &tables::YAcDht, &tables::CAcDht}, restart_interval);
+    }
 
     // the same header with the four DHT segments carrying the tables of an optimised encode ([0=DC,1=AC][0=luma,1=chroma],
     // jpezyb200_encode_optimized) instead of the Annex K tables: same segments in the same order, lengths from the tables
-    void write_header(const jpezyb200_huff (&ht)[2][2])
+    void write_header(const jpezyb200_huff (&ht)[2][2], unsigned restart_interval = 0)
     {
         tables::dht_spec d[4];
         const unsigned char tc_th[4] = {0x00, 0x01, 0x10, 0x11};
@@ -93,7 +98,7 @@ struct jpezy_writer {
             for (int i = 0; i < 16; ++i) d[k].bits[i] = h.bits[i], d[k].nvals += h.bits[i];
             d[k].vals = h.vals;
         }
-        write_header_with({&d[0], &d[1], &d[2], &d[3]});
+        write_header_with({&d[0], &d[1], &d[2], &d[3]}, restart_interval);
     }
 
     stream_type& get_stream() noexcept { return buf; }
@@ -113,9 +118,10 @@ struct jpezy_writer {
     explicit operator bool() const noexcept { return fp != nullptr; }
 
 private:
-    void write_header_with(std::initializer_list<const tables::dht_spec*> dhts)
+    void write_header_with(std::initializer_list<const tables::dht_spec*> dhts, unsigned restart_interval)
     {
         if (!fp) throw std::runtime_error(__func__);
+        if (restart_interval > 65535u) throw std::runtime_error("jpezy_writer: restart interval above 65535 MCUs");
         marker(MARKER::SOI);
         marker(MARKER::APP0), word(16), bytes("JFIF", 5), word(0x0102), put(static_cast<int>(pr.get<property::At::Units>()));
         word(pr.get<property::At::HDensity>()), word(pr.get<property::At::VDensity>());
@@ -137,6 +143,7 @@ private:
         word(static_cast<unsigned>(pr.get<property::At::VSize>())), word(static_cast<unsigned>(pr.get<property::At::HSize>())), put(dim);
         put(0), put(0x22), put(0);
         for (int i = 1; i < 3; ++i) put(i), put(0x11), put(1);
+        if (restart_interval) marker(MARKER::DRI), word(4), word(restart_interval);   // T.81 B.2.4.4
         marker(MARKER::SOS), word(2 * dim + 6), put(dim);
         for (int i = 0; i < dim; ++i) put(i), put(i == 0 ? 0 : 0x11);
         put(0), put(63), put(0);

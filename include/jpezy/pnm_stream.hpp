@@ -113,6 +113,7 @@ struct pnm_stream {
     pnm_stream() : initializing_succeed(true), width(0), height(0), max_color(0) {}
     pnm_stream(bool b, std::size_t w, std::size_t h, std::size_t max) : initializing_succeed(b), width(w), height(h), max_color(max) {}
     explicit operator bool() const noexcept { return initializing_succeed; }
+    std::size_t get_width() const noexcept { return width; }
 
 protected:
     typedef byte value_type;

@@ -73,11 +73,22 @@ enum {
                                      1 = on inputs too small to fill the device (a single frame) one chain per block position of
                                      the MCU, all at once: shortest latency of ONE decode (a 1080p frame: -11 %), six times the
                                      work -- with several decodes in flight on other contexts the default is faster */
-    JPEZYB200_OPT_SYNC_ROUNDS = 3 /* self-synchronisation launches enqueued after the first one by the
+    JPEZYB200_OPT_SYNC_ROUNDS = 3, /* self-synchronisation launches enqueued after the first one by the
                                      decoder: n > 0 = exactly n, no host round trip (default 3; the first launch checks
                                      the boundaries of its thread blocks itself, so on ordinary streams none of them has work and
                                      all return at once); 0 = the host polls a device flag after every launch until the fixed
                                      point */
+    JPEZYB200_OPT_RESTART_INTERVAL = 7 /* encoders: MCUs per restart interval, 0..65535 (other values: EINVAL); 0 (default) =
+                                     no restart markers.  Applies to every single-context encode: jpezyb200_encode,
+                                     _encode_batch, _encode_batch_dev, _entropy_encode_dev and the three *_optimized* forms.
+                                     The segment then holds the RSTn markers: interval i >= 1 is preceded by FF D((i-1) mod 8),
+                                     no marker follows the last one; every interval ends on a byte boundary padded as
+                                     JPEZYB200_OPT_PAD_ONES says, and its DC predictors start at 0 (T.81 F.1.2.3, E.1.4).
+                                     scan_bytes counts the stuffed bytes, markers included; scan_bits the Huffman-coded bits
+                                     only (no padding, no markers).  The file needs a DRI segment (FF DD 00 04 Ri) in front of
+                                     SOS (jpezy::jpezy_writer::write_header does that), and jpezyb200_frame.restart_interval to
+                                     decode it.  The MCU-row sharded encoders and jpezyb200_group_encode write restart-less
+                                     segments only: with a non-zero interval they return JPEZYB200_EUNSUPPORTED. */
 };
 JPEZYB200_API int jpezyb200_set_option(jpezyb200_ctx* ctx, int option, int64_t value);
 
@@ -149,7 +160,9 @@ typedef struct jpezyb200_huff {
  * src/encoder/huffman_table.hpp): copy them into the file's four DHT segments to write it, and into
  * jpezyb200_frame.ht[c][i] (jpezyb200_default_frame's td = {0,1,1}) to decode it.  d_ht is a device array of
  * [nimg][2][2] records.  jpezyb200_encode_optimized reads the sizes and the tables back in one copy; it synchronises
- * as often as jpezyb200_encode.  The MCU-row sharded encoders and jpezyb200_encode_batch have no optimised form. */
+ * as often as jpezyb200_encode.  The MCU-row sharded encoders and jpezyb200_encode_batch have no optimised form.
+ * With JPEZYB200_OPT_RESTART_INTERVAL set, the tables are fitted to the symbols of the restart stream (DC differences
+ * against predictors that restart at 0 in every interval). */
 JPEZYB200_API int jpezyb200_encode_optimized(jpezyb200_ctx* ctx, const uint8_t* r, const uint8_t* g, const uint8_t* b, uint32_t W,
                                uint32_t H, int gray, uint8_t* scan_out, size_t scan_cap, size_t* scan_bytes, uint64_t* scan_bits,
                                jpezyb200_huff ht[2][2]);
@@ -168,7 +181,7 @@ JPEZYB200_API int jpezyb200_transform_fwd_dev(jpezyb200_ctx* ctx, const uint8_t*
 
 /* Stage E3 only: coefficients (layout above) -> stuffed, padded entropy segment(s)
  * (src/encoder/jpezy_encoder.hpp:174-225).  Byte-identical to the reference given identical
- * coefficients. */
+ * coefficients (with JPEZYB200_OPT_RESTART_INTERVAL = 0). */
 JPEZYB200_API int jpezyb200_entropy_encode_dev(jpezyb200_ctx* ctx, const int16_t* d_coefs, uint32_t W, uint32_t H, uint32_t nimg,
                                  int gray, uint8_t* d_scan, size_t slot_bytes, uint64_t* d_scan_bytes,
                                  uint64_t* d_scan_bits, void* stream);
@@ -187,7 +200,8 @@ typedef struct jpezyb200_frame {
     uint8_t hs[3], vs[3], tq[3];   /* Frame_component H, V, Tq (src/decoder/tables.hpp:18-21); on the
                                       device: luma H, V in {1, 2}, chroma 1x1                         */
     uint8_t td[3], ta[3];          /* Scan_component Td, Ta (:23-26); the reference uses Td for both  */
-    uint16_t restart_interval;     /* DRI (src/decoder/jpezy_decoder.hpp:400-404); must be 0          */
+    uint16_t restart_interval;     /* DRI (src/decoder/jpezy_decoder.hpp:400-404): MCUs per restart
+                                      interval, 0 = none                                              */
     uint16_t qt[4][64];            /* natural order, as analyze_dqt stores them (:258-277)            */
     jpezyb200_huff ht[2][4];       /* [class 0=DC,1=AC][id]                                           */
 } jpezyb200_frame;

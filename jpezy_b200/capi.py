@@ -8,6 +8,7 @@ _LIB = None
 
 OK, EINVAL, ECAPACITY, ECUDA, ENCCL, ECORRUPT, ENODEVICE, ENOMEM, EUNSUPPORTED, EAGAIN = range(10)
 OPT_PAD_ONES, OPT_TRANSFORM, OPT_SYNC_ROUNDS, OPT_BATCH_GROUP_BYTES, OPT_SHARD_SCRATCH_BYTES, OPT_SYNC_GUESSES = 1, 2, 3, 4, 5, 6
+OPT_RESTART_INTERVAL = 7   # MCUs per restart interval of the encoders (0 = none); decode with Frame.restart_interval
 STAT_KERNEL_LAUNCHES, STAT_GUARD_FWD, STAT_GUARD_INV, STAT_SYNC_ROUNDS, STAT_SYNC_ITERS0, STAT_SYNC_ITERS1 = 1, 2, 3, 4, 5, 6
 
 EXPORTS = [

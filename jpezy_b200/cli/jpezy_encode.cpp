@@ -1,14 +1,18 @@
 // jpezy_encode -- drop-in for the reference's encoder CLI (src/encoder/main.cpp:56-116):
-//   jpezy_encode <input.ppm> ( <output.(jpeg | jpg)> [--optimize] [--gray] | <output.ppm> | --debug )
+//   jpezy_encode <input.ppm> ( <output.(jpeg | jpg)> [--optimize] [--gray] [--restart N[B]] | <output.ppm> | --debug )
 // Same argv sniffing (substring search after the first '.'), same console lines, same exit codes; the MCU loop runs on the
 // B200 through libjpezy_b200.so.  Unlike the reference, argv[3] is only looked at when it exists (:67-69 reads argv[argc]).
 // --optimize (not in the reference) writes Huffman tables fitted to the image instead of the Annex K tables.
+// --restart N (not in the reference) writes restart markers every N MCU rows, --restart NB every N MCUs, as cjpeg's -restart
+// does; 0 = none.  It may stand anywhere after the output name; the other arguments are read as if it were not there.
+#include <cstdint>
 #include <cstdlib>
 #include <fstream>
 #include <iostream>
 #include <optional>
 #include <stdexcept>
 #include <string_view>
+#include <vector>
 
 #include "jpezy/encode_io.hpp"
 
@@ -16,15 +20,35 @@ namespace {
 
 int disp_error()
 {
-    std::cerr << "Usage: jpezy_encode <input.ppm> ( <ouput.(jpeg | jpg) [OPT: --optimize] [OPT: --gray]> | <output.ppm> | --debug )" << std::endl;
+    std::cerr << "Usage: jpezy_encode <input.ppm> ( <ouput.(jpeg | jpg) [OPT: --optimize] [OPT: --gray] [OPT: --restart N[B]]> | <output.ppm> | --debug )"
+              << std::endl;
     return EXIT_FAILURE;
 }
 
 enum class Mode { JPEG, GRAY, PPM, DEBUG, UD };
 
-void exec(const jpezy::encode_io& pnm, const char* ofile, Mode m1, Mode m2, bool optimize)
+// --restart's value: N MCU rows or NB MCUs (decimal, at most 65535 either way)
+struct restart_arg {
+    unsigned long value = 0;
+    bool in_mcus = false;
+};
+
+bool parse_restart(std::string_view s, restart_arg& out)
 {
-    const jpezy::to_jpeg jpeg = optimize ? jpezy::to_jpeg(ofile, jpezy::optimize_huffman) : jpezy::to_jpeg(ofile);
+    if (!s.empty() && (s.back() == 'B' || s.back() == 'b')) out.in_mcus = true, s.remove_suffix(1);
+    if (s.empty() || s.size() > 5) return false;
+    out.value = 0;
+    for (char c : s) {
+        if (c < '0' || c > '9') return false;
+        out.value = out.value * 10 + unsigned(c - '0');
+    }
+    return out.value <= 65535;
+}
+
+void exec(const jpezy::encode_io& pnm, const char* ofile, Mode m1, Mode m2, bool optimize, unsigned restart)
+{
+    const jpezy::restart_interval rst{restart};
+    const jpezy::to_jpeg jpeg = optimize ? jpezy::to_jpeg(ofile, jpezy::optimize_huffman, rst) : jpezy::to_jpeg(ofile, rst);
     if (m2 == Mode::GRAY) {
         if (m1 != Mode::JPEG) throw std::invalid_argument("2nd Mode parameter must be GRAY");
         std::ofstream ofs(ofile, std::ios::binary);
@@ -49,8 +73,22 @@ void exec(const jpezy::encode_io& pnm, const char* ofile, Mode m1, Mode m2, bool
 
 }  // namespace
 
-int main(const int argc, const char* argv[])
+int main(int argc, const char* argv[])
 {
+    // take --restart <value> out of the arguments; the rest is read exactly as without it
+    std::vector<const char*> args(argv, argv + argc);
+    std::optional<restart_arg> restart;
+    for (std::size_t i = 3; i < args.size(); ++i) {
+        if (std::string_view(args[i]) != "--restart") continue;
+        restart_arg ra;
+        if (restart || i + 1 >= args.size() || !parse_restart(args[i + 1], ra)) return disp_error();
+        restart = ra;
+        args.erase(args.begin() + std::ptrdiff_t(i), args.begin() + std::ptrdiff_t(i) + 2);
+        --i;
+    }
+    argc = int(args.size());
+    args.push_back(nullptr);
+    argv = args.data();
     if (argc < 3) return disp_error();
     Mode m1 = Mode::UD, m2 = Mode::UD;
     bool optimize = false;
@@ -83,10 +121,17 @@ int main(const int argc, const char* argv[])
         std::cerr << "The file is not found or the formatting error" << std::endl;
         return disp_error();
     }
+    // the interval in MCUs: N rows are N * ceil(width / 16) MCUs
+    unsigned rst_mcus = 0;
+    if (restart) {
+        const std::uint64_t mcus = restart->in_mcus ? restart->value : restart->value * ((std::uint64_t(pnm.get_width()) + 15) / 16);
+        if (mcus > 65535) return disp_error();
+        rst_mcus = unsigned(mcus);
+    }
     auto t1 = section.stop();
     section.restart("Start encoding and writing ...");
     try {
-        exec(pnm, argv[2], m1, m2, optimize);
+        exec(pnm, argv[2], m1, m2, optimize, rst_mcus);
     } catch (const std::runtime_error& e) {
         std::cerr << e.what() << std::endl;
         return EXIT_FAILURE;

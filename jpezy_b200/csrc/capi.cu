@@ -177,6 +177,10 @@ int jpezyb200_set_option(jpezyb200_ctx* ctx, int option, int64_t value)
     if (!ctx) return JPEZYB200_EINVAL;
     switch (option) {
     case JPEZYB200_OPT_PAD_ONES: ctx->pad_ones = value ? 1 : 0; return JPEZYB200_OK;
+    case JPEZYB200_OPT_RESTART_INTERVAL:
+        if (value < 0 || value > 65535) return ctx->fail(JPEZYB200_EINVAL, "restart interval: 0 (none) or 1..65535 MCUs");
+        ctx->restart_interval = uint32_t(value);
+        return JPEZYB200_OK;
     case JPEZYB200_OPT_TRANSFORM:
         if (value != 0 && value != 1) return ctx->fail(JPEZYB200_EINVAL, "transform: 0 (production kernels) or 1 (FP64 validation kernels)");
         ctx->fp64_transforms = value == 1;
@@ -269,10 +273,14 @@ static int launch_fwd(jpezyb200_ctx* ctx, const uint8_t* d_r, const uint8_t* d_g
 static size_t round_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 // the entropy coder's scratch for nimg images of p.nblk blocks, p.ntile tiles, p.uslot un-stuffed bytes and p.nchunk
-// stuffing chunks each; sets p's pointers to it
-static int ensure_entropy_scratch(jpezyb200_ctx* ctx, EntParams& p, uint32_t nimg)
+// stuffing chunks each, and of r->nint restart intervals when r is given; sets p's (and r's) pointers to it
+static int ensure_entropy_scratch(jpezyb200_ctx* ctx, EntParams& p, uint32_t nimg, RstParams* r = nullptr)
 {
     int rc;
+    if (r) {
+        if ((rc = ctx->ensure(ctx->rst_base, size_t(nimg) * (size_t(r->nint) + 1) * 8))) return rc;
+        r->base = static_cast<uint64_t*>(ctx->rst_base.p);
+    }
     if ((rc = ctx->ensure(ctx->blk_off, size_t(nimg) * p.nblk * 4))) return rc;
     if ((rc = ctx->ensure(ctx->tile_sum, size_t(nimg) * p.ntile * 4))) return rc;
     if ((rc = ctx->ensure(ctx->tile_base, size_t(nimg) * p.ntile * 8))) return rc;
@@ -313,8 +321,12 @@ static int launch_entropy(jpezyb200_ctx* ctx, const int16_t* d_coefs, uint32_t W
     p.lut = ctx->d_enc_lut;
     p.dc_init = nullptr;
     p.pad_ones = ctx->pad_ones;
+    RstParams r{};
+    r.rst = ctx->restart_interval;
+    r.nint = r.rst ? uint32_t((nmcu + r.rst - 1) / r.rst) : 0;
+    const bool rst = r.rst != 0;
     int rc;
-    if ((rc = ensure_entropy_scratch(ctx, p, nimg))) return rc;
+    if ((rc = ensure_entropy_scratch(ctx, p, nimg, rst ? &r : nullptr))) return rc;
     if (d_ht) {
         const size_t hist_bytes = size_t(nimg) * 2 * kHistBins * sizeof(unsigned long long);
         const bool fresh = hist_bytes > ctx->sym_hist.cap;
@@ -323,21 +335,25 @@ static int launch_entropy(jpezyb200_ctx* ctx, const int16_t* d_coefs, uint32_t W
         if ((rc = ctx->ensure(ctx->huff_lut, size_t(nimg) * 2 * sizeof(HuffEncLut)))) return rc;
         unsigned long long* counts = static_cast<unsigned long long*>(ctx->sym_hist.p);
         HuffEncLut* lut = static_cast<HuffEncLut*>(ctx->huff_lut.p);
-        (void)jz_launch(k_sym_hist, dim3(p.ntile, nimg), dim3(kEntThreads), 0, st, p, counts);
+        (void)jz_launch(rst ? k_sym_hist<true> : k_sym_hist<false>, dim3(p.ntile, nimg), dim3(kEntThreads), 0, st, p, counts, r);
         (void)jz_launch(k_huff_build, dim3(nimg), dim3(128), 0, st, counts, lut, d_ht);
         ctx->launches += 2;
         p.lut = lut;
         p.lut_stride = 2;
     }
-    (void)jz_launch(k_block_bits, dim3(p.ntile, nimg), dim3(kEntThreads), 0, st, p);
+    (void)jz_launch(rst ? k_block_bits<true> : k_block_bits<false>, dim3(p.ntile, nimg), dim3(kEntThreads), 0, st, p, r);
     (void)jz_launch(k_scan_tiles, dim3(nimg), dim3(1024), 0, st, p);
+    if (rst) {
+        (void)jz_launch(k_rst_intervals, dim3(nimg), dim3(1024), 0, st, p, r);
+        ++ctx->launches;
+    }
     // grid-stride helpers: enough CTAs to fill the machine, split evenly over the images
     const uint32_t per_img = std::max<uint32_t>(1u, std::min<uint32_t>(p.nchunk, (uint32_t(ctx->num_sms) * 8u + nimg - 1) / nimg));
     (void)jz_launch(k_zero_ustream, dim3(per_img, nimg), dim3(256), 0, st, p);
-    (void)jz_launch(k_scatter, dim3(p.ntile, nimg), dim3(kEntThreads), 0, st, p);
+    (void)jz_launch(rst ? k_scatter<true> : k_scatter<false>, dim3(p.ntile, nimg), dim3(kEntThreads), 0, st, p, r);
     (void)jz_launch(k_ff_count, dim3(per_img, nimg), dim3(kStuffThreads), 0, st, p);
-    (void)jz_launch(k_scan_ff, dim3(nimg), dim3(1024), 0, st, p);
-    (void)jz_launch(k_stuff_write, dim3(per_img, nimg), dim3(kStuffThreads), 0, st, p);
+    (void)jz_launch(rst ? k_scan_ff<true> : k_scan_ff<false>, dim3(nimg), dim3(1024), 0, st, p, r);
+    (void)jz_launch(rst ? k_stuff_write<true> : k_stuff_write<false>, dim3(per_img, nimg), dim3(kStuffThreads), 0, st, p, r);
     ctx->launches += 7;
     JZ_CUDA_TRY(ctx, cudaGetLastError());
     return JPEZYB200_OK;

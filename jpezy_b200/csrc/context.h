@@ -84,6 +84,7 @@ struct jpezyb200_ctx {
     cudaEvent_t aux_fork = nullptr, aux_join = nullptr;
     std::string err;
     int pad_ones = 1;
+    uint32_t restart_interval = 0;   // JPEZYB200_OPT_RESTART_INTERVAL: MCUs per restart interval of the encoders, 0 = none
     bool fp64_transforms = false;   // JPEZYB200_OPT_TRANSFORM = 1: the FP64 validation kernels
     int sync_guesses = 0;     // JPEZYB200_OPT_SYNC_GUESSES
     int sync_rounds = 3;      // launches behind launch 0 (which checks the CTA boundaries itself): two that repair, one that verifies
@@ -107,6 +108,7 @@ struct jpezyb200_ctx {
     // scratch
     jz_devbuf coefs, blk_off, tile_sum, tile_base, img_bits, ustream, ff_sum, ff_base, planes_in, planes_out, scan_io, sizes_io;
     jz_devbuf dec_scanbytes, dec_chunk_cnt, dec_chunk_base, dec_ubytes, dec_state, dec_dirty, dec_subblk, dec_dc, dec_dcd, blk_meta, dec_status, dec_changed, dec_flags, dec_mcnt, dec_mbase, dec_seg;
+    jz_devbuf rst_base;        // [nimg][intervals + 1] byte bases of the restart intervals (enc_entropy.cuh)
     jz_devbuf sym_hist, huff_lut;  // optimised Huffman tables (enc_huffopt.cuh): symbol counts (zeroed when allocated), [nimg][2] LUTs
     jz_devbuf shard_geom;      // ShardGeom + scratch of the MCU-row sharded encoder (enc_shard.cuh)
     jz::BatchPipe pipe;

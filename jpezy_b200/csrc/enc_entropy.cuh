@@ -10,6 +10,15 @@
 //   E3c k_scatter      one thread per block: re-generate the code words and OR them into the
 //                      (zeroed) un-stuffed stream at the block's bit offset; pads the last byte
 //   E3d k_ff_count / k_scan_ff / k_stuff_write   count 0xFF bytes, scan, copy with 0x00 inserted
+//
+// Restart intervals (JPEZYB200_OPT_RESTART_INTERVAL = R > 0, the kernels' RST = true instantiations; RST = false compiles to
+// the restart-less pipeline): the DC predictors restart at 0 in every interval of R MCUs (T.81 F.1.2.3), and one more
+// kernel, k_rst_intervals, runs between E3b and E3c.  It rounds every interval up to whole bytes and scans them into the
+// byte base B_i of interval i in the un-stuffed stream (B_nint = its length).  k_scatter writes block b of interval i at
+// bit 8 B_i + G(b) - G(first block of i), G being the block's offset without padding, and the last block of every interval
+// writes that interval's pad bits.  The RSTn markers are not stored in the un-stuffed stream (the stuffing would put a 00
+// behind their FF): k_stuff_write inserts FF D((i-1) mod 8) in front of byte B_i, i >= 1, so un-stuffed byte k lands at
+// k + (0xFF bytes before k) + 2 (interval starts in 1..k).
 #pragma once
 #include "common.cuh"
 
@@ -48,12 +57,23 @@ struct EntParams {
     uint32_t lut_stride;     // HuffEncLut per image: 0 = every image reads lut[0..1], 2 = per-image tables (enc_huffopt.cuh)
 };
 
-// index of the previous block of the same component in scan order, or -1
-__device__ __forceinline__ long long prev_same_component(uint32_t b)
+// restart intervals: read by the RST = true kernels only (a kernel argument of its own, so that EntParams, and with it the
+// layout of ShardParams, stays as the restart-less kernels have it)
+struct RstParams {
+    uint32_t rst;            // MCUs per interval
+    uint32_t nint;           // intervals per image = ceil(MCUs / rst)
+    uint64_t* base;          // [nimg][nint + 1]  byte base B_i of each interval in the un-stuffed stream, then its length
+};
+
+// index of the previous block of the same component in scan order, or -1; with RST, -1 also for the first block of each
+// component in an interval of `rst` MCUs (the predictors restart at 0)
+template <bool RST = false>
+__device__ __forceinline__ long long prev_same_component(uint32_t b, uint32_t rst = 0)
 {
     const uint32_t k = b % 6u;
     if (k >= 1 && k <= 3) return (long long)b - 1;
     if (b < 6) return -1;
+    if (RST && (b / 6u) % rst == 0) return -1;
     return (long long)b - (k == 0 ? 3 : 6);
 }
 
@@ -174,8 +194,32 @@ __device__ __forceinline__ void load_lut(const HuffEncLut* __restrict__ g, uint3
     if (threadIdx.x < 32) s_dc[threadIdx.x >> 4][threadIdx.x & 15] = g[threadIdx.x >> 4].dc[threadIdx.x & 15];
 }
 
+__device__ __forceinline__ uint64_t block_scan_excl64(uint64_t v, uint64_t* s_warp, uint64_t* total)
+{
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    uint64_t x = v;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const uint64_t y = __shfl_up_sync(0xffffffffu, x, d);
+        if (lane >= d) x += y;
+    }
+    if (lane == 31) s_warp[wid] = x;
+    __syncthreads();
+    const int nw = blockDim.x >> 5;
+    uint64_t base = 0, tot = 0;
+    for (int w = 0; w < nw; ++w) {
+        const uint64_t s = s_warp[w];
+        if (w < wid) base += s;
+        tot += s;
+    }
+    __syncthreads();
+    *total = tot;
+    return base + x - v;
+}
+
 // ---- E3a ------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(kEntThreads) k_block_bits(const EntParams p)
+template <bool RST>
+__global__ void __launch_bounds__(kEntThreads) k_block_bits(const EntParams p, const RstParams r)
 {
     pdl_wait();
     __shared__ uint32_t s_ac[2][256];
@@ -189,7 +233,7 @@ __global__ void __launch_bounds__(kEntThreads) k_block_bits(const EntParams p)
     bool bad = false;
     if (b < p.nblk) {
         const int16_t* base = p.coefs + img * p.coef_stride;
-        const long long pb = prev_same_component(b);
+        const long long pb = prev_same_component<RST>(b, r.rst);
         const int cls = (b % 6u) >= 4;
         const int comp = (b % 6u) < 4 ? 0 : int(b % 6u) - 3;
         BlockRegs blk;
@@ -240,6 +284,46 @@ __global__ void __launch_bounds__(1024) k_scan_tiles(const EntParams p)
     }
 }
 
+// ---- restart intervals: one CTA per image, 64-bit running carry ------------------------------------------
+// Interval i covers blocks [6 R i, 6 R (i + 1)); its length is G(first block of i + 1) - G(first block of i) bits, rounded
+// up to bytes.  Writes B_i (and B_nint = the padded length) to rst_base and replaces img_bits with 8 B_nint, so the zeroing
+// and stuffing kernels size the padded stream; scan_bits (out_bits, written by k_scan_tiles) stays the Huffman bit count.
+__device__ __forceinline__ uint64_t block_bit_offset(const EntParams& p, size_t img, uint32_t b)
+{
+    return p.tile_base[img * p.ntile + b / kEntThreads] + p.blk_off[img * p.nblk + b];
+}
+
+__global__ void __launch_bounds__(1024) k_rst_intervals(const EntParams p, const RstParams r)
+{
+    pdl_wait();
+    __shared__ uint64_t s_warp[32];
+    const size_t img = blockIdx.x;
+    const uint64_t bits = p.img_bits[img];
+    if (bits >= (1ull << 62)) return;   // a coefficient without a code (k_scan_tiles): nothing to lay out
+    const uint32_t per = 6u * r.rst;     // blocks per interval
+    uint64_t* base = r.base + img * (size_t(r.nint) + 1);
+    uint64_t carry = 0;
+    for (uint32_t i0 = 0; i0 < r.nint; i0 += 1024) {
+        const uint32_t i = i0 + threadIdx.x;
+        uint64_t len = 0;
+        if (i < r.nint) {
+            const uint32_t b0 = i * per;
+            const uint64_t g0 = block_bit_offset(p, img, b0);
+            const uint64_t g1 = p.nblk - b0 > per ? block_bit_offset(p, img, b0 + per) : bits;
+            len = (g1 - g0 + 7) / 8;
+        }
+        uint64_t total;
+        const uint64_t off = block_scan_excl64(len, s_warp, &total);
+        if (i < r.nint) base[i] = carry + off;
+        carry += total;
+    }
+    // (every thread read img_bits before the first scan's barrier)
+    if (threadIdx.x == 0) {
+        base[r.nint] = carry;
+        p.img_bits[img] = carry * 8;
+    }
+}
+
 // ---- zero the part of the un-stuffed stream that will be written (grid-stride, data dependent) -----------
 __global__ void __launch_bounds__(256) k_zero_ustream(const EntParams p)
 {
@@ -254,7 +338,8 @@ __global__ void __launch_bounds__(256) k_zero_ustream(const EntParams p)
 }
 
 // ---- E3c ------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(kEntThreads) k_scatter(const EntParams p)
+template <bool RST>
+__global__ void __launch_bounds__(kEntThreads) k_scatter(const EntParams p, const RstParams r)
 {
     pdl_wait();
     __shared__ uint32_t s_ac[2][256];
@@ -267,13 +352,17 @@ __global__ void __launch_bounds__(kEntThreads) k_scatter(const EntParams p)
     const uint64_t total = p.img_bits[img];
     if ((total + 7) / 8 + 4 > p.uslot) return;   // does not fit: reported by k_scan_ff
     const int16_t* base = p.coefs + img * p.coef_stride;
-    const long long pb = prev_same_component(b);
+    const long long pb = prev_same_component<RST>(b, r.rst);
     const int cls = (b % 6u) >= 4;
     const int comp = (b % 6u) < 4 ? 0 : int(b % 6u) - 3;
     BlockRegs blk;
     int pred;
     load_block(base, p.bmeta ? p.bmeta + img * p.nblk : nullptr, b, pb, p.dc_init ? p.dc_init[img * 3 + comp] : 0, blk, pred);
-    const uint64_t pos = p.tile_base[img * p.ntile + blockIdx.x] + p.blk_off[img * p.nblk + b];
+    uint64_t pos = p.tile_base[img * p.ntile + blockIdx.x] + p.blk_off[img * p.nblk + b];
+    if constexpr (RST) {   // from the interval's byte base instead of its unpadded bit offset
+        const uint32_t i = b / (6u * r.rst);
+        pos += 8 * r.base[img * (size_t(r.nint) + 1) + i] - block_bit_offset(p, img, i * 6u * r.rst);
+    }
     uint32_t* out = reinterpret_cast<uint32_t*>(p.ustream + img * p.uslot) + (pos >> 5);
     uint64_t acc = 0;
     int n = int(pos & 31u);     // bits already occupied in the current word (not ours)
@@ -291,7 +380,13 @@ __global__ void __launch_bounds__(kEntThreads) k_scatter(const EntParams p)
         }
     };
     encode_block(blk, pred, s_ac[cls], s_dc[cls], emit);
-    if (b == p.nblk - 1 && p.pad_ones) {   // complete the last byte with 1-bits (write_eoi)
+    if constexpr (RST) {
+        // the last block of every interval completes the interval's last byte (n = where the block's bits end, modulo 32)
+        if (((b + 1) % (6u * r.rst) == 0 || b == p.nblk - 1) && p.pad_ones) {
+            const int padn = (8 - (n & 7)) & 7;
+            if (padn) emit((1u << padn) - 1u, padn);
+        }
+    } else if (b == p.nblk - 1 && p.pad_ones) {   // complete the last byte with 1-bits (write_eoi)
         const int padn = int((8u - uint32_t(total & 7u)) & 7u);
         if (padn) emit((1u << padn) - 1u, padn);
     }
@@ -331,7 +426,8 @@ __global__ void __launch_bounds__(kStuffThreads) k_ff_count(const EntParams p)
     }
 }
 
-__global__ void __launch_bounds__(1024) k_scan_ff(const EntParams p)
+template <bool RST>
+__global__ void __launch_bounds__(1024) k_scan_ff(const EntParams p, const RstParams r)
 {
     pdl_wait();
     __shared__ uint32_t s_warp[32];
@@ -357,13 +453,14 @@ __global__ void __launch_bounds__(1024) k_scan_ff(const EntParams p)
         __syncthreads();
     }
     if (threadIdx.x == 0) {
-        const uint64_t outb = nbytes + s_carry;
+        const uint64_t outb = nbytes + s_carry + (RST ? 2ull * (r.nint - 1) : 0ull);   // (RST: the markers)
         if (p.out_bytes) p.out_bytes[img] = outb <= p.slot ? outb : ~0ull;
         p.img_bytes[img] = outb;
     }
 }
 
-__global__ void __launch_bounds__(kStuffThreads) k_stuff_write(const EntParams p)
+template <bool RST>
+__global__ void __launch_bounds__(kStuffThreads) k_stuff_write(const EntParams p, const RstParams r)
 {
     pdl_wait();
     __shared__ uint32_t s_warp[kStuffThreads / 32];
@@ -385,12 +482,39 @@ __global__ void __launch_bounds__(kStuffThreads) k_stuff_write(const EntParams p
         if (!live) continue;
         uint64_t o = i16 * 16 + p.ff_base[img * p.nchunk + ch] + off;
         const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+        if constexpr (RST) {
+            // the first interval j >= 1 that starts at or after this group (B strictly increasing, B_nint = nbytes), and the
+            // markers in front of the group
+            const uint64_t* B = r.base + img * (size_t(r.nint) + 1);
+            const uint64_t k0 = i16 * 16;
+            uint32_t lo = 1, hi = r.nint;
+            while (lo < hi) {
+                const uint32_t mid = (lo + hi) >> 1;
+                if (B[mid] < k0) lo = mid + 1;
+                else hi = mid;
+            }
+            o += 2ull * (lo - 1);
+            uint64_t next = B[lo];
+            for (int i = 0; i < 16; ++i) {
+                const uint64_t k = k0 + i;
+                if (k >= nbytes) break;
+                if (k == next) {   // RST((j - 1) mod 8) in front of interval j's first byte
+                    dst[o++] = 0xffu;
+                    dst[o++] = uint8_t(0xd0u + ((lo - 1) & 7u));
+                    next = B[++lo];
+                }
+                const uint8_t byte = uint8_t(w[i >> 2] >> ((i & 3) * 8));
+                dst[o++] = byte;
+                if (byte == 0xffu) dst[o++] = 0;
+            }
+        } else {
 #pragma unroll
-        for (int i = 0; i < 16; ++i) {
-            if (i16 * 16 + i >= nbytes) break;
-            const uint8_t byte = uint8_t(w[i >> 2] >> ((i & 3) * 8));
-            dst[o++] = byte;
-            if (byte == 0xffu) dst[o++] = 0;
+            for (int i = 0; i < 16; ++i) {
+                if (i16 * 16 + i >= nbytes) break;
+                const uint8_t byte = uint8_t(w[i >> 2] >> ((i & 3) * 8));
+                dst[o++] = byte;
+                if (byte == 0xffu) dst[o++] = 0;
+            }
         }
     }
 }

@@ -60,7 +60,8 @@ __device__ __forceinline__ int count_block(const BlockRegs& blk, int dc_pred, ui
     return cat;
 }
 
-__global__ void __launch_bounds__(kEntThreads) k_sym_hist(const EntParams p, unsigned long long* __restrict__ counts)
+template <bool RST>   // RST: the DC differences of a stream with restart intervals (enc_entropy.cuh)
+__global__ void __launch_bounds__(kEntThreads) k_sym_hist(const EntParams p, unsigned long long* __restrict__ counts, const RstParams r)
 {
     pdl_wait();
     __shared__ uint32_t s_cnt[2][kHistBins];
@@ -77,7 +78,7 @@ __global__ void __launch_bounds__(kEntThreads) k_sym_hist(const EntParams p, uns
         const int comp = (b % 6u) < 4 ? 0 : int(b % 6u) - 3;
         BlockRegs blk;
         int pred;
-        load_block(base, p.bmeta ? p.bmeta + img * p.nblk : nullptr, b, prev_same_component(b),
+        load_block(base, p.bmeta ? p.bmeta + img * p.nblk : nullptr, b, prev_same_component<RST>(b, r.rst),
                    p.dc_init ? p.dc_init[img * 3 + comp] : 0, blk, pred);
         key = cls * kHistBins + count_block(blk, pred, &s_cnt[cls][16], eob);
     }
