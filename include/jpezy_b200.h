@@ -39,7 +39,11 @@ enum {
                                    returns an empty optional, src/decoder/jpezy_decoder.hpp:109-114) */
     JPEZYB200_ENODEVICE = 6,    /* no CUDA device: there is no CPU path                            */
     JPEZYB200_ENOMEM = 7,
-    JPEZYB200_EUNSUPPORTED = 8, /* frame layout outside what the device decoder handles            */
+    JPEZYB200_EUNSUPPORTED = 8, /* frame layout outside what the device decoder handles; from the
+                                   decode entry points also per image: a DC coefficient (predictor
+                                   plus differences) leaves the int16 range of the coefficient
+                                   format.  The reference keeps it in an int and decodes such a
+                                   stream; the device reports it instead of a wrapped result.    */
     JPEZYB200_EAGAIN = 9        /* *_dev decode only (reported per image in d_status): the parallel
                                    Huffman decoder did not reach its fixed point within the enqueued
                                    rounds; decode again with JPEZYB200_OPT_SYNC_ROUNDS = 0.  The
@@ -220,7 +224,8 @@ JPEZYB200_API int jpezyb200_decode(jpezyb200_ctx* ctx, const uint8_t* scan, size
 
 /* Batch, device resident, all images share the frame descriptor.  Image i: segment at
  * d_scan + i*slot_bytes with length h_scan_bytes[i] (HOST array: the file length is host knowledge),
- * planes at d_r + i*plane_bytes.  d_status[i] (device, may be NULL) receives 0, JPEZYB200_ECORRUPT or JPEZYB200_EAGAIN (the
+ * planes at d_r + i*plane_bytes.  d_status[i] (device, may be NULL) receives 0, JPEZYB200_ECORRUPT, JPEZYB200_EUNSUPPORTED (a DC
+ * coefficient outside the int16 range; that image's planes are not the reference's) or JPEZYB200_EAGAIN (the
  * self-synchronising decoder did not reach its fixed point in the enqueued launches: decode that image again with
  * JPEZYB200_OPT_SYNC_ROUNDS = 0, the host-polled loop). */
 JPEZYB200_API int jpezyb200_decode_batch_dev(jpezyb200_ctx* ctx, const uint8_t* d_scan, size_t slot_bytes, const uint64_t* h_scan_bytes,
@@ -243,7 +248,8 @@ JPEZYB200_API int jpezyb200_decode_batch_dev2(jpezyb200_ctx* ctx, const uint8_t*
 JPEZYB200_API int jpezyb200_decode_batch(jpezyb200_ctx* ctx, const uint8_t* scan, size_t slot_bytes, const uint64_t* scan_bytes, uint32_t nimg,
                            const jpezyb200_frame* f, int gray, uint8_t* r, uint8_t* g, uint8_t* b, size_t plane_bytes, int32_t* status);
 
-/* Stage D1 only: segment(s) -> coefficients (layout of jpezyb200_transform_fwd_dev, DC absolute). */
+/* Stage D1 only: segment(s) -> coefficients (layout of jpezyb200_transform_fwd_dev, DC absolute).  d_status as above: an image
+ * whose DC leaves the int16 range reports JPEZYB200_EUNSUPPORTED (its DC coefficients are wrapped). */
 JPEZYB200_API int jpezyb200_entropy_decode_dev(jpezyb200_ctx* ctx, const uint8_t* d_scan, size_t slot_bytes,
                                  const uint64_t* h_scan_bytes, uint32_t nimg, const jpezyb200_frame* f, int16_t* d_coefs,
                                  int32_t* d_status, void* stream);

@@ -985,6 +985,7 @@ __global__ void __launch_bounds__(128) k_decode_segments(const DecParams p)
     int16_t* out = p.coefs + img * p.coef_stride;
     int pred[3] = {0, 0, 0};
     int corrupt = 0;
+    bool dc_wide = false;     // a DC coefficient outside the int16 range of the coefficient format
     for (uint32_t m = mcu0; m < mcu1 && !corrupt; ++m) {
         for (uint32_t k = 0; k < p.nb; ++k) {
             const uint32_t comp = k < p.ny ? 0u : k - p.ny + 1u;
@@ -1010,7 +1011,10 @@ __global__ void __launch_bounds__(128) k_decode_segments(const DecParams p)
                     const uint32_t vbits = (w << len) >> (32 - sz);
                     int v = int(vbits);
                     if (!(vbits & (1u << (sz - 1)))) v -= (1 << sz) - 1;
-                    if (z == 0u) v = (pred[comp] += v);
+                    if (z == 0u) {
+                        v = (pred[comp] += v);
+                        dc_wide |= v != int(int16_t(v));
+                    }
                     blk[kk] = int16_t(v);
                 } else if (z == 0u) {
                     blk[0] = int16_t(pred[comp]);
@@ -1021,6 +1025,7 @@ __global__ void __launch_bounds__(128) k_decode_segments(const DecParams p)
         }
     }
     if (corrupt && p.status) p.status[img] = JPEZYB200_ECORRUPT;
+    else if (dc_wide && p.status) atomicCAS(p.status + img, 0, int(JPEZYB200_EUNSUPPORTED));
 }
 
 // ---- D1d: DC differences -> absolute DC (pred_dct[sc] += diff, src/decoder/jpezy_decoder.hpp:596-597) -----
@@ -1116,10 +1121,14 @@ __global__ void __launch_bounds__(256) k_dc_apply(const DecParams p)
         d[k] = py;
     }
     if (p.nb > p.ny) d[p.ny] = incl[1], d[p.ny + 1] = incl[2];
+    bool dc_wide = false;     // a DC coefficient outside the int16 range of the coefficient format
     for (uint32_t k = 0; k < p.nb; ++k) {
         dd[k] = int16_t(d[k]);
         if (!p.dc_dense) c[k * 64] = int16_t(d[k]);
+        dc_wide |= d[k] != int(int16_t(d[k]));
     }
+    // (only over "ok": an EAGAIN of the first attempt keeps driving the host's retry)
+    if (dc_wide && p.status) atomicCAS(p.status + img, 0, int(JPEZYB200_EUNSUPPORTED));
 }
 
 }  // namespace jz

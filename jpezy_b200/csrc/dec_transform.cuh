@@ -41,6 +41,14 @@ struct InvParams {
 
 constexpr double kGuardInv = 1e-6;
 
+// IDCT samples of valid baseline streams are not bounded by 16 bits (|AC| <= 1023 with Annex K tables reaches |sample| ~ 2e5),
+// while the reference keeps them in int and clamps only in make_rgb.  A tile (block) with a sample at or beyond this magnitude
+// in the FP32 flowgraph leaves the int16 sample path and is decided pixel by pixel with sample_ref and the reference's FP64
+// colour expressions.  (The margin to 32768 absorbs the flowgraph's error; it also keeps every fast-path value below 2^22, where
+// the floor trick of the second-generation kernels holds.)
+constexpr float kWideSample = 16384.0f;
+__device__ __forceinline__ bool wide_int(int v) { return uint32_t(v + 16383) > 32766u; }     // |v| >= 16384
+
 // exact-order IDCT sample (src/decoder/jpezy_decoder.hpp:657-668):
 //   sum += cu*cv*dct[v*8+u]*cos[u*8+x]*cos[v*8+y]   (v outer, u inner, left-to-right products)
 //   block[y*8+x] = int(sum / 4 + 128)
@@ -61,6 +69,25 @@ __device__ __noinline__ int idct_exact(const int* __restrict__ dq, unsigned long
     return __double2int_rz(__dadd_rn(__dmul_rn(sum, 0.25), 128.0));
 }
 
+// the reference's sample (x, y) of a block of zig-zag int16 coefficients: int dequantisation and the FP64 sum in its operation
+// order (natural order ascending; zero terms cannot change the sum), int(sum / 4 + 128) without narrowing (:645-670)
+__device__ __noinline__ int sample_ref(const int16_t* __restrict__ cz, const uint16_t* __restrict__ qt, int x, int y)
+{
+    double sum = 0.0;
+    for (int nat = 0; nat < 64; ++nat) {
+        const int c = cz[cC.izz[nat]];
+        if (!c) continue;
+        const int v = nat >> 3, u = nat & 7;
+        const double cu = u ? 1.0 : cC.inv_sqrt2_ref, cv = v ? 1.0 : cC.inv_sqrt2_ref;
+        double t = __dmul_rn(cu, cv);
+        t = __dmul_rn(t, double(c * int(qt[nat])));
+        t = __dmul_rn(t, cC.cos_ref[u * 8 + x]);
+        t = __dmul_rn(t, cC.cos_ref[v * 8 + y]);
+        sum = __dadd_rn(sum, t);
+    }
+    return __double2int_rz(__dadd_rn(__dmul_rn(sum, 0.25), 128.0));
+}
+
 // colour conversion, bit-exact with to_r/to_g/to_b + revise_value (:567-578, :672-676)
 __device__ __forceinline__ uint8_t revise(double v) { return v < 0.0 ? uint8_t(0) : (v > 255.0 ? uint8_t(255) : uint8_t(__double2int_rz(v))); }
 __device__ __forceinline__ uint8_t ref_R(int y, int cr) { return revise(__dadd_rn(double(y), __dmul_rn(double(cr - 128), 1.4020))); }
@@ -71,6 +98,22 @@ __device__ __forceinline__ uint8_t ref_G(int y, int cb, int cr)
 }
 __device__ __forceinline__ uint8_t ref_B(int y, int cb) { return revise(__dadd_rn(double(y), __dmul_rn(double(cb - 128), 1.7718))); }
 
+// pixel (px, py) of a 4:2:0 MCU whose six blocks (Y0 Y1 Y2 Y3 Cb Cr, zig-zag int16, `bstride` bytes apart) lie at `mcu`, every
+// sample by sample_ref: the route of the tiles with samples outside the int16 range
+__device__ __noinline__ void pixel420_ref(const InvParams& p, const uint8_t* mcu, uint32_t bstride, uint32_t px, uint32_t py, size_t idx,
+                                          uint8_t* R, uint8_t* G, uint8_t* B)
+{
+    const int16_t* yb = reinterpret_cast<const int16_t*>(mcu + ((py >> 3) * 2 + (px >> 3)) * bstride);
+    const int yv = sample_ref(yb, p.qt[0], int(px & 7u), int(py & 7u));
+    if (p.gray) {
+        R[idx] = G[idx] = B[idx] = revise(double(yv));
+        return;
+    }
+    const int cb = sample_ref(reinterpret_cast<const int16_t*>(mcu + 4 * bstride), p.qt[1], int(px >> 1), int(py >> 1));
+    const int cr = sample_ref(reinterpret_cast<const int16_t*>(mcu + 5 * bstride), p.qt[2], int(px >> 1), int(py >> 1));
+    R[idx] = ref_R(yv, cr), G[idx] = ref_G(yv, cb, cr), B[idx] = ref_B(yv, cb);
+}
+
 // ---- general layouts + validation build: FP64 separable IDCT -----------------------------------------------
 // Handles every frame layout the device decoder accepts (1 or 3 components, luma H, V in {1, 2}, chroma 1x1): the
 // production kernel below is specialised for jpezy's own 2x2 / 1x1 / 1x1.  One CTA = kMcuPerCta MCUs of one MCU row.
@@ -80,8 +123,7 @@ __global__ void __launch_bounds__(kFwdThreads) k_inv_transform_f64(const InvPara
 {
     pdl_wait();
     __shared__ int s_dq[kBlkPerCta][64];                 // dequantised, natural order
-    __shared__ double s_tmp[kBlkPerCta][64];
-    __shared__ short s_pix[kBlkPerCta][64];              // IDCT output (unclamped int, fits 16 bits)
+    __shared__ double s_tmp[kBlkPerCta][64];             // column pass; then the IDCT output, unclamped ints as in the reference
     __shared__ unsigned long long s_nz[kBlkPerCta];
 
     const int t = threadIdx.x;
@@ -134,13 +176,13 @@ __global__ void __launch_bounds__(kFwdThreads) k_inv_transform_f64(const InvPara
             for (int u = 0; u < 8; ++u) s = fma(row[u], cC.cos_ref[u * 8 + x], s);
             const double val = s * 0.25 + 128.0;
             int iv;
-            if (fabs(val - rint(val)) < kGuardInv) {
+            if (fabs(val - rint(val)) < kGuardInv || fabs(val) >= double(kWideSample)) {
                 iv = idct_exact(&s_dq[blk][0], s_nz[blk], x, y);
                 ++guard_hits;
             } else {
                 iv = __double2int_rz(val);
             }
-            s_pix[blk][y * 8 + x] = short(iv);
+            s_tmp[blk][y * 8 + x] = double(iv);      // (the row was read into registers above)
         }
     }
     __syncthreads();
@@ -159,7 +201,7 @@ __global__ void __launch_bounds__(kFwdThreads) k_inv_transform_f64(const InvPara
         const uint32_t gx = (mx0 + mcu) * mw + px;
         if (mcu >= nvalid || gx >= p.W) continue;
         const uint32_t sx0 = px / dx0, sy0 = ry / dy0;
-        const int yv = s_pix[mcu * nb + (sy0 >> 3) * p.hs[0] + (sx0 >> 3)][(sy0 & 7) * 8 + (sx0 & 7)];
+        const int yv = int(s_tmp[mcu * nb + (sy0 >> 3) * p.hs[0] + (sx0 >> 3)][(sy0 & 7) * 8 + (sx0 & 7)]);
         const size_t idx = (size_t(my) * mh + ry) * p.W + gx;
         if (p.gray) {
             const uint8_t v = revise(double(yv));
@@ -168,8 +210,8 @@ __global__ void __launch_bounds__(kFwdThreads) k_inv_transform_f64(const InvPara
             int cb = 128, cr = 128;      // comp tiles of absent components stay 0x80 (src/decoder/jpezy_decoder.hpp:105)
             if (p.ncomp == 3) {
                 const uint32_t sx1 = px / dx1, sy1 = ry / dy1, sx2 = px / dx2, sy2 = ry / dy2;
-                cb = s_pix[mcu * nb + ny + (sy1 >> 3) * p.hs[1] + (sx1 >> 3)][(sy1 & 7) * 8 + (sx1 & 7)];
-                cr = s_pix[mcu * nb + ny + p.hs[1] * p.vs[1] + (sy2 >> 3) * p.hs[2] + (sx2 >> 3)][(sy2 & 7) * 8 + (sx2 & 7)];
+                cb = int(s_tmp[mcu * nb + ny + (sy1 >> 3) * p.hs[1] + (sx1 >> 3)][(sy1 & 7) * 8 + (sx1 & 7)]);
+                cr = int(s_tmp[mcu * nb + ny + p.hs[1] * p.vs[1] + (sy2 >> 3) * p.hs[2] + (sx2 >> 3)][(sy2 & 7) * 8 + (sx2 & 7)]);
             }
             R[idx] = ref_R(yv, cr), G[idx] = ref_G(yv, cb, cr), B[idx] = ref_B(yv, cb);
         }
@@ -430,7 +472,7 @@ __global__ void __launch_bounds__(kInvThreads, 3) k_inv_transform(const __grid_c
     const uint32_t my = blockIdx.y + p.row0;
     const size_t img = blockIdx.z;
     const uint32_t nvalid = min(uint32_t(kTileMcu), p.HU - mx0);
-    if (t == 0) *s_nfix = 0;
+    if (t == 0) s_nfix[0] = 0, s_nfix[1] = 0;      // fix-up count, "a sample leaves the int16 range" (kWideSample)
     // the block this thread transforms in phase 1 (warps 0..3 luma, 4 Cb, 5 Cr); luma: warp 0 = top blocks of MCUs 0..15,
     // warp 1 = their bottom blocks, warps 2/3 = MCUs 16..31
     const uint32_t my_blk = warp < 4 ? ((warp >> 1) * 16 + (lane >> 1)) * 6 + (warp & 1) * 2 + (lane & 1) : uint32_t(lane) * 6 + warp;
@@ -487,6 +529,7 @@ __global__ void __launch_bounds__(kInvThreads, 3) k_inv_transform(const __grid_c
 #pragma unroll
             for (int y = 0; y < 8; ++y) *reinterpret_cast<uint4*>(tile + y * stride) = make_uint4(vv, vv, vv, vv);
             if (lane == 0) atomicAdd(p.guard_counter, 32ull * 64ull);
+            if (wide_int(v)) s_nfix[1] = 1;
         } else {
             float d[64];
             float gsum;
@@ -501,7 +544,9 @@ __global__ void __launch_bounds__(kInvThreads, 3) k_inv_transform(const __grid_c
 #pragma unroll
                 for (int y = 0; y < 8; ++y) *reinterpret_cast<uint4*>(tile + y * stride) = make_uint4(vv, vv, vv, vv);
                 dc_exact = 64;
+                if (wide_int(v)) s_nfix[1] = 1;
             } else {
+                float vmax = 0.0f;
 #pragma unroll
                 for (int y = 0; y < 8; ++y) {
                     int iv[8];
@@ -514,6 +559,7 @@ __global__ void __launch_bounds__(kInvThreads, 3) k_inv_transform(const __grid_c
                         iv[x] = __float2int_rz(val);
                         const float kf = (val + 12582912.0f) - 12582912.0f;   // rint(val), |val| < 2^22
                         m = fminf(m, fabsf(val - kf));
+                        vmax = fmaxf(vmax, fabsf(val));
                     }
                     if (m < gsum) flag_row(vr, gsum, blk, y, s_nfix, s_fix);
                     uint4 v;
@@ -521,12 +567,26 @@ __global__ void __launch_bounds__(kInvThreads, 3) k_inv_transform(const __grid_c
                     v.z = __byte_perm(uint32_t(iv[4]), uint32_t(iv[5]), 0x5410), v.w = __byte_perm(uint32_t(iv[6]), uint32_t(iv[7]), 0x5410);
                     *reinterpret_cast<uint4*>(tile + y * stride) = v;
                 }
+                if (vmax >= kWideSample && blk < nvalid * 6u) s_nfix[1] = 1;
             }
             dc_exact = __reduce_add_sync(0xffffffffu, dc_exact);
             if (lane == 0 && dc_exact) atomicAdd(p.guard_counter, (unsigned long long)dc_exact);
         }
     }
     __syncthreads();
+
+    uint8_t* R = p.r + img * p.plane_stride;
+    uint8_t* G = p.g + img * p.plane_stride;
+    uint8_t* B = p.b + img * p.plane_stride;
+    if (s_nfix[1]) {
+        // a sample outside the int16 range: every pixel of the tile from the coefficients, as the reference computes it
+        for (uint32_t e = t; e < nvalid * 256u; e += kInvThreads) {
+            const uint32_t mcu = e >> 8, py = (e >> 4) & 15u, px = e & 15u, gx = (mx0 + mcu) * 16u + px;
+            if (gx < p.W) pixel420_ref(p, &s_coef[mcu * 6u * kOutStride], kOutStride, px, py, (size_t(my) * 16 + py) * p.W + gx, R, G, B);
+        }
+        if (t == 0) atomicAdd(p.guard_counter, nvalid * 256ull);     // (JPEZYB200_STAT_GUARD_INV: exact-order pixels)
+        return;
+    }
 
     // ---- phase 1b: dense re-evaluation of the queue (guard-band samples) ----
     {
@@ -606,9 +666,8 @@ __global__ void __launch_bounds__(kInvThreads, 3) k_inv_transform(const __grid_c
     }
 
     // ---- phase 2: colour + planar stores; one thread per (row, MCU) ----
-    uint8_t* R = p.r + img * p.plane_stride;
-    uint8_t* G = p.g + img * p.plane_stride;
-    uint8_t* B = p.b + img * p.plane_stride;
+    // (this kernel runs for buffers that are not all 16-byte aligned: whole-row stores only where the planes are)
+    const bool planes16 = ((reinterpret_cast<uintptr_t>(R) | reinterpret_cast<uintptr_t>(G) | reinterpret_cast<uintptr_t>(B)) & 15u) == 0;
 #pragma unroll 1
     for (uint32_t task = t; task < 512u; task += kInvThreads) {
         const uint32_t ry = task >> 5, mcu = task & 31u;
@@ -650,7 +709,7 @@ __global__ void __launch_bounds__(kInvThreads, 3) k_inv_transform(const __grid_c
             }
         }
         const size_t rowoff = (size_t(my) * 16 + ry) * p.W;
-        if ((p.W & 15u) == 0 && x0 + 16u <= p.W) {
+        if (planes16 && (p.W & 15u) == 0 && x0 + 16u <= p.W) {
             *reinterpret_cast<uint4*>(R + rowoff + x0) = make_uint4(ro[0], ro[1], ro[2], ro[3]);
             *reinterpret_cast<uint4*>(G + rowoff + x0) = make_uint4(go[0], go[1], go[2], go[3]);
             *reinterpret_cast<uint4*>(B + rowoff + x0) = make_uint4(bo[0], bo[1], bo[2], bo[3]);

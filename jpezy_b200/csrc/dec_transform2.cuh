@@ -125,6 +125,12 @@ __device__ __forceinline__ float fmin3_abs(float a, float b, float c)
     asm("{\n\t.reg .f32 x, y;\n\tabs.f32 x, %1;\n\tabs.f32 y, %2;\n\tmin.f32 %0, x, y, %3;\n\t}" : "=f"(r) : "f"(a), "f"(b), "f"(c));
     return r;
 }
+__device__ __forceinline__ float fmax3_abs(float a, float b, float c)
+{
+    float r;
+    asm("{\n\t.reg .f32 x, y;\n\tabs.f32 x, %1;\n\tabs.f32 y, %2;\n\tmax.f32 %0, x, y, %3;\n\t}" : "=f"(r) : "f"(a), "f"(b), "f"(c));
+    return r;
+}
 // base + byte K of w (one IDP.4A)
 template <int K>
 __device__ __forceinline__ uint32_t add_byte(uint32_t w, uint32_t base)
@@ -289,7 +295,7 @@ __global__ void __launch_bounds__(T * 24, T == 8 ? 5 : 2) k_inv_transform2(const
 
     if (t == 0) {
         mbar_init(bar, 1);
-        *s_nfix = 0;
+        s_nfix[0] = 0, s_nfix[1] = 0;      // fix-up count, "a sample leaves the int16 range" (kWideSample)
         mbar_fence_init();
     }
     __syncthreads();
@@ -337,11 +343,14 @@ __global__ void __launch_bounds__(T * 24, T == 8 ? 5 : 2) k_inv_transform2(const
         dcA = __shfl_sync(0xffffffffu, dcA, lane & 24), dcB = __shfl_sync(0xffffffffu, dcB, lane & 24);
 
         uint4 rowA, rowB;         // the 8 + 8 samples of row sub as int16 pairs
+        bool wide;                // a sample of this row of the two blocks leaves the int16 range
         if ((balA | balB) == 0u) {
             // every block of the warp is DC-only
-            const uint32_t va = uint32_t(dc_only_value(dcA, qA)) & 0xffffu, vb = uint32_t(dc_only_value(dcB, qB)) & 0xffffu;
+            const int ia = dc_only_value(dcA, qA), ib = dc_only_value(dcB, qB);
+            const uint32_t va = uint32_t(ia) & 0xffffu, vb = uint32_t(ib) & 0xffffu;
             rowA = make_uint4(va * 0x10001u, va * 0x10001u, va * 0x10001u, va * 0x10001u);
             rowB = make_uint4(vb * 0x10001u, vb * 0x10001u, vb * 0x10001u, vb * 0x10001u);
+            wide = valid && (wide_int(ia) || wide_int(ib));
             if (lane == 0) atomicAdd(p.guard_counter, 32ull * 16ull);
         } else {
             const bool pruned = ((balA | balB) & 0xfefefefeu) == 0u;      // nothing beyond zig-zag position 7 in the warp
@@ -413,14 +422,16 @@ __global__ void __launch_bounds__(T * 24, T == 8 ? 5 : 2) k_inv_transform2(const
             // floor (low mantissa bits of v + 1.5 * 2^23, rounded down) and distance to the nearest integer
             const f32x2 mg = pk2(kMagic15, kMagic15);
             uint32_t ia[8], ib[8];
-            float ma = 1.0f, mb = 1.0f;
+            float ma = 1.0f, mb = 1.0f, va = 0.0f, vb = 0.0f;
 #pragma unroll
             for (int x = 0; x < 8; x += 2) {
                 const f32x2 f0 = add2_rm(d[x], mg), f1 = add2_rm(d[x + 1], mg);
                 ia[x] = uint32_t(f0), ib[x] = uint32_t(f0 >> 32), ia[x + 1] = uint32_t(f1), ib[x + 1] = uint32_t(f1 >> 32);
                 const f32x2 e0 = sub2(d[x], sub2(add2(d[x], mg), mg)), e1 = sub2(d[x + 1], sub2(add2(d[x + 1], mg), mg));
                 ma = fmin3_abs(lo2(e0), lo2(e1), ma), mb = fmin3_abs(hi2(e0), hi2(e1), mb);
+                va = fmax3_abs(lo2(d[x]), lo2(d[x + 1]), va), vb = fmax3_abs(hi2(d[x]), hi2(d[x + 1]), vb);
             }
+            wide = valid && fmaxf(va, vb) >= kWideSample;
             rowA = make_uint4(__byte_perm(ia[0], ia[1], 0x5410), __byte_perm(ia[2], ia[3], 0x5410), __byte_perm(ia[4], ia[5], 0x5410), __byte_perm(ia[6], ia[7], 0x5410));
             rowB = make_uint4(__byte_perm(ib[0], ib[1], 0x5410), __byte_perm(ib[2], ib[3], 0x5410), __byte_perm(ib[4], ib[5], 0x5410), __byte_perm(ib[6], ib[7], 0x5410));
             const bool dcoA = maskA == 0u, dcoB = maskB == 0u;
@@ -443,6 +454,7 @@ __global__ void __launch_bounds__(T * 24, T == 8 ? 5 : 2) k_inv_transform2(const
             exact = __reduce_add_sync(0xffffffffu, valid ? exact : 0u);
             if (lane == 0 && exact) atomicAdd(p.guard_counter, (unsigned long long)exact);
         }
+        if (__any_sync(0xffffffffu, wide) && lane == 0) s_nfix[1] = 1;
         // ---- hand the row over: luma samples to the tile, chroma samples as colour offsets ----
         if (luma) {
             uint8_t* dst = s_y + sub * C::kYRow + (mcu * 16u + (pr & 1u) * 8u) * 2u;
@@ -460,6 +472,19 @@ __global__ void __launch_bounds__(T * 24, T == 8 ? 5 : 2) k_inv_transform2(const
         }
     }
     __syncthreads();
+
+    uint8_t* R = p.r + img * p.plane_stride;
+    uint8_t* G = p.g + img * p.plane_stride;
+    uint8_t* B = p.b + img * p.plane_stride;
+    if (s_nfix[1]) {
+        // a sample outside the int16 range: every pixel of the tile from the coefficients (DC in place), as the reference computes it
+        for (uint32_t e = t; e < nvalid * 256u; e += C::kThreads) {
+            const uint32_t m = e >> 8, py = (e >> 4) & 15u, px = e & 15u, gx = (mx0 + m) * 16u + px;
+            if (gx < p.W) pixel420_ref(p, s_coef + m * 768u, 128u, px, py, (size_t(my) * 16 + py) * p.W + gx, R, G, B);
+        }
+        if (t == 0) atomicAdd(p.guard_counter, nvalid * 256ull);     // (JPEZYB200_STAT_GUARD_INV: exact-order pixels)
+        return;
+    }
 
     // ---- phase 1b: dense FP64 re-evaluation of the queue (guard-band samples) ----
     {
@@ -505,9 +530,6 @@ __global__ void __launch_bounds__(T * 24, T == 8 ? 5 : 2) k_inv_transform2(const
     }
 
     // ---- phase 2: colour + planar stores; one thread per (row, MCU) ----
-    uint8_t* R = p.r + img * p.plane_stride;
-    uint8_t* G = p.g + img * p.plane_stride;
-    uint8_t* B = p.b + img * p.plane_stride;
     if (t < T * 16) {
         const uint32_t ry = uint32_t(t) / T, m = uint32_t(t) % T;
         const uint32_t x0 = (mx0 + m) * 16u;

@@ -10,7 +10,8 @@
 //    FADD2.RM, per-block guard band, DC-only blocks in the reference's order, FP64 fix-up queue with the exact-order tier --
 //    over the image's blocks in scan order, whatever component they belong to: a pair is two consecutive blocks, its constants
 //    come from the table of its (component A, component B) class.  The 8x8 samples of every block go to a scratch array
-//    (int16, 128 bytes per block, scan order).
+//    (int16, 128 bytes per block, scan order).  A block with a sample outside the int16 range (kWideSample) is written as
+//    kWideMark in every sample instead: k_colour_general recomputes its pixels from the coefficients.
 //  * k_colour_general: one thread per 8 pixels of a row: gathers the Y, Cb, Cr samples through the MCU geometry (replication =
 //    index arithmetic), evaluates the reference's FP64 expressions (40 TFLOP/s of FP64 make that 8 us for a 4K frame), stores
 //    8 bytes per plane.
@@ -44,6 +45,7 @@ __global__ void k_build_invg_tab(const InvParams p, InvGTab* __restrict__ tab)
 }
 
 constexpr int kGBlk = 48;                       // blocks per CTA
+constexpr int16_t kWideMark = -32768;           // every sample of a block whose samples leave the int16 range (never a sample otherwise)
 constexpr int kGThreads = kGBlk * 4;            // eight lanes per pair
 struct InvG {
     static constexpr int kCoef = kGBlk * 128;
@@ -66,6 +68,7 @@ __global__ void __launch_bounds__(kGThreads, 5) k_idct_blocks(const __grid_const
     uint32_t* s_nfix = reinterpret_cast<uint32_t*>(s_fix + kFixCap);
     const uint32_t bar = smem_u32(s_nfix + 2);
     uint8_t* s_mask = reinterpret_cast<uint8_t*>(s_nfix + 4);    // [kGBlk] non-zero zig-zag groups of every block
+    unsigned long long* s_wide = reinterpret_cast<unsigned long long*>(s_mask + kGBlk);     // blocks with samples outside int16
 
     const int t = threadIdx.x, lane = t & 31;
     const size_t img = blockIdx.y;
@@ -74,6 +77,7 @@ __global__ void __launch_bounds__(kGThreads, 5) k_idct_blocks(const __grid_const
     if (t == 0) {
         mbar_init(bar, 1);
         *s_nfix = 0;
+        *s_wide = 0;
         mbar_fence_init();
     }
     __syncthreads();
@@ -113,11 +117,14 @@ __global__ void __launch_bounds__(kGThreads, 5) k_idct_blocks(const __grid_const
         dcA = __shfl_sync(0xffffffffu, dcA, lane & 24), dcB = __shfl_sync(0xffffffffu, dcB, lane & 24);
 
         uint4 rowA, rowB;         // the 8 + 8 samples of row sub as int16 pairs
+        bool wideA, wideB;        // a sample of this row leaves the int16 range
         if ((balA | balB) == 0u) {
             // every block of the warp is DC-only
-            const uint32_t va = uint32_t(dc_only_value(dcA, qA)) & 0xffffu, vb = uint32_t(dc_only_value(dcB, qB)) & 0xffffu;
+            const int ia = dc_only_value(dcA, qA), ib = dc_only_value(dcB, qB);
+            const uint32_t va = uint32_t(ia) & 0xffffu, vb = uint32_t(ib) & 0xffffu;
             rowA = make_uint4(va * 0x10001u, va * 0x10001u, va * 0x10001u, va * 0x10001u);
             rowB = make_uint4(vb * 0x10001u, vb * 0x10001u, vb * 0x10001u, vb * 0x10001u);
+            wideA = wide_int(ia), wideB = wide_int(ib);
             if (lane == 0) atomicAdd(p.guard_counter, 32ull * 16ull);
         } else {
             const bool pruned = ((balA | balB) & 0xfefefefeu) == 0u;      // nothing beyond zig-zag position 7 in the warp
@@ -179,14 +186,16 @@ __global__ void __launch_bounds__(kGThreads, 5) k_idct_blocks(const __grid_const
             else aan_idct8_x2(d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7]);
             const f32x2 mg = pk2(kMagic15, kMagic15);
             uint32_t ia[8], ib[8];
-            float ma = 1.0f, mb = 1.0f;
+            float ma = 1.0f, mb = 1.0f, va = 0.0f, vb = 0.0f;
 #pragma unroll
             for (int x = 0; x < 8; x += 2) {
                 const f32x2 f0 = add2_rm(d[x], mg), f1 = add2_rm(d[x + 1], mg);
                 ia[x] = uint32_t(f0), ib[x] = uint32_t(f0 >> 32), ia[x + 1] = uint32_t(f1), ib[x + 1] = uint32_t(f1 >> 32);
                 const f32x2 e0 = sub2(d[x], sub2(add2(d[x], mg), mg)), e1 = sub2(d[x + 1], sub2(add2(d[x + 1], mg), mg));
                 ma = fmin3_abs(lo2(e0), lo2(e1), ma), mb = fmin3_abs(hi2(e0), hi2(e1), mb);
+                va = fmax3_abs(lo2(d[x]), lo2(d[x + 1]), va), vb = fmax3_abs(hi2(d[x]), hi2(d[x + 1]), vb);
             }
+            wideA = va >= kWideSample, wideB = vb >= kWideSample;
             rowA = make_uint4(__byte_perm(ia[0], ia[1], 0x5410), __byte_perm(ia[2], ia[3], 0x5410), __byte_perm(ia[4], ia[5], 0x5410), __byte_perm(ia[6], ia[7], 0x5410));
             rowB = make_uint4(__byte_perm(ib[0], ib[1], 0x5410), __byte_perm(ib[2], ib[3], 0x5410), __byte_perm(ib[4], ib[5], 0x5410), __byte_perm(ib[6], ib[7], 0x5410));
             const bool dcoA = maskA == 0u, dcoB = maskB == 0u;
@@ -211,6 +220,7 @@ __global__ void __launch_bounds__(kGThreads, 5) k_idct_blocks(const __grid_const
         }
         if (validA) *reinterpret_cast<uint4*>(s_smp + blkA * 128u + sub * 16u) = rowA;
         if (validB) *reinterpret_cast<uint4*>(s_smp + blkB * 128u + sub * 16u) = rowB;
+        if ((wideA && validA) || (wideB && validB)) atomicOr(s_wide, (wideA && validA ? 1ull << blkA : 0ull) | (wideB && validB ? 1ull << blkB : 0ull));
     }
     __syncthreads();
 
@@ -251,7 +261,10 @@ __global__ void __launch_bounds__(kGThreads, 5) k_idct_blocks(const __grid_const
     }
     // ---- the samples leave, 16 bytes per thread and round ----
     uint4* dst = reinterpret_cast<uint4*>(samples + (img * (p.coef_stride >> 6) + blk0) * 64);
-    for (uint32_t i = t; i < nvalid * 8u; i += kGThreads) dst[i] = reinterpret_cast<const uint4*>(s_smp)[i];
+    const unsigned long long wide = *s_wide;
+    constexpr uint32_t kMark2 = uint32_t(uint16_t(kWideMark)) * 0x10001u;
+    for (uint32_t i = t; i < nvalid * 8u; i += kGThreads)
+        dst[i] = (wide >> (i >> 3)) & 1ull ? make_uint4(kMark2, kMark2, kMark2, kMark2) : reinterpret_cast<const uint4*>(s_smp)[i];
 }
 
 // one thread per 8 pixels of a row of MCU rows [row0, row0 + rows).  The 8 pixels lie in one MCU and, per component, in one row of
@@ -266,6 +279,28 @@ __device__ __forceinline__ void load_samples8(const int16_t* __restrict__ smp, s
     } else {
         const uint2 w = *reinterpret_cast<const uint2*>(src);
         v[0] = v[1] = sx_lo(w.x), v[2] = v[3] = sx_hi(w.x), v[4] = v[5] = sx_lo(w.y), v[6] = v[7] = sx_hi(w.y);
+    }
+}
+
+// the 8 pixels of k_colour_general, every sample by sample_ref from the coefficients (blocks marked kWideMark)
+__device__ __noinline__ void colour_general_ref(const InvParams& p, size_t img, size_t mcu, uint32_t ry, uint32_t px0, uint32_t gx0, size_t idx)
+{
+    const int16_t* cz = p.coefs + img * p.coef_stride;
+    for (uint32_t i = 0; i < 8 && gx0 + i < p.W; ++i) {
+        const uint32_t px = px0 + i;
+        int v[3] = {0, 128, 128};          // comp tiles of absent components stay 0x80 (src/decoder/jpezy_decoder.hpp:105)
+        const int nc = (p.ncomp == 3 && !p.gray) ? 3 : 1;
+        size_t first = mcu;
+        for (int c = 0; c < nc; ++c) {
+            const uint32_t sx = px / (p.hmax / p.hs[c]), sy = ry / (p.vmax / p.vs[c]);
+            v[c] = sample_ref(cz + (first + (sy >> 3) * p.hs[c] + (sx >> 3)) * 64, p.qt[c], int(sx & 7u), int(sy & 7u));
+            first += p.hs[c] * p.vs[c];
+        }
+        uint8_t* R = p.r + img * p.plane_stride + idx + i;
+        uint8_t* G = p.g + img * p.plane_stride + idx + i;
+        uint8_t* B = p.b + img * p.plane_stride + idx + i;
+        if (p.gray) *R = *G = *B = revise(double(v[0]));
+        else *R = ref_R(v[0], v[2]), *G = ref_G(v[0], v[1], v[2]), *B = ref_B(v[0], v[1]);
     }
 }
 
@@ -296,6 +331,15 @@ __global__ void __launch_bounds__(256) k_colour_general(const __grid_constant__ 
 #pragma unroll
         for (int i = 0; i < 8; ++i) cb[i] = cr[i] = 128;      // comp tiles of absent components stay 0x80 (src/decoder/jpezy_decoder.hpp:105)
     }
+    const size_t idx = size_t(y) * p.W + gx0;
+    bool wide = false;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) wide |= yv[i] == kWideMark || cb[i] == kWideMark || cr[i] == kWideMark;
+    if (wide) {
+        colour_general_ref(p, img, mcu, ry, px0, gx0, idx);
+        atomicAdd(p.guard_counter, 8ull);     // (JPEZYB200_STAT_GUARD_INV: exact-order pixels)
+        return;
+    }
     uint32_t ro[2] = {0, 0}, go[2] = {0, 0}, bo[2] = {0, 0};
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
@@ -304,7 +348,6 @@ __global__ void __launch_bounds__(256) k_colour_general(const __grid_constant__ 
         else r = ref_R(yv[i], cr[i]), g = ref_G(yv[i], cb[i], cr[i]), b = ref_B(yv[i], cb[i]);
         ro[i >> 2] |= r << (8 * (i & 3)), go[i >> 2] |= g << (8 * (i & 3)), bo[i >> 2] |= b << (8 * (i & 3));
     }
-    const size_t idx = size_t(y) * p.W + gx0;
     uint8_t* R = p.r + img * p.plane_stride;
     uint8_t* G = p.g + img * p.plane_stride;
     uint8_t* B = p.b + img * p.plane_stride;

@@ -12,6 +12,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _u8p = C.POINTER(C.c_uint8)
 _i16p = C.POINTER(C.c_int16)
+_i32p = C.POINTER(C.c_int32)
 
 
 def build(force=False):
@@ -119,7 +120,12 @@ class Oracle:
         L.orc_header.argtypes = [C.c_int, C.c_int, C.c_int, _u8p, C.c_size_t, C.POINTER(C.c_size_t)]
         L.orc_scan_from_coefs.argtypes = [_i16p, C.c_size_t, C.c_int, _u8p, C.c_size_t, C.POINTER(C.c_size_t),
                                           C.POINTER(C.c_uint64)]
-        L.orc_probe.argtypes = [_u8p, C.c_size_t, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_size_t)]
+        L.orc_scan_from_coefs32.argtypes = [_i32p, C.c_size_t, C.c_int, C.c_int, _u8p, C.c_size_t, C.POINTER(C.c_size_t),
+                                            C.POINTER(C.c_uint64)]
+        L.orc_probe.argtypes = [_u8p, C.c_size_t, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_size_t), _i32p, _i32p,
+                                _i32p, C.POINTER(C.c_size_t)]
+        L.orc_pixels_from_coefs.argtypes = [_i32p, C.c_size_t, C.c_int, C.c_int, C.c_int, _i32p, _i32p, C.POINTER(C.c_uint16),
+                                            C.c_int, _u8p, _u8p, _u8p, C.c_size_t]
         L.orc_decode.argtypes = [_u8p, C.c_size_t, C.c_int, _u8p, _u8p, _u8p, C.c_size_t]
         L.orc_decode_coefs.argtypes = [_u8p, C.c_size_t, _i16p, C.c_size_t, C.POINTER(C.c_size_t)]
         L.orc_enc_lut.argtypes = [C.c_int] + [C.POINTER(C.c_int)] * 4
@@ -168,25 +174,34 @@ class Oracle:
             raise RuntimeError("orc_header failed")
         return out[: n.value].tobytes()
 
-    def scan_from_coefs(self, coefs, pad_ones=True):
-        coefs = np.ascontiguousarray(coefs, dtype=np.int16).reshape(-1, 6, 64)
-        cap = coefs.size * 4 + 1024
+    def scan_from_coefs(self, coefs, pad_ones=True, restart_interval=0):
+        """4:2:0 coefficients (zig-zag, scan order; int32, so a DC may walk past the int16 range) -> entropy-coded segment,
+        with RSTn markers every restart_interval MCUs when it is > 0."""
+        coefs = np.ascontiguousarray(coefs, dtype=np.int32).reshape(-1, 6, 64)
+        cap = coefs.size * 4 + coefs.shape[0] * 2 + 1024
         out = np.zeros(cap, dtype=np.uint8)
         n = C.c_size_t(0)
         nb = C.c_uint64(0)
-        rc = self.lib.orc_scan_from_coefs(_ptr(coefs, _i16p), coefs.shape[0], int(pad_ones), _ptr(out), cap, C.byref(n),
-                                          C.byref(nb))
+        rc = self.lib.orc_scan_from_coefs32(_ptr(coefs, _i32p), coefs.shape[0], int(pad_ones), int(restart_interval), _ptr(out), cap,
+                                            C.byref(n), C.byref(nb))
         if rc:
-            raise RuntimeError("orc_scan_from_coefs failed")
+            raise RuntimeError("orc_scan_from_coefs32 failed")
         return out[: n.value].tobytes()
 
     # ---- decoder side -------------------------------------------------------------------------
     def probe(self, data):
+        return self.layout(data)[:3]
+
+    def layout(self, data):
+        """-> (W, H, plane_len, ncomp, hs, vs, nblocks) from the file's frame header"""
         a = np.frombuffer(data, dtype=np.uint8)
-        W, H, pl = C.c_int(0), C.c_int(0), C.c_size_t(0)
-        if self.lib.orc_probe(_ptr(a), a.size, C.byref(W), C.byref(H), C.byref(pl)):
+        W, H, pl, nb = C.c_int(0), C.c_int(0), C.c_size_t(0), C.c_size_t(0)
+        nc, hs, vs = np.zeros(1, np.int32), np.zeros(3, np.int32), np.zeros(3, np.int32)
+        if self.lib.orc_probe(_ptr(a), a.size, C.byref(W), C.byref(H), C.byref(pl), _ptr(nc, _i32p), _ptr(hs, _i32p), _ptr(vs, _i32p),
+                              C.byref(nb)):
             raise RuntimeError("orc_probe failed")
-        return W.value, H.value, pl.value
+        n = int(nc[0])
+        return W.value, H.value, pl.value, n, tuple(int(x) for x in hs[:n]), tuple(int(x) for x in vs[:n]), nb.value
 
     def decode(self, data, gray=False):
         """-> (W, H, r, g, b) with planes of the reference's padded length (stride W)."""
@@ -199,15 +214,34 @@ class Oracle:
         return W, H, r, g, b
 
     def decode_coefs(self, data):
+        """-> int16 zig-zag coefficients in scan order, absolute DC: [nmcu, 6, 64] for 4:2:0 frames, flat for the other layouts."""
         a = np.frombuffer(data, dtype=np.uint8)
-        W, H, _ = self.probe(data)
-        cap = self.num_mcus(W, H) * 6 * 64
+        _, _, _, nc, hs, vs, nblk = self.layout(data)
+        cap = nblk * 64
         out = np.zeros(cap, dtype=np.int16)
         n = C.c_size_t(0)
         rc = self.lib.orc_decode_coefs(_ptr(a), a.size, _ptr(out, _i16p), cap, C.byref(n))
         if rc:
             raise RuntimeError("orc_decode_coefs failed rc=%d" % rc)
-        return out[: n.value].reshape(-1, 6, 64)
+        out = out[: n.value]
+        return out.reshape(-1, 6, 64) if (nc, hs, vs) == (3, (2, 1, 1), (2, 1, 1)) else out
+
+    def pixels_from_coefs(self, coefs, W, H, qt, ncomp=3, hs=(2, 1, 1), vs=(2, 1, 1), gray=False):
+        """The reference decoder's pixel stage (dequant, idct, replication, make_rgb) on given coefficients: zig-zag, scan order,
+        absolute DC (int32, so DC values beyond int16 can be expressed); qt: one natural-order table per component (16 bit).
+        -> (r, g, b) planes of the reference's padded length (stride W)."""
+        c = np.ascontiguousarray(coefs, dtype=np.int32).reshape(-1)
+        q = np.ascontiguousarray(qt, dtype=np.uint16).reshape(ncomp, 64)
+        hs_a, vs_a = np.array(hs[:ncomp], np.int32), np.array(vs[:ncomp], np.int32)
+        hmax, vmax = int(hs_a.max()), int(vs_a.max())
+        hb, vb = (W + 7) // 8, (H + 7) // 8
+        pl = ((vb + vmax - 1) // vmax) * vmax * 8 * ((hb + hmax - 1) // hmax) * hmax * 8
+        r, g, b = (np.zeros(pl, dtype=np.uint8) for _ in range(3))
+        rc = self.lib.orc_pixels_from_coefs(_ptr(c, _i32p), c.size, W, H, ncomp, _ptr(hs_a, _i32p), _ptr(vs_a, _i32p),
+                                            _ptr(q, C.POINTER(C.c_uint16)), int(gray), _ptr(r), _ptr(g), _ptr(b), pl)
+        if rc:
+            raise RuntimeError("orc_pixels_from_coefs failed rc=%d" % rc)
+        return r, g, b
 
     # ---- tables -------------------------------------------------------------------------------
     def enc_lut(self, chroma):

@@ -17,6 +17,7 @@
 // Build: see oracle/Makefile.  Canonical semantics = strict IEEE double, no FMA contraction
 // (-ffp-contract=off, decision O3); the "as shipped" flag set is built beside it.
 
+#include <algorithm>
 #include <cmath>
 #include <cstdint>
 #include <cstdlib>
@@ -350,18 +351,27 @@ static void encode_core(Encoder& e, BitWriter* w, int16_t* coefs, double* raw)
         }
 }
 
-// entropy-code a given coefficient array (zig-zag int16, scan order) -- lets the tests check
+// entropy-code a given coefficient array (zig-zag, scan order) -- lets the tests check
 // "given identical coefficients the stream is byte-identical" independently of the DCT.
-static void encode_from_coefs(const int16_t* coefs, size_t nmcu, BitWriter& w)
+// restart_interval > 0: after every restart_interval MCUs but the last, the predictors are reset, the
+// segment is padded to a byte and RSTn is written (T.81 F.1.2.3 / E.1.4; the decoder side is :152-163).
+template <typename T>
+static void encode_from_coefs(const T* coefs, size_t nmcu, BitWriter& w, int restart_interval = 0)
 {
     Encoder e{};
-    for (size_t m = 0; m < nmcu; ++m)
+    for (size_t m = 0; m < nmcu; ++m) {
+        if (restart_interval > 0 && m > 0 && m % size_t(restart_interval) == 0) {
+            w.align();
+            w.byte(0xff), w.byte(0xd0 + int((m / size_t(restart_interval) - 1) & 7));
+            e.preDC[0] = e.preDC[1] = e.preDC[2] = 0;
+        }
         for (int k = 0; k < 6; ++k) {
             const int cs = k < 4 ? 0 : k - 3;
-            const int16_t* c = coefs + (m * 6 + k) * 64;
-            for (int n = 0; n < 64; ++n) e.F[kZZ[n]] = c[n];
+            const T* c = coefs + (m * 6 + k) * 64;
+            for (int n = 0; n < 64; ++n) e.F[kZZ[n]] = int(c[n]);
             e.huff(cs, w, cs ? lutC() : lutY());
         }
+    }
 }
 
 // ================================= decoder =====================================================
@@ -615,6 +625,65 @@ struct Decoder {
     static inline uint8_t revise(double v) { return v < 0.0 ? 0 : (v > 255.0 ? 255 : static_cast<uint8_t>(v)); }
 };
 
+// MCU geometry (src/decoder/jpezy_decoder.hpp:94-101): hu x vu MCUs, planes of plane_len bytes
+struct Geom {
+    size_t hu, vu, plane_len;
+};
+static Geom geometry(const Decoder& d)
+{
+    const size_t Vb = (d.H >> 3) + ((d.H & 7) > 0), Hb = (d.W >> 3) + ((d.W & 7) > 0);
+    Geom g;
+    g.hu = Hb / d.hmax + ((Hb % d.hmax) ? 1 : 0), g.vu = Vb / d.vmax + ((Vb % d.vmax) ? 1 : 0);
+    g.plane_len = (g.vu * d.vmax) * 8 * (g.hu * d.hmax) * 8;
+    return g;
+}
+
+// The pixel stage of one MCU, shared by the file decoder and orc_pixels_from_coefs: the component tiles
+// (value-initialised as at :105) and make_rgb (:531-565).
+struct PixelStage {
+    std::vector<int> comp[3];
+    size_t vstep;
+    explicit PixelStage(const Decoder& d)
+    {
+        const size_t unit = size_t(d.hmax) * d.vmax * 64;
+        comp[0].assign(unit, 0), comp[1].assign(unit, 0x80), comp[2].assign(unit, 0x80);
+        vstep = size_t(d.hmax) * 8;
+    }
+    // block (ky, kx) of component s, quantised coefficients in d.dctc (natural order): dequant, idct and the pixel
+    // replication of decode_mcu (:519-524)
+    void block(Decoder& d, int s, int ky, int kx)
+    {
+        const int dy = d.vmax / d.fc[s].Vs, dx = d.hmax / d.fc[s].Hs;
+        d.dequant(s);
+        d.idct();
+        int* tp = comp[s].data() + ky * vstep * 8 + kx * 8;
+        for (int yu = 0; yu < 8 * dy; ++yu)
+            for (int xu = 0; xu < 8 * dx; ++xu) tp[yu * vstep + xu] = d.block[(yu / dy) * 8 + (xu / dx)];
+    }
+    // make_rgb :531-565
+    void rgb(const Decoder& d, size_t ux, size_t uy, bool gray, std::vector<uint8_t>* planes) const
+    {
+        const int *yp = comp[0].data(), *up = comp[1].data(), *vp = comp[2].data();
+        const size_t off_h = ux * d.hmax * 8;
+        const size_t off = uy * d.vmax * 8 * size_t(d.W) + off_h;
+        const size_t ex = size_t(d.hmax) * 8, ey = size_t(d.vmax) * 8;
+        for (size_t py = 0; py < ey; ++py)
+            for (size_t px = 0; px < ex; ++px) {
+                if (px + off_h >= size_t(d.W)) { yp += ex - px, up += ex - px, vp += ex - px; break; }
+                const size_t idx = off + py * d.W + px;
+                if (!gray) {
+                    const double Y = *yp, U = *up, V = *vp;
+                    planes[0][idx] = Decoder::revise(Y + (V - 0x80) * 1.4020);
+                    planes[1][idx] = Decoder::revise(Y - (U - 0x80) * 0.3441 - (V - 0x80) * 0.7139);
+                    planes[2][idx] = Decoder::revise(Y + (U - 0x80) * 1.7718);
+                    ++yp, ++up, ++vp;
+                } else {
+                    planes[0][idx] = planes[1][idx] = planes[2][idx] = Decoder::revise(*yp++);
+                }
+            }
+    }
+};
+
 // src/decoder/jpezy_decoder.hpp:76-134 + 504-565.  Outputs: planes of plane_len bytes (zero
 // filled beyond what the MCU loop writes), optional coefficient dump (zig-zag int16, scan order,
 // DC already de-predicted = absolute).
@@ -625,54 +694,25 @@ static int decode_core(const uint8_t* file, size_t n, bool gray, std::vector<uin
     try { d.header(); } catch (const std::exception&) { return 1; }
     // :89 only requires one of is_htable|is_qtable|is_start_data; SOS is always set here.
     if (d.hmax <= 0 || d.vmax <= 0) return 1;   // the reference would divide by zero (no SOF0 seen)
-    const size_t Vb = (d.H >> 3) + ((d.H & 7) > 0), Hb = (d.W >> 3) + ((d.W & 7) > 0);
-    const size_t hu = Hb / d.hmax + ((Hb % d.hmax) ? 1 : 0), vu = Vb / d.vmax + ((Vb % d.vmax) ? 1 : 0);
-    const size_t plane = (vu * d.vmax) * 8 * (hu * d.hmax) * 8;
+    const Geom g = geometry(d);
     *Wout = d.W, *Hout = d.H;
-    if (planes) for (int c = 0; c < 3; ++c) planes[c].assign(plane, 0);
-    const size_t unit = size_t(d.hmax) * d.vmax * 64;
-    std::vector<int> comp[3];
-    comp[0].assign(unit, 0), comp[1].assign(unit, 0x80), comp[2].assign(unit, 0x80);
+    if (planes) for (int c = 0; c < 3; ++c) planes[c].assign(g.plane_len, 0);
+    PixelStage px(d);
     size_t restart_counter = 0;
-    const size_t vstep = size_t(d.hmax) * 8;
     try {
-        for (size_t uy = 0; uy < vu; ++uy)
-            for (size_t ux = 0; ux < hu; ++ux) {
+        for (size_t uy = 0; uy < g.vu; ++uy)
+            for (size_t ux = 0; ux < g.hu; ++ux) {
                 for (int s = 0; s < d.ncomp; ++s) {                      // decode_mcu :504-528
                     const int nv = d.fc[s].Vs, nh = d.fc[s].Hs;
                     if (nv <= 0 || nh <= 0) return 2;
-                    const int dy = d.vmax / nv, dx = d.hmax / nh;
                     for (int ky = 0; ky < nv; ++ky)
                         for (int kx = 0; kx < nh; ++kx) {
                             d.huff(s);
                             if (coefs) { for (int k = 0; k < 64; ++k) coefs->push_back(static_cast<int16_t>(d.dctc[kZZ[k]])); }
-                            d.dequant(s);
-                            d.idct();
-                            int* tp = comp[s].data() + ky * vstep * 8 + kx * 8;
-                            for (int yu = 0; yu < 8 * dy; ++yu)
-                                for (int xu = 0; xu < 8 * dx; ++xu) tp[yu * vstep + xu] = d.block[(yu / dy) * 8 + (xu / dx)];
+                            px.block(d, s, ky, kx);
                         }
                 }
-                if (planes) {                                            // make_rgb :531-565
-                    const int *yp = comp[0].data(), *up = comp[1].data(), *vp = comp[2].data();
-                    const size_t off_h = ux * d.hmax * 8;
-                    const size_t off = uy * d.vmax * 8 * size_t(d.W) + off_h;
-                    const size_t ex = size_t(d.hmax) * 8, ey = size_t(d.vmax) * 8;
-                    for (size_t py = 0; py < ey; ++py)
-                        for (size_t px = 0; px < ex; ++px) {
-                            if (px + off_h >= size_t(d.W)) { yp += ex - px, up += ex - px, vp += ex - px; break; }
-                            const size_t idx = off + py * d.W + px;
-                            if (!gray) {
-                                const double Y = *yp, U = *up, V = *vp;
-                                planes[0][idx] = Decoder::revise(Y + (V - 0x80) * 1.4020);
-                                planes[1][idx] = Decoder::revise(Y - (U - 0x80) * 0.3441 - (V - 0x80) * 0.7139);
-                                planes[2][idx] = Decoder::revise(Y + (U - 0x80) * 1.7718);
-                                ++yp, ++up, ++vp;
-                            } else {
-                                planes[0][idx] = planes[1][idx] = planes[2][idx] = Decoder::revise(*yp++);
-                            }
-                        }
-                }
+                if (planes) px.rgb(d, ux, uy, gray, planes);
                 if (d.restart_interval && ++restart_counter >= size_t(d.restart_interval)) {   // :152-163
                     restart_counter = 0;
                     try {
@@ -748,15 +788,80 @@ int orc_scan_from_coefs(const int16_t* coefs, size_t nmcu, int pad_ones, uint8_t
     return 0;
 }
 
-// JPEG file -> geometry (W, H, padded plane length as in jpezy_decoder.hpp:94-101)
-int orc_probe(const uint8_t* file, size_t n, int* W, int* H, size_t* plane_len)
+// coefficients (zig-zag int32, scan order, 4:2:0 MCUs) -> stuffed + padded entropy segment, with RSTn markers every
+// restart_interval MCUs when it is > 0
+int orc_scan_from_coefs32(const int32_t* coefs, size_t nmcu, int pad_ones, int restart_interval, uint8_t* out, size_t cap, size_t* out_len,
+                          uint64_t* nbits)
+{
+    try {
+        orc::BitWriter w(cap, pad_ones != 0);
+        orc::encode_from_coefs(coefs, nmcu, w, restart_interval);
+        if (nbits) *nbits = w.total_bits;   // before the fill bits
+        w.align();
+        *out_len = w.buf.size();
+        std::memcpy(out, w.buf.data(), w.buf.size());
+    } catch (const std::exception&) { return 1; }
+    return 0;
+}
+
+// JPEG file -> geometry (W, H, padded plane length as in jpezy_decoder.hpp:94-101); ncomp / hs / vs / nblocks may be null
+int orc_probe(const uint8_t* file, size_t n, int* W, int* H, size_t* plane_len, int* ncomp, int* hs, int* vs, size_t* nblocks)
 {
     orc::Decoder d(file, n);
     try { d.header(); } catch (const std::exception&) { return 1; }
     if (d.hmax <= 0 || d.vmax <= 0) return 1;
-    const size_t Vb = (d.H >> 3) + ((d.H & 7) > 0), Hb = (d.W >> 3) + ((d.W & 7) > 0);
-    const size_t hu = Hb / d.hmax + ((Hb % d.hmax) ? 1 : 0), vu = Vb / d.vmax + ((Vb % d.vmax) ? 1 : 0);
-    *W = d.W, *H = d.H, *plane_len = (vu * d.vmax) * 8 * (hu * d.hmax) * 8;
+    const orc::Geom g = orc::geometry(d);
+    *W = d.W, *H = d.H, *plane_len = g.plane_len;
+    size_t nb = 0;
+    for (int i = 0; i < d.ncomp; ++i) {
+        if (hs) hs[i] = d.fc[i].Hs;
+        if (vs) vs[i] = d.fc[i].Vs;
+        nb += size_t(d.fc[i].Hs) * d.fc[i].Vs;
+    }
+    if (ncomp) *ncomp = d.ncomp;
+    if (nblocks) *nblocks = nb * g.hu * g.vu;
+    return 0;
+}
+
+// quantised coefficients (zig-zag int32, scan order, absolute DC, the blocks of every MCU in decode_mcu's order) ->
+// planar RGB of plane_len bytes each, through the file decoder's own dequant / idct / replication / make_rgb.
+// qt: one table per component, natural order.  Returns 0 ok, 1 bad layout, 3 planes too small.
+int orc_pixels_from_coefs(const int32_t* coefs, size_t ncoefs, int W, int H, int ncomp, const int* hs, const int* vs, const uint16_t* qt,
+                          int gray, uint8_t* r, uint8_t* g, uint8_t* b, size_t plane_len)
+{
+    if ((ncomp != 1 && ncomp != 3) || W <= 0 || H <= 0) return 1;
+    orc::Decoder d(nullptr, 0);
+    d.W = W, d.H = H, d.ncomp = ncomp, d.prec = 8;
+    size_t nb = 0;
+    for (int i = 0; i < ncomp; ++i) {
+        if (hs[i] <= 0 || vs[i] <= 0) return 1;
+        d.fc[i].Hs = hs[i], d.fc[i].Vs = vs[i], d.fc[i].Tq = i;
+        d.hmax = std::max(d.hmax, hs[i]), d.vmax = std::max(d.vmax, vs[i]);
+        for (int k = 0; k < 64; ++k) d.qt[i][k] = qt[i * 64 + k];
+        nb += size_t(hs[i]) * vs[i];
+    }
+    for (int i = 0; i < ncomp; ++i)
+        if (d.hmax % hs[i] || d.vmax % vs[i]) return 1;
+    const orc::Geom geo = orc::geometry(d);
+    if (ncoefs != geo.hu * geo.vu * nb * 64) return 1;
+    if (geo.plane_len > plane_len) return 3;
+    std::vector<uint8_t> planes[3];
+    for (int c = 0; c < 3; ++c) planes[c].assign(geo.plane_len, 0);
+    orc::PixelStage px(d);
+    const int32_t* c = coefs;
+    for (size_t uy = 0; uy < geo.vu; ++uy)
+        for (size_t ux = 0; ux < geo.hu; ++ux) {
+            for (int s = 0; s < ncomp; ++s)
+                for (int ky = 0; ky < vs[s]; ++ky)
+                    for (int kx = 0; kx < hs[s]; ++kx, c += 64) {
+                        for (int k = 0; k < 64; ++k) d.dctc[orc::kZZ[k]] = c[k];
+                        px.block(d, s, ky, kx);
+                    }
+            px.rgb(d, ux, uy, gray != 0, planes);
+        }
+    std::memcpy(r, planes[0].data(), geo.plane_len);
+    std::memcpy(g, planes[1].data(), geo.plane_len);
+    std::memcpy(b, planes[2].data(), geo.plane_len);
     return 0;
 }
 

@@ -5,6 +5,23 @@ import torch
 import jpezy_b200 as J
 from jpezy_b200.capi import num_mcus
 
+GUARD = 4096
+
+
+class Guarded:
+    """n bytes of `dtype` elements with GUARD poisoned bytes on either side (the payload starts `offset` bytes past a 256-byte
+    boundary): a kernel that writes outside its buffer leaves a trace that intact() finds"""
+    def __init__(self, nelem, dtype, fill=0, offset=0):
+        self.esz = torch.empty(0, dtype=dtype).element_size()
+        self.n = nelem * self.esz
+        self.lo = GUARD + offset
+        self.raw = torch.full((self.lo + self.n + GUARD,), 0xA5, dtype=torch.uint8, device="cuda")
+        self.view = self.raw[self.lo: self.lo + self.n].view(dtype)
+        self.view.fill_(fill)
+
+    def intact(self):
+        return bool((self.raw[:self.lo] == 0xA5).all().item()) and bool((self.raw[self.lo + self.n:] == 0xA5).all().item())
+
 
 def to_dev(a):
     return torch.from_numpy(np.ascontiguousarray(a)).cuda()

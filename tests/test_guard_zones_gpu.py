@@ -7,24 +7,9 @@ import torch
 
 import jpezy_b200 as J
 from jpezy_b200 import capi
+from gpu_util import Guarded
 
 pytestmark = pytest.mark.gpu
-GUARD = 4096
-
-
-class Guarded:
-    """n bytes of `dtype` elements with GUARD poisoned bytes on either side (the payload starts `offset` bytes past a 256-byte
-    boundary)"""
-    def __init__(self, nelem, dtype, fill=0, offset=0):
-        self.esz = torch.empty(0, dtype=dtype).element_size()
-        self.n = nelem * self.esz
-        self.lo = GUARD + offset
-        self.raw = torch.full((self.lo + self.n + GUARD,), 0xA5, dtype=torch.uint8, device="cuda")
-        self.view = self.raw[self.lo: self.lo + self.n].view(dtype)
-        self.view.fill_(fill)
-
-    def intact(self):
-        return bool((self.raw[:self.lo] == 0xA5).all().item()) and bool((self.raw[self.lo + self.n:] == 0xA5).all().item())
 
 
 @pytest.mark.parametrize("W,H,family,gray,nimg", [(208, 128, 0, False, 1), (1920, 1080, 0, False, 2), (200, 120, 1, False, 3),
@@ -79,7 +64,7 @@ def test_device_entry_points_stay_inside_their_buffers(ctx, W, H, family, gray, 
 def test_unaligned_planes_take_the_first_generation_inverse_kernel(ctx):
     """4:2:0 output planes that start 1 byte past a 256-byte boundary (coefficients aligned) go to k_inv_transform, the 4:2:0
     kernel that needs no 16-byte aligned buffers: the planes equal those of the aligned call and the guard zones stay intact.
-    (W is not a multiple of 16: that kernel stores whole 16-byte rows of an MCU when it is.)"""
+    (tests/test_inverse_reference_gpu.py takes that kernel through W a multiple of 16 too.)"""
     W, H, nimg = 200, 120, 2
     frame = J.default_frame(W, H)
     pl = capi.plane_bytes(frame)
@@ -108,10 +93,11 @@ LAYOUTS = {"444": ((1, 1, 1), (1, 1, 1)), "422": ((2, 1, 1), (1, 1, 1)), "440": 
 @pytest.mark.parametrize("layout", sorted(LAYOUTS))
 @pytest.mark.parametrize("W,H", [(70, 45), (129, 257), (640, 368), (8, 8)])
 @pytest.mark.parametrize("gray", [False, True])
-def test_general_layout_inverse_equals_validation_kernel_and_stays_inside(ctx, layout, W, H, gray):
-    """the fast inverse path of the sampling layouts jpezy's encoder never writes (dec_transform_g.cuh) against the FP64 validation
-    kernel (JPEZYB200_OPT_TRANSFORM = 1) on random coefficients -- small ones, DC-only blocks, full-range ones that drive the
-    samples far outside [0, 255] -- with guard zones around the planes."""
+def test_general_layout_inverse_equals_validation_kernel_and_stays_inside(ctx, oracle, layout, W, H, gray):
+    """the fast inverse path of the sampling layouts jpezy's encoder never writes (dec_transform_g.cuh) and the FP64 validation
+    kernel (JPEZYB200_OPT_TRANSFORM = 1), each against the reference decoder's pixel stage, on random coefficients -- small ones,
+    DC-only blocks, full-range ones that drive the samples beyond the int16 range -- with guard zones around the planes.  (Checked
+    against each other only, both kernels once wrapped such samples to 16 bits the same way.)"""
     hs, vs = LAYOUTS[layout]
     f = J.default_frame(W, H)
     f.ncomp = len(hs)
@@ -148,6 +134,9 @@ def test_general_layout_inverse_equals_validation_kernel_and_stays_inside(ctx, l
             assert o.intact(), "guard zone around an output plane was written (variant %d)" % variant
         outs.append([o.view.clone() for o in out])
     assert d.intact()
-    for a, b in zip(*outs):
-        nd = int((a != b).sum())
-        assert nd == 0, "%d samples differ from the validation kernel" % nd
+    want = oracle.pixels_from_coefs(c.astype(np.int32), W, H, np.array([list(f.qt[f.tq[i]]) for i in range(len(hs))]), ncomp=len(hs),
+                                    hs=hs, vs=vs, gray=gray)
+    for variant, out in enumerate(outs):
+        for a, w in zip(out, want):
+            nd = int((a.cpu().numpy() != w).sum())
+            assert nd == 0, "%d samples differ from the reference decoder (variant %d)" % (nd, variant)
