@@ -13,6 +13,9 @@
 //    belongs to the warp (__syncwarp, not a CTA barrier), lane y transforms row y and decides its 8 + 8 samples;
 //  * when no block of the warp has a coefficient beyond zig-zag position 7 the flowgraphs are pruned to 3 inputs per column
 //    and 4 per row (operations on structural zeros dropped: bit-identical to the full flowgraph);
+//  * when no block of the warp has a coefficient beyond zig-zag position 2 (photographic content at normal quality: nearly
+//    every warp) the sample is the separable sum F00 q00 / 8 + 128 + F10 Ly[y] + F01 Lx[x]: lane y evaluates its row of both
+//    blocks with eight FFMA2, no column pass and no transpose, under a guard band of its own (tools/lowfreq_idct_error_bound.py);
 //  * floor(v) is one FADD2.RM against 1.5 * 2^23 (the integer sits in the low mantissa bits), the distance to the nearest
 //    integer three more packed adds; one 3-input-min chain per block row decides whether any sample is inside the guard
 //    band; negative samples (where the reference's truncation is not floor) and guard hits take the slow row function;
@@ -20,8 +23,8 @@
 //    trunc(y + t) = y + floor(t)); the colour phase is integer adds and saturating packs on 16 pixels of one row per thread,
 //    three 16-byte planar stores.
 //
-// Numerics: same AAN flowgraphs, same per-block guard band (tools/aan_idct_error_bound.py), same FP64 fix-up queue and
-// exact-order tier as k_inv_transform; DC-only blocks are evaluated in the reference's operation order.  Decoded samples are
+// Numerics: same AAN flowgraphs, same per-block guard band (tools/aan_idct_error_bound.py; the low-frequency class has its
+// own), same FP64 fix-up queue and exact-order tier as k_inv_transform; DC-only blocks are evaluated in the reference's operation order.  Decoded samples are
 // identical to the reference decoder's.  Algorithmic HBM traffic: 3 B/px read + 3 B/px written = 6 B/px.
 #pragma once
 #include "dec_transform.cuh"
@@ -96,7 +99,16 @@ struct Inv2Tab {
                            // class 0 = two luma blocks, class 1 = Cb | Cr (their quantisation tables may differ)
     float2 Wg[2][8][8];    // [pair class][u][v]: guard-band weights per unit |coefficient|
     uint2 zoff[8];         // [u]: byte offsets (2 * zig-zag position) of coefficients (0..7, u), one byte each
+    // blocks with nothing beyond zig-zag position 2: sample (x, y) = F(0,0) q / 8 + 128 + F(1,0) Ly[y] + F(0,1) Lx[x]
+    float2 Lx[2][8];       // [pair class][x]: q(0,1) cos((2x+1) pi / 16) / (4 sqrt 2)
+    float2 Ly[2][8];       // [pair class][y]: q(1,0) cos((2y+1) pi / 16) / (4 sqrt 2)
+    float2 Lg[2][4];       // [pair class]: guard-band weights of zig-zag positions 0..2 per unit |coefficient|, then the constant term
 };
+
+// worst-case FP32 error of that evaluation per unit dequantised coefficient of zig-zag position 0, 1, 2 (units of 2^-24, margin
+// 1.25 included) and its constant term, the level shift rounded three times (tools/lowfreq_idct_error_bound.py)
+constexpr double kLowErrSens0 = 0.625, kLowErrSens1 = 0.434, kLowErrSens2 = 0.651;
+constexpr float kLowGuard0 = 2.87e-5f;
 
 __global__ void k_build_inv2_tab(const InvParams p, Inv2Tab* __restrict__ tab)
 {
@@ -110,6 +122,16 @@ __global__ void k_build_inv2_tab(const InvParams p, Inv2Tab* __restrict__ tab)
         uint32_t w[2] = {0, 0};
         for (int vv = 0; vv < 8; ++vv) w[vv >> 2] |= uint32_t(cC.izz[vv * 8 + t] * 2) << (8 * (vv & 3));
         tab->zoff[t] = make_uint2(w[0], w[1]);
+    }
+    if (nat < 8) {      // the low-frequency class: column / row `nat`
+        const double s = cC.cos_ref[8 + nat] * cC.inv_sqrt2_ref * 0.25;
+        tab->Lx[c][nat] = make_float2(float(p.qt[ca][1] * s), float(p.qt[cb][1] * s));
+        tab->Ly[c][nat] = make_float2(float(p.qt[ca][8] * s), float(p.qt[cb][8] * s));
+        if (nat < 4) {
+            const int n = nat == 2 ? 8 : nat;      // natural position of zig-zag position `nat`
+            const double e = (nat == 0 ? kLowErrSens0 : nat == 1 ? kLowErrSens1 : kLowErrSens2) / 16777216.0;
+            tab->Lg[c][nat] = nat == 3 ? make_float2(kLowGuard0, kLowGuard0) : make_float2(float(p.qt[ca][n] * e), float(p.qt[cb][n] * e));
+        }
     }
 }
 
@@ -337,6 +359,8 @@ __global__ void __launch_bounds__(T * 24, T == 8 ? 5 : 2) k_inv_transform2(const
         }
         const uint32_t balA = __ballot_sync(0xffffffffu, (gA.x | gA.y | gA.z | gA.w) != 0u);
         const uint32_t balB = __ballot_sync(0xffffffffu, (gB.x | gB.y | gB.z | gB.w) != 0u);
+        // zig-zag positions 3..7 (the high half of word y, words z and w of group 0)
+        const uint32_t bal37 = __ballot_sync(0xffffffffu, sub == 0u && (((gA.y | gB.y) >> 16) | gA.z | gA.w | gB.z | gB.w) != 0u);
         const uint32_t maskA = (balA >> (lane & 24)) & 0xffu, maskB = (balB >> (lane & 24)) & 0xffu;
         if (sub == 0 && valid) s_mask[blkA] = uint8_t(maskA), s_mask[blkB] = uint8_t(maskB);
         const int qA = int(p.qt[compA][0]), qB = int(p.qt[compB][0]);
@@ -354,16 +378,38 @@ __global__ void __launch_bounds__(T * 24, T == 8 ? 5 : 2) k_inv_transform2(const
             if (lane == 0) atomicAdd(p.guard_counter, 32ull * 16ull);
         } else {
             const bool pruned = ((balA | balB) & 0xfefefefeu) == 0u;      // nothing beyond zig-zag position 7 in the warp
-            const uint32_t u = sub;
-            // ---- column u: de-zig-zag, dequantise (x AAN input scale), guard-band sum ----
-            f32x2 d[8];
-            f32x2 gs = pk2(0.0f, 0.0f);
-            {
-                const uint2 zo = __ldg(&tab->zoff[u]);
+            f32x2 d[8];           // samples of row sub of both blocks, level shift included
+            f32x2 gs;             // per-block guard band
+            if (pruned && bal37 == 0u) {
+                // ---- nothing beyond zig-zag position 2 in the warp: the sample is a separable sum, row sub evaluated directly
+                // (no column pass, no transpose).  FP32 order: ((F00 M00 + 128) + F10 Ly[sub]) + F01 Lx[x], one rounding per
+                // step; its own guard band (Lg) ----
                 const int cls = luma ? 0 : 1;
-                const ulonglong2* mq = reinterpret_cast<const ulonglong2*>(&tab->M[cls][u][0]);
-                const ulonglong2* wq = reinterpret_cast<const ulonglong2*>(&tab->Wg[cls][u][0]);
-                const uint32_t base = smem_u32(cA);
+                uint2 wA, wB;     // zig-zag 0..3 of both blocks (F(0,1) is the high half of x, F(1,0) the low half of y)
+                asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(wA.x), "=r"(wA.y) : "r"(smem_u32(cA)));
+                asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(wB.x), "=r"(wB.y) : "r"(smem_u32(cA) + dAB));
+                const f32x2 fd = pk2(float(dcA), float(dcB));
+                const f32x2 fa = pk2(float(sx_hi(wA.x)), float(sx_hi(wB.x))), fb = pk2(float(sx_lo(wA.y)), float(sx_lo(wB.y)));
+                const f32x2 m00 = __ldg(reinterpret_cast<const unsigned long long*>(&tab->M[cls][0][0]));
+                const f32x2 ly = __ldg(reinterpret_cast<const unsigned long long*>(&tab->Ly[cls][sub]));
+                const ulonglong2* lx = reinterpret_cast<const ulonglong2*>(&tab->Lx[cls][0]);
+                const ulonglong2* lg = reinterpret_cast<const ulonglong2*>(&tab->Lg[cls][0]);
+                const ulonglong2 x01 = __ldg(lx), x23 = __ldg(lx + 1), x45 = __ldg(lx + 2), x67 = __ldg(lx + 3), g01 = __ldg(lg), g23 = __ldg(lg + 1);
+                const f32x2 base = fma2(fb, ly, add2(mul2(fd, m00), pk2(128.0f, 128.0f)));
+                d[0] = fma2(fa, x01.x, base), d[1] = fma2(fa, x01.y, base), d[2] = fma2(fa, x23.x, base), d[3] = fma2(fa, x23.y, base);
+                d[4] = fma2(fa, x45.x, base), d[5] = fma2(fa, x45.y, base), d[6] = fma2(fa, x67.x, base), d[7] = fma2(fa, x67.y, base);
+                constexpr f32x2 kAbs = 0x7fffffff7fffffffull;
+                gs = fma2(fd & kAbs, g01.x, fma2(fa & kAbs, g01.y, fma2(fb & kAbs, g23.x, g23.y)));
+            } else {
+                const uint32_t u = sub;
+                // ---- column u: de-zig-zag, dequantise (x AAN input scale), guard-band sum ----
+                gs = pk2(0.0f, 0.0f);
+                {
+                    const uint2 zo = __ldg(&tab->zoff[u]);
+                    const int cls = luma ? 0 : 1;
+                    const ulonglong2* mq = reinterpret_cast<const ulonglong2*>(&tab->M[cls][u][0]);
+                    const ulonglong2* wq = reinterpret_cast<const ulonglong2*>(&tab->Wg[cls][u][0]);
+                    const uint32_t base = smem_u32(cA);
 #define JZ_LOAD_COEF(V, ZW, K, MM, WW)                                                                                   \
     {                                                                                                                     \
         const uint32_t ad = add_byte<K>(ZW, base);                                                                        \
@@ -374,51 +420,52 @@ __global__ void __launch_bounds__(T * 24, T == 8 ? 5 : 2) k_inv_transform2(const
         d[V] = mul2(f, MM);                                                                                               \
         const f32x2 g = mul2(f, WW);                                                                                      \
         gs = add2(gs, pk2(fabsf(lo2(g)), fabsf(hi2(g))));                                                                 \
-    }
-                const ulonglong2 m01 = __ldg(mq), m23 = __ldg(mq + 1), w01 = __ldg(wq), w23 = __ldg(wq + 1);
-                JZ_LOAD_COEF(0, zo.x, 0, m01.x, w01.x)
-                if (u == 0) {      // the DC coefficient is in registers (dense array or position 0 of the block)
-                    const f32x2 f = pk2(float(dcA), float(dcB));
-                    d[0] = mul2(f, m01.x);
-                    const f32x2 g = mul2(f, w01.x);
-                    gs = pk2(fabsf(lo2(g)), fabsf(hi2(g)));
-                }
-                JZ_LOAD_COEF(1, zo.x, 1, m01.y, w01.y)
-                JZ_LOAD_COEF(2, zo.x, 2, m23.x, w23.x)
-                if (pruned) {
-                    d[3] = d[4] = d[5] = d[6] = d[7] = pk2(0.0f, 0.0f);
-                } else {
-                    const ulonglong2 m45 = __ldg(mq + 2), m67 = __ldg(mq + 3), w45 = __ldg(wq + 2), w67 = __ldg(wq + 3);
-                    JZ_LOAD_COEF(3, zo.x, 3, m23.y, w23.y)
-                    JZ_LOAD_COEF(4, zo.y, 0, m45.x, w45.x)
-                    JZ_LOAD_COEF(5, zo.y, 1, m45.y, w45.y)
-                    JZ_LOAD_COEF(6, zo.y, 2, m67.x, w67.x)
-                    JZ_LOAD_COEF(7, zo.y, 3, m67.y, w67.y)
-                }
+        }
+                    const ulonglong2 m01 = __ldg(mq), m23 = __ldg(mq + 1), w01 = __ldg(wq), w23 = __ldg(wq + 1);
+                    JZ_LOAD_COEF(0, zo.x, 0, m01.x, w01.x)
+                    if (u == 0) {      // the DC coefficient is in registers (dense array or position 0 of the block)
+                        const f32x2 f = pk2(float(dcA), float(dcB));
+                        d[0] = mul2(f, m01.x);
+                        const f32x2 g = mul2(f, w01.x);
+                        gs = pk2(fabsf(lo2(g)), fabsf(hi2(g)));
+                    }
+                    JZ_LOAD_COEF(1, zo.x, 1, m01.y, w01.y)
+                    JZ_LOAD_COEF(2, zo.x, 2, m23.x, w23.x)
+                    if (pruned) {
+                        d[3] = d[4] = d[5] = d[6] = d[7] = pk2(0.0f, 0.0f);
+                    } else {
+                        const ulonglong2 m45 = __ldg(mq + 2), m67 = __ldg(mq + 3), w45 = __ldg(wq + 2), w67 = __ldg(wq + 3);
+                        JZ_LOAD_COEF(3, zo.x, 3, m23.y, w23.y)
+                        JZ_LOAD_COEF(4, zo.y, 0, m45.x, w45.x)
+                        JZ_LOAD_COEF(5, zo.y, 1, m45.y, w45.y)
+                        JZ_LOAD_COEF(6, zo.y, 2, m67.x, w67.x)
+                        JZ_LOAD_COEF(7, zo.y, 3, m67.y, w67.y)
+                    }
 #undef JZ_LOAD_COEF
-            }
-            if (u == 0) d[0] = add2(d[0], pk2(128.0f, 128.0f));       // level shift rides on the DC term (gain 1 through the flowgraph)
-            if (pruned) aan_idct8_in3_x2(d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7]);
-            else aan_idct8_x2(d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7]);
+                }
+                if (u == 0) d[0] = add2(d[0], pk2(128.0f, 128.0f));       // level shift rides on the DC term (gain 1 through the flowgraph)
+                if (pruned) aan_idct8_in3_x2(d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7]);
+                else aan_idct8_x2(d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7]);
 #pragma unroll
-            for (int y = 0; y < 8; ++y) *reinterpret_cast<f32x2*>(mid + y * C::kPairRow + u * 8u) = d[y];
-            // per-block guard band: sum over the eight columns
-            {
-                float ga = lo2(gs), gb = hi2(gs);
-                ga += __shfl_xor_sync(0xffffffffu, ga, 1), gb += __shfl_xor_sync(0xffffffffu, gb, 1);
-                ga += __shfl_xor_sync(0xffffffffu, ga, 2), gb += __shfl_xor_sync(0xffffffffu, gb, 2);
-                ga += __shfl_xor_sync(0xffffffffu, ga, 4), gb += __shfl_xor_sync(0xffffffffu, gb, 4);
-                gs = pk2(ga + 2e-5f, gb + 2e-5f);
+                for (int y = 0; y < 8; ++y) *reinterpret_cast<f32x2*>(mid + y * C::kPairRow + u * 8u) = d[y];
+                // per-block guard band: sum over the eight columns
+                {
+                    float ga = lo2(gs), gb = hi2(gs);
+                    ga += __shfl_xor_sync(0xffffffffu, ga, 1), gb += __shfl_xor_sync(0xffffffffu, gb, 1);
+                    ga += __shfl_xor_sync(0xffffffffu, ga, 2), gb += __shfl_xor_sync(0xffffffffu, gb, 2);
+                    ga += __shfl_xor_sync(0xffffffffu, ga, 4), gb += __shfl_xor_sync(0xffffffffu, gb, 4);
+                    gs = pk2(ga + 2e-5f, gb + 2e-5f);
+                }
+                __syncwarp();
+                // ---- row sub of both blocks ----
+                {
+                    const ulonglong2* src = reinterpret_cast<const ulonglong2*>(mid + sub * C::kPairRow);
+                    const ulonglong2 a = src[0], b = src[1], c = src[2], e = src[3];
+                    d[0] = a.x, d[1] = a.y, d[2] = b.x, d[3] = b.y, d[4] = c.x, d[5] = c.y, d[6] = e.x, d[7] = e.y;
+                }
+                if (pruned) aan_idct8_in4_x2(d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7]);
+                else aan_idct8_x2(d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7]);
             }
-            __syncwarp();
-            // ---- row sub of both blocks ----
-            {
-                const ulonglong2* src = reinterpret_cast<const ulonglong2*>(mid + sub * C::kPairRow);
-                const ulonglong2 a = src[0], b = src[1], c = src[2], e = src[3];
-                d[0] = a.x, d[1] = a.y, d[2] = b.x, d[3] = b.y, d[4] = c.x, d[5] = c.y, d[6] = e.x, d[7] = e.y;
-            }
-            if (pruned) aan_idct8_in4_x2(d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7]);
-            else aan_idct8_x2(d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7]);
             // floor (low mantissa bits of v + 1.5 * 2^23, rounded down) and distance to the nearest integer
             const f32x2 mg = pk2(kMagic15, kMagic15);
             uint32_t ia[8], ib[8];
