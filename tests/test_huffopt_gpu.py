@@ -12,6 +12,7 @@ import torch
 import jpezy_b200 as J
 from jpezy_b200 import capi
 from gpu_util import planes, to_dev
+from jpeg_build import dht, fibonacci_coefs, gen_optimal_table, symbol_hist
 
 pytestmark = pytest.mark.gpu
 
@@ -22,91 +23,6 @@ HB = capi.HUFF_TABLES_BYTES
 
 
 # ---- Python reference ------------------------------------------------------------------------------
-def bit_length(a):
-    a = np.abs(np.asarray(a, dtype=np.int64))
-    return sum((a >= (1 << i)).astype(np.int64) for i in range(16))
-
-
-def symbol_hist(coefs):
-    """[2 classes][16 DC categories + 256 AC symbols] counts of the symbols the encoder emits for zig-zag coefficients
-    [nmcu, 6, 64] (categories and sizes clamped to 11 and 10 as the encoder clamps them), and the magnitude bits"""
-    c = np.asarray(coefs, dtype=np.int64).reshape(-1, 6, 64)
-    hist = np.zeros((2, 272), np.int64)
-    extra = 0
-    dc = c[:, :, 0]
-    for cls, seq in ((0, dc[:, :4].reshape(-1)), (1, dc[:, 4]), (1, dc[:, 5])):
-        cat = np.minimum(bit_length(np.diff(seq, prepend=0)), 11)
-        hist[cls, :16] += np.bincount(cat, minlength=16)
-        extra += int(cat.sum())
-    ac = c[:, :, 1:].reshape(-1, 63)
-    blk_cls = np.tile((np.arange(6) >= 4).astype(np.int64), c.shape[0])
-    bi, pos = np.nonzero(ac)
-    prev = np.full(pos.shape, -1, np.int64)
-    prev[1:] = np.where(bi[1:] == bi[:-1], pos[:-1], -1)
-    run = pos - prev - 1
-    size = np.minimum(bit_length(ac[bi, pos]), 10)
-    cls = blk_cls[bi]
-    for k in (0, 1):
-        m = cls == k
-        hist[k, 16 + 0xF0] += int((run[m] // 16).sum())
-        hist[k, 16:] += np.bincount(((run[m] % 16) << 4) | size[m], minlength=256)
-        hist[k, 16 + 0x00] += int(((ac[:, 62] == 0) & (blk_cls == k)).sum())
-    extra += int(size.sum())
-    return hist, extra
-
-
-def gen_optimal_table(counts):
-    """T.81 K.2 (Figures K.1-K.4) line for line after libjpeg's jpeg_gen_optimal_table -> (BITS[16], HUFFVAL, codesize)"""
-    MAX_CLEN = 32
-    freq = [int(x) for x in counts] + [0] * (257 - len(counts))
-    bits = [0] * (MAX_CLEN + 1)
-    codesize = [0] * 257
-    others = [-1] * 257
-    freq[256] = 1
-    while True:
-        c1, v = -1, 1 << 62
-        for i in range(257):
-            if freq[i] and freq[i] <= v:
-                v, c1 = freq[i], i
-        c2, v = -1, 1 << 62
-        for i in range(257):
-            if freq[i] and freq[i] <= v and i != c1:
-                v, c2 = freq[i], i
-        if c2 < 0:
-            break
-        freq[c1] += freq[c2]
-        freq[c2] = 0
-        codesize[c1] += 1
-        while others[c1] >= 0:
-            c1 = others[c1]
-            codesize[c1] += 1
-        others[c1] = c2
-        codesize[c2] += 1
-        while others[c2] >= 0:
-            c2 = others[c2]
-            codesize[c2] += 1
-    for i in range(257):
-        if codesize[i]:
-            assert codesize[i] <= MAX_CLEN
-            bits[codesize[i]] += 1
-    i = MAX_CLEN
-    while i > 16:
-        while bits[i] > 0:
-            j = i - 2
-            while bits[j] == 0:
-                j -= 1
-            bits[i] -= 2
-            bits[i - 1] += 1
-            bits[j + 1] += 2
-            bits[j] -= 1
-        i -= 1
-    while bits[i] == 0:
-        i -= 1
-    bits[i] -= 1
-    huffval = [j for i in range(1, MAX_CLEN + 1) for j in range(256) if codesize[j] == i]
-    return bits[1:17], huffval, codesize
-
-
 def code_lengths(bits, huffval):
     return {s: L for s, L in zip(huffval, [L for L in range(1, 17) for _ in range(bits[L - 1])])}
 
@@ -132,11 +48,6 @@ def check_tables(ht, coefs):
         acl = check_table(ht[1][cls], hist[cls, 16:])
         total += sum(int(hist[cls, s]) * L for s, L in dcl.items()) + sum(int(hist[cls, 16 + s]) * L for s, L in acl.items())
     return total
-
-
-def dht(tc_th, h):
-    n = sum(h.bits)
-    return bytes([0xFF, 0xC4, (19 + n) >> 8, (19 + n) & 0xFF, tc_th]) + bytes(h.bits) + bytes(h.vals[:n])
 
 
 def with_tables(header, ht):
@@ -185,24 +96,6 @@ def test_tables_match_reference(ctx, oracle, W, H, family, gray):
 
 
 # ---- 2: length limiting and coefficients without a baseline code ---------------------------------------
-def fibonacci_coefs():
-    """luma AC symbols (run, size), run 0..1 and size 1..10, counted 1, 1, 3, 5, 9, 15, ... (f[k] = f[k-1] + f[k-2] + 1,
-    20 symbols: with the plain Fibonacci counts the tie rule balances the tree); one symbol per luma block, so EOB (one per
-    block) outweighs them all and the unconstrained code is a chain of depth 21"""
-    syms = [(r, s) for r in (0, 1) for s in range(1, 11)]
-    fib = [1, 1]
-    while len(fib) < len(syms):
-        fib.append(fib[-1] + fib[-2] + 1)
-    seq = [sym for sym, f in zip(syms, fib) for _ in range(f)]
-    np.random.default_rng(7).shuffle(seq)
-    HU = 64
-    VU = -(-len(seq) // (4 * HU))
-    coefs = np.zeros((HU * VU, 6, 64), np.int16)
-    for k, (run, s) in enumerate(seq):
-        coefs[k // 4, k % 4, run + 1] = (1 << (s - 1)) * (1 if k % 2 else -1)
-    return coefs, HU * 16, VU * 16
-
-
 def test_length_limiting(ctx, oracle):
     coefs, W, H = fibonacci_coefs()
     hist, _ = symbol_hist(coefs)

@@ -17,7 +17,8 @@ import jpezy_b200 as J
 from jpezy_b200 import capi
 from jpezy_b200.capi import EINVAL, EUNSUPPORTED, ECAPACITY, OPT_PAD_ONES, OPT_RESTART_INTERVAL, _dp
 from gpu_util import planes, to_dev
-from test_huffopt_gpu import bit_length, check_table, symbol_hist, with_tables
+from jpeg_build import bit_length, symbol_hist
+from test_huffopt_gpu import check_table, with_tables
 
 pytestmark = pytest.mark.gpu
 
